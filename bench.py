@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the Loraine.jl per-iteration interior-point hot path on B200.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload C5|C2|C3|C4|...-mini]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload C5|C2|C3|C4|...-mini] [--dump-outputs DIR]
 
 A "step" is ONE interior-point iteration (find_mu, prepare_W, predictor, sigma_update, corrector, check_convergence).
 The workload is the configuration BASELINE.json's metric ("... at 1/2/4/8 B200") is quoted on: configs[4], the synthetic
@@ -9,6 +9,8 @@ large-Schur SDP with n_var = 40000 constraints and one PSD block of side 1000 (k
 workload for EVERY N, 1 included: `--gpus N` (under torchrun) runs ONE solve whose Schur assembly and Cholesky
 factorisation are sharded over the N ranks (row-block-cyclic, NCCL) -- strong scaling; `value` = seconds per iteration of
 that one solve, max over ranks.  At N = 1 the line also carries the single-GPU configs[1..3] as `sub_records`.
+`--dump-outputs DIR` writes the iterate left by the last timed step (see dump_outputs) so that two builds can be compared
+output for output: the instance comes from a seeded generator, so the same arguments give the same inputs on every run.
 
 `value`  : seconds per IP iteration with the problem and the iterate resident in HBM.
 `e2e`    : the same iteration driven through the C ABI with the iterate in HOST (pinned) memory: X, S, y uploaded before and
@@ -51,7 +53,9 @@ def emit(line):
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=4)
+    ap.add_argument("--steps", type=int, default=4,
+                    help="timed IP iterations of the workload; the --impl reference arm times at most --cpu-max-steps of them "
+                         "and the N = 1 sub-records at most 4, each record states the count it timed")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="C5")
@@ -60,7 +64,13 @@ def parse():
     ap.add_argument("--no-sub", action="store_true", help="N = 1: skip the configs[1..3] sub-records")
     ap.add_argument("--no-parity", action="store_true", help="N > 1: skip the sharded-vs-single-GPU parity check")
     ap.add_argument("--cpu-max-steps", type=int, default=2, help="reference arm: timed CPU iterations are capped at this number")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the iterate of the last timed step as DIR/<name>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 implementation")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------------------------------
@@ -135,6 +145,42 @@ def use_all_host_threads():
         return max(got) if got else n
     except Exception:
         return int(os.environ.get("OMP_NUM_THREADS", n))
+
+
+DUMP_BYTES = 64 << 20
+
+
+def iterate_arrays(S, s):
+    """what a caller of the iteration receives: the blocks X_i and S_i, y, x_lin and s_lin (when there is an LP block), and
+    (primal objective, dual objective, DIMACS error)"""
+    md = s.model
+    y, X, xl = S.get_solution(s)
+    Sm = [np.zeros((m, m), order="F") for m in md.msizes]
+    sl = np.zeros(md.nlin)
+    PD = C.POINTER(C.c_double)
+    s._call("lrn_get_slack", (PD * max(1, md.nlmi))(*[x.ctypes.data_as(PD) for x in Sm]), sl.ctypes.data_as(PD) if md.nlin else None)
+    out = {f"X_{i}": x for i, x in enumerate(X)}
+    out.update({f"S_{i}": x for i, x in enumerate(Sm)})
+    out["y"] = y
+    if md.nlin:
+        out.update(x_lin=xl, s_lin=sl)
+    out["objectives"] = np.array([s.primal_obj, s.dual_obj, s.DIMACS_error])
+    return out
+
+
+def dump_outputs(out_dir, arrays):
+    """writes every array as out_dir/<name>.npy in float64.  When they would take more than DUMP_BYTES together, each array
+    larger than an even share of that budget is replaced by a sample of its entries (column-major flat indices drawn with
+    seed 0, sorted), which is the same on every run for the same shapes."""
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_BYTES - 256 * len(arrays)                        # 256 bytes per file cover the .npy header
+    share = budget // (8 * len(arrays))
+    sample = 8 * sum(np.size(a) for a in arrays.values()) > budget
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        if sample and a.size > share:
+            a = a.ravel(order="F")[np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def workload_name(w):
@@ -221,6 +267,7 @@ class Runner:
         S.setup_solver(self.s, self.ha)
         self.sharded = bool(sharded and pkg.dist.init_distributed(self.s))
         S.initial_point(self.s)
+        self.restart = False
 
     def _optimizer(self):
         opt = self.pkg.Optimizer()
@@ -237,17 +284,19 @@ class Runner:
 
     def step(self, sync_status=None):
         S, s = self.S, self.s
+        if self.restart:          # the last step converged (or failed): restart the same solve so that every step is a real iteration
+            S.initial_point(s)
         S.myIPstep(s, self.ha)
         s.itertime = 0.0
         s.tol_cg = max(s.tol_cg * s.tol_cg_up, s.tol_cg_min)
         S.check_convergence(s)
-        st = s.status if sync_status is None else sync_status(s.status)
-        if st != 0:               # converged (or failed): restart the same solve so that every step is a real iteration
-            S.initial_point(s)
+        # restarting at the start of the next step keeps this step's iterate on the device until then (--dump-outputs)
+        self.restart = (s.status if sync_status is None else sync_status(s.status)) != 0
 
 
-def measure(run, args, world, rank, barrier, sync_status, L, want_solve):
-    """timed device-resident steps, e2e steps, per-launch DMMA profile, optional full solve -> dict of raw results"""
+def measure(run, args, world, rank, barrier, sync_status, L, want_solve, dump_dir=None):
+    """timed device-resident steps, e2e steps, per-launch DMMA profile, optional full solve -> dict of raw results;
+    dump_dir: rank 0 writes the iterate of the last timed step there"""
     import torch
     S, s, md = run.S, run.s, run.s.model
     warm = max(args.warmup, 3)
@@ -268,8 +317,11 @@ def measure(run, args, world, rank, barrier, sync_status, L, want_solve):
     launches = L.lrn_kernel_launches() - launches0
     phase = s.timers(reset=True)
     clocks = sampler.stop() if rank == 0 else None
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, iterate_arrays(S, s))
     # ---- e2e: the iterate lives in HOST memory; upload before / download after every iteration ------------------------
     S.initial_point(s)
+    run.restart = False
     s.tol_cg = tol_cg0
     y, X, xl = S.get_solution(s)
     PD = C.POINTER(C.c_double)
@@ -386,7 +438,7 @@ def run_b200(args):
             dist.all_reduce(flag, op=dist.ReduceOp.MAX)
             return int(flag.item())
     s, md = run.s, run.s.model
-    res = measure(run, args, world, rank, barrier, sync_status, L, want_solve=not args.no_solve)
+    res = measure(run, args, world, rank, barrier, sync_status, L, want_solve=not args.no_solve, dump_dir=args.dump_outputs)
     # ---- sharded path against the single-GPU path on the same inputs (outside the timed regions) ---------------------
     parity = None
     if run.sharded and not args.no_parity:

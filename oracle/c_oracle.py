@@ -2,35 +2,43 @@
 assembly, /root/reference/src/makeBBBB.jl:39-64,139-213) -- built by `make -C oracle` (also run by __graft_entry__.build())."""
 from __future__ import annotations
 
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-_SO = os.path.join(_HERE, "_build", "liboracle.so")
 _lib = None
 
 
 def build():
-    # -march=native code must be rebuilt on the machine that runs it (the GPU box has another CPU than the build container)
-    stamp = os.path.join(_HERE, "_build", "host")
+    """path of liboracle.so compiled on this host: oracle/_build/, or, when the checkout is read-only, a private directory
+    of this process (tempfile.mkdtemp: mode 0700, unpredictable name, removed at exit)"""
+    # -march=native code must be rebuilt on the machine that runs it (the build machine may have another CPU than the GPU host)
     host = os.uname().nodename + ":" + (open("/proc/cpuinfo").read().split("model name")[1].split("\n")[0] if os.path.exists("/proc/cpuinfo") else "")
-    if os.path.exists(_SO) and os.path.exists(stamp) and open(stamp).read() == host and \
-            os.path.getmtime(_SO) >= os.path.getmtime(os.path.join(_HERE, "schur_pairs.c")):
-        return _SO
-    subprocess.run(["make", "-C", _HERE, "-B", "_build/liboracle.so"], check=True, capture_output=True)
+    d = os.path.join(_HERE, "_build")
+    so, stamp = os.path.join(d, "liboracle.so"), os.path.join(d, "host")
+    if os.path.exists(so) and os.path.exists(stamp) and open(stamp).read() == host and \
+            os.path.getmtime(so) >= os.path.getmtime(os.path.join(_HERE, "schur_pairs.c")):
+        return so
+    if not os.access(d if os.path.isdir(d) else _HERE, os.W_OK):
+        d = tempfile.mkdtemp(prefix="liboracle_")
+        atexit.register(shutil.rmtree, d, True)
+        so, stamp = os.path.join(d, "liboracle.so"), os.path.join(d, "host")
+    subprocess.run(["make", "-C", _HERE, "-B", f"O={d}", so], check=True, capture_output=True)
     with open(stamp, "w") as f:
         f.write(host)
-    return _SO
+    return so
 
 
 def lib():
     global _lib
     if _lib is None:
-        build()
-        L = C.CDLL(_SO)
+        L = C.CDLL(build())
         L.lrn_oracle_schur_pairs.restype = None
         L.lrn_oracle_schur_pairs.argtypes = [C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                              C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int64]

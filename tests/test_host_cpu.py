@@ -362,14 +362,20 @@ def test_options_struct_layout_is_the_same_in_c_python_and_julia(pkg):
     assert C.sizeof(_lib.lrn_options_t) == 8 * 4 + 2 * 8 + 2 * 4
 
 
+def _reference_src():
+    """src/ of a Loraine.jl v0.2.5 checkout named by LORAINE_JL_DIR; the repository does not carry the Julia sources"""
+    d = os.environ.get("LORAINE_JL_DIR")
+    if not d or not os.path.isdir(os.path.join(d, "src")):
+        pytest.skip("reference sources not present (set LORAINE_JL_DIR to a Loraine.jl checkout)")
+    return os.path.join(d, "src")
+
+
 @pytest.mark.parametrize("fname", ["LoraineB200.jl", "LoraineB200DD.jl"])
 def test_julia_shim_overrides_existing_reference_methods(fname):
     """Every `function S.name(...)` of the shims must be a method of a function the reference defines in module Solvers with the
     same number of positional arguments, and every `invoke(S.name, Tuple{...}, ...)` must name as many types.  Reads the
-    reference sources: skipped where /root/reference does not exist (the GPU box)."""
-    ref = "/root/reference/src"
-    if not os.path.isdir(ref):
-        pytest.skip("reference sources not present")
+    reference sources: skipped unless LORAINE_JL_DIR names a checkout of Loraine.jl."""
+    ref = _reference_src()
     defs = {}
     for f in ("Solvers.jl", "predictor_corrector.jl", "prepare_W.jl", "initial_point.jl"):
         for m in re.finditer(r"^function\s+(\w+)\(([^)]*)\)", open(os.path.join(ref, f)).read(), flags=re.M):
@@ -391,10 +397,8 @@ def test_julia_shim_overrides_existing_reference_methods(fname):
 @pytest.mark.parametrize("fname", ["LoraineB200.jl", "LoraineB200DD.jl"])
 def test_julia_shim_uses_existing_solver_and_model_fields(fname):
     """Every `solver.field` / `md.field` the shims touch must be a field of the reference's MySolver / MyModel structs
-    (src/Solvers.jl:18-107, src/model.jl:34-60).  Skipped where /root/reference does not exist."""
-    ref = "/root/reference/src"
-    if not os.path.isdir(ref):
-        pytest.skip("reference sources not present")
+    (src/Solvers.jl:18-107, src/model.jl:34-60).  Skipped unless LORAINE_JL_DIR names a checkout of Loraine.jl."""
+    ref = _reference_src()
 
     def struct_fields(path, name):
         txt = open(path).read()
