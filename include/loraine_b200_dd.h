@@ -21,6 +21,18 @@ typedef struct lrn_dd_solver* lrn_dd_handle_t;
 
 /* MySolver{Float64x2} state for nlmi = 0: n_var multipliers y, nlin LP rows (src/Solvers.jl:363-446).  device < 0: current */
 int32_t lrn_dd_create(lrn_dd_handle_t* out, int64_t n_var, int64_t nlin, int32_t device);
+/* Multi-GPU, in-process: one host thread drives `ngpus` devices (devices[r], or 0 .. ngpus-1 when devices is NULL); the NCCL
+ * communicator is made inside the library (ncclCommInitAll).  Returns a facade that every other lrn_dd_* entry point accepts:
+ * each call runs on every device, host-visible outputs come from the first.  The Schur matrix is assembled and factored
+ * row-block-cyclically over the devices (row blocks of 256 rows for n_var >= 4096, 128 for n_var >= 1024, 64 otherwise), the
+ * rest of the iteration is replicated; results equal the single-GPU ones bit for bit.  ngpus == 1: same as lrn_dd_create;
+ * ngpus <= 0: every visible device; more than visible: LRN_ERR_ARG; no device: LRN_ERR_NO_DEVICE (no CPU fallback). */
+int32_t lrn_dd_create_multi(lrn_dd_handle_t* out, int64_t n_var, int64_t nlin, int32_t ngpus, const int32_t* devices);
+/* Multi-GPU, one process per GPU: attach the handle to rank `rank` of a `world`-rank NCCL communicator; unique_id128 comes
+ * from lrn_dist_unique_id (loraine_b200.h) on rank 0 and is passed to every rank.  Call after lrn_dd_create, before the
+ * first lrn_dd_schur_assemble.  From then on lrn_dd_schur_factor is a collective (every rank calls it, in the same order as
+ * the others), and so is lrn_dd_get_array(h, 1, ...).  world = 1 runs the distributed code path on one GPU. */
+int32_t lrn_dd_dist_init(lrn_dd_handle_t h, int32_t rank, int32_t world, const void* unique_id128);
 /* C_lin (n_var x nlin, CSC, 1-based) and d_lin, src/model.jl:70-84 */
 int32_t lrn_dd_set_lin(lrn_dd_handle_t h, const int64_t* colptr, const int64_t* rowval, const double* nz_hi, const double* nz_lo,
                        const double* d_hi, const double* d_lo);
@@ -61,7 +73,9 @@ int32_t lrn_dd_sigma_trace(lrn_dd_handle_t h, double dot_lin[2]);
 int32_t lrn_dd_dimacs(lrn_dd_handle_t h, double err6[12], double by[2], double dx[2]);
 
 /* parity hook: which = 1 H (n x n, column-major, lower mirrored), 2 L (lower), 3 Rp, 4 Rd_lin, 5 rhs h, 6 dely, 7 delX_lin,
- * 8 delS_lin, 9 Xn_lin, 10 Sn_lin, 11 RNT_lin, 12 Si_lin */
+ * 8 delS_lin, 9 Xn_lin, 10 Sn_lin, 11 RNT_lin, 12 Si_lin.  On a multi-GPU handle H is gathered from the row shards of all
+ * ranks (exact: the shards are disjoint); with lrn_dd_dist_init that makes which = 1 a collective that every rank must call
+ * (hi may be NULL on the ranks that do not want the copy). */
 int32_t lrn_dd_get_array(lrn_dd_handle_t h, int32_t which, double* hi, double* lo);
 /* device milliseconds since the last reset: [0] schur_assemble, [1] schur_factor, [2] schur_solve, [3] everything else */
 int32_t lrn_dd_timers(lrn_dd_handle_t h, double ms[4], int32_t reset);

@@ -5,6 +5,7 @@
 #define LORAINE_B200_DEBUG_H
 #include <stdint.h>
 #include "loraine_b200.h"
+#include "loraine_b200_dd.h"
 #ifdef __cplusplus
 extern "C" {
 #endif
@@ -47,6 +48,10 @@ int64_t lrn_dbg_model_block(int64_t n_var, int64_t nblocks, const int64_t* block
  * the library's default for n_var) WITHOUT a communicator: lrn_schur_assemble then fills only the owned row blocks, so a test
  * on one GPU can check that the shards of all ranks add up to the full matrix.  lrn_schur_factor refuses to run in that state. */
 int32_t lrn_dbg_set_shard(lrn_handle_t h, int32_t rank, int32_t world, int32_t block_rows);
+/* the same for a double-double LP handle (loraine_b200_dd.h): block_rows a multiple of 32 (0 = the library's default for n_var).
+ * lrn_dd_schur_assemble then writes the owned rows of the lower triangle only (zeros elsewhere, no upper mirror),
+ * lrn_dd_get_array(h, 1, ...) returns that shard, and lrn_dd_schur_factor fails with LRN_ERR_STATE. */
+int32_t lrn_dd_dbg_set_shard(lrn_dd_handle_t h, int32_t rank, int32_t world, int32_t block_rows);
 /* relative Frobenius distance ||A_a - A_b||_F / ||A_b||_F over the LOWER triangles of the n_var x n_var Schur matrices
  * (which = LRN_ARR_H) or Cholesky factors (LRN_ARR_L) of two handles living on the same device; computed on the device
  * (bench.py's dist_parity: sharded handle against a single-GPU handle at n_var = 40000 without a 12.8 GB download) */

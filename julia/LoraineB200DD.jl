@@ -17,7 +17,7 @@ module LoraineB200DD
 using Loraine
 using LinearAlgebra, Printf, SparseArrays
 using MultiFloats
-import ..LoraineB200: LIB, ENABLED
+import ..LoraineB200: LIB, ENABLED, NGPUS
 const S = Loraine.Solvers
 const T2 = Float64x2
 
@@ -41,8 +41,13 @@ function S.setup_solver(solver::S.MySolver{T2}, halpha::S.Halpha)
     md = solver.model
     md.nlmi == 0 || throw(ArgumentError("Loraine.Optimizer{Float64x2} on the B200 path: models without PSD blocks only (no fallback)"))
     hr = Ref{Ptr{Cvoid}}(C_NULL)
-    rc = ccall((:lrn_dd_create, LIB[]), Int32, (Ref{Ptr{Cvoid}}, Int64, Int64, Int32), hr, md.n, md.nlin, -1)
-    rc == 0 || error("loraine_b200: lrn_dd_create failed ($rc); there is no CPU fallback")
+    # enable!(...; ngpus) other than 1: one host thread drives several GPUs (Schur matrix sharded, NCCL inside the library)
+    rc = if NGPUS[] == 1
+        ccall((:lrn_dd_create, LIB[]), Int32, (Ref{Ptr{Cvoid}}, Int64, Int64, Int32), hr, md.n, md.nlin, -1)
+    else
+        ccall((:lrn_dd_create_multi, LIB[]), Int32, (Ref{Ptr{Cvoid}}, Int64, Int64, Int32, Ptr{Int32}), hr, md.n, md.nlin, NGPUS[], C_NULL)
+    end
+    rc == 0 || error("loraine_b200: lrn_dd_create / lrn_dd_create_multi failed ($rc); there is no CPU fallback")
     HANDLES[solver] = hr[]
     Cl = SparseMatrixCSC{Float64,Int64}(md.C_lin); d = Vector{Float64}(vec(md.d_lin)); b = Vector{Float64}(vec(md.b))
     GC.@preserve Cl d b begin        # model data are Float64 in the reference (src/model.jl:44, src/Solvers.jl:576)

@@ -84,6 +84,9 @@ def lib():
         "lrn_dist_init": (i32, [vp, i32, i32, C.c_char_p]),
         # include/loraine_b200_dd.h (double-double LP path)
         "lrn_dd_create": (i32, [C.POINTER(vp), i64, i64, i32]),
+        "lrn_dd_create_multi": (i32, [C.POINTER(vp), i64, i64, i32, pi32]),
+        "lrn_dd_dist_init": (i32, [vp, i32, i32, C.c_char_p]),
+        "lrn_dd_dbg_set_shard": (i32, [vp, i32, i32, i32]),
         "lrn_dd_set_lin": (i32, [vp, pi64, pi64, pdbl, pdbl, pdbl, pdbl]),
         "lrn_dd_set_b": (i32, [vp, pdbl, pdbl]),
         "lrn_dd_finalize": (i32, [vp]),
@@ -126,9 +129,10 @@ DECLARED_SYMBOLS = ["lrn_default_options", "lrn_create", "lrn_set_block_AA", "lr
 DD_SYMBOLS = ["lrn_dd_create", "lrn_dd_set_lin", "lrn_dd_set_b", "lrn_dd_finalize", "lrn_dd_destroy", "lrn_dd_last_error",
               "lrn_dd_set_iterate", "lrn_dd_get_solution", "lrn_dd_find_mu", "lrn_dd_prepare_W", "lrn_dd_residuals",
               "lrn_dd_schur_assemble", "lrn_dd_rhs_predictor", "lrn_dd_rhs_corrector", "lrn_dd_schur_factor", "lrn_dd_schur_shift",
-              "lrn_dd_schur_solve", "lrn_dd_find_step", "lrn_dd_sigma_trace", "lrn_dd_dimacs", "lrn_dd_get_array", "lrn_dd_timers"]
+              "lrn_dd_schur_solve", "lrn_dd_find_step", "lrn_dd_sigma_trace", "lrn_dd_dimacs", "lrn_dd_get_array", "lrn_dd_timers",
+              "lrn_dd_create_multi", "lrn_dd_dist_init"]
 DD_ARR = dict(H=1, L=2, RP=3, RD=4, RHS=5, DELY=6, DELX=7, DELS=8, XN=9, SN=10, RNT=11, SI=12)
 
 DEBUG_SYMBOLS = ["lrn_dbg_gemm", "lrn_dbg_cholesky", "lrn_dbg_eig_small", "lrn_dbg_svd", "lrn_dbg_lanczos",
                  "lrn_dbg_batched_lambda_min", "lrn_dbg_peak", "lrn_dbg_gemm_profile", "lrn_dbg_set_shard", "lrn_dbg_compare",
-                 "lrn_dbg_gather_H", "lrn_dbg_model_block"]
+                 "lrn_dbg_gather_H", "lrn_dbg_model_block", "lrn_dd_dbg_set_shard"]

@@ -8,32 +8,11 @@
 // instructions (24 DADD + 2 DMUL + 2 DFMA), most of them dependent, so these kernels are bound by FP64 issue (the trailing
 // update runs the FP64 pipe at 89 %, profiles/r2_dd_syrk_ncu_full.csv) or by dependent-issue latency, not by memory.  Layout: vectors as arrays of dd (16 B per
 // entry, one 128-bit access), H and L dense column-major with leading dimension n.
-#include "common.cuh"
-#include "dd.cuh"
-#include "../../include/loraine_b200.h"
-#include "../../include/loraine_b200_dd.h"
-#include <algorithm>
+#include "ddlp.cuh"
+#include "group.cuh"
+#include "dist.cuh"
 
 using namespace lrn;
-
-struct lrn_dd_solver {
-    int device = 0;
-    cudaStream_t st = nullptr, st2 = nullptr;
-    cudaEvent_t evP = nullptr, evR = nullptr;
-    std::string err;
-    int n = 0, nlin = 0;
-    long long nnz = 0;
-    // C_lin by LP column (CSC) and by multiplier row (CSR): the transposed product and the Schur rows each want one of them
-    DevBuf<int> cptr, cidx, rptr, ridx;
-    DevBuf<dd> cval, rval;
-    DevBuf<dd> d, b, x, s, si, y, rp, rd, rhs, dely, dx, ds, xn, sn, rnt, w, tl, tn;
-    DevBuf<dd> H, L, red, rdiag;
-    DevBuf<int> info, flags;      // info[0]: Cholesky pivot, info[1]: time-out of the flag wait in the multi-CTA solves
-    int trsv_ctas = 0, trsv_epoch = 0;
-    bool have_lin = false, have_b = false, finalized = false, have_iterate = false, have_H = false, have_factor = false;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    double t_ms[4] = {0, 0, 0, 0};
-};
 
 namespace {
 
@@ -60,10 +39,14 @@ __global__ void __launch_bounds__(TB) k_dd_spmv(int rows, const int* __restrict_
 
 // H(:, i) (rows j >= i) = sum_k C[i,k] w[k] C[j,k]: one CTA per multiplier row i; the LP columns k of that row one after the
 // other (two of them may hit the same j), the entries j of column k in parallel.          src/predictor_corrector.jl:37
+// SHARD: only the rows j of row blocks (height pw) g with g % world == rank are written, every other entry of the column is
+// zero.  An owned entry receives the same dd_fma sequence as without sharding, so the shards of all ranks add up to the
+// single-GPU matrix bit for bit.
+template <bool SHARD>
 __global__ void __launch_bounds__(TB) k_dd_lp_schur(int n, const int* __restrict__ rptr, const int* __restrict__ ridx,
                                                      const dd* __restrict__ rval, const int* __restrict__ cptr,
                                                      const int* __restrict__ cidx, const dd* __restrict__ cval,
-                                                     const dd* __restrict__ w, dd* __restrict__ H) {
+                                                     const dd* __restrict__ w, dd* __restrict__ H, int rank, int world, int pw) {
     const int i = blockIdx.x;
     dd* col = H + (size_t)i * n;
     for (int j = threadIdx.x; j < n; j += blockDim.x) col[j] = dd_make(0.0);
@@ -73,7 +56,7 @@ __global__ void __launch_bounds__(TB) k_dd_lp_schur(int n, const int* __restrict
         const dd coef = dd_mul(rval[e], w[k]);
         for (int f = cptr[k] + threadIdx.x; f < cptr[k + 1]; f += blockDim.x) {
             const int j = cidx[f];
-            if (j >= i) col[j] = dd_fma(coef, cval[f], col[j]);
+            if (j >= i && (!SHARD || (j / pw) % world == rank)) col[j] = dd_fma(coef, cval[f], col[j]);
         }
         __syncthreads();
     }
@@ -88,112 +71,10 @@ __global__ void k_dd_shift_diag(int n, dd* __restrict__ H, double delta) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) H[(size_t)i * n + i] = dd_add_d(H[(size_t)i * n + i], delta);
 }
-
-// ------------------------------------------------------------------------------------------------------------------------
-// tiled right-looking Cholesky (32 x 32 tiles): factor the diagonal tile, solve the tiles below it, update the trailing tiles
-// ------------------------------------------------------------------------------------------------------------------------
-// (the reciprocals of the pivots go to rdiag: the solves below multiply by them instead of dividing -- a double-double division
-// is ~10 times a multiplication)
-__global__ void __launch_bounds__(TS * TS) k_dd_potrf_tile(dd* __restrict__ A, int n, int k0, int w, int* __restrict__ info,
-                                                           dd* __restrict__ rdiag) {
-    __shared__ dd t[TS][TS + 1];
-    __shared__ dd rinv[TS];
-    __shared__ int bad;
-    const int r = threadIdx.x, c = threadIdx.y;           // r fastest: coalesced along a column
-    if (r == 0 && c == 0) bad = 0;
-    if (r < w && c < w) t[r][c] = A[(size_t)(k0 + c) * n + k0 + r];
-    __syncthreads();
-    if (*info != 0) return;                                // an earlier tile already failed
-    for (int j = 0; j < w; j++) {
-        if (r == j && c == j) {
-            if (dd_le_zero(t[j][j]) || !(t[j][j].hi == t[j][j].hi)) bad = 1;
-            else {
-                const dd rs = dd_rsqrt(t[j][j]);            // pivot = a * rsqrt(a), its reciprocal = rsqrt(a)
-                t[j][j] = dd_mul(t[j][j], rs);
-                rinv[j] = rs;
-                rdiag[k0 + j] = rs;
-            }
-        }
-        __syncthreads();
-        if (bad) {
-            if (r == 0 && c == 0) *info = k0 + j + 1;
-            return;
-        }
-        if (c == j && r > j && r < w) t[r][j] = dd_mul(t[r][j], rinv[j]);
-        __syncthreads();
-        if (c > j && c < w && r >= c && r < w) t[r][c] = dd_fms(t[r][j], t[c][j], t[r][c]);
-        __syncthreads();
-    }
-    if (r < w && c < w) A[(size_t)(k0 + c) * n + k0 + r] = (r >= c) ? t[r][c] : dd_make(0.0);
-}
-
-// X Lkk' = A for the 32-row tile `blockIdx.x` below the diagonal tile.  Eight warps per tile, lane = row of the tile.  The 32
-// columns are solved in four blocks of eight: first all warps subtract the contribution of the finished blocks from the eight
-// columns of the current block (warp = column: independent dot products), then warp 0 runs the short substitution inside the
-// block.  The dependent chain per row is 4 x 28 multiply-adds instead of 496 (a single warp doing the whole substitution took
-// 41 us per step at n = 2000 and was the longest kernel of the panel chain).
-constexpr int TRSM_CB = 8;
-__global__ void __launch_bounds__(TS * TRSM_CB) k_dd_trsm_tile(dd* __restrict__ A, int n, int k0, int w, const dd* __restrict__ rdiag) {
-    __shared__ dd l[TS][TS + 1];
-    __shared__ dd xr[TS][TS + 1];
-    __shared__ dd rd[TS];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int i0 = k0 + w + blockIdx.x * TS, row = i0 + lane;
-    if (warp == 0 && lane < w) rd[lane] = rdiag[k0 + lane];
-    for (int c = warp; c < w; c += TRSM_CB) {
-        if (lane < w) l[lane][c] = A[(size_t)(k0 + c) * n + k0 + lane];
-        xr[lane][c] = (row < n) ? A[(size_t)(k0 + c) * n + row] : dd_make(0.0);
-    }
-    __syncthreads();
-    for (int c0 = 0; c0 < w; c0 += TRSM_CB) {
-        const int c = c0 + warp;
-        if (c0 > 0 && c < w) {
-            dd a0 = xr[lane][c], a1 = dd_make(0.0), a2 = dd_make(0.0), a3 = dd_make(0.0);
-            for (int p = 0; p < c0; p += 4) {                       // c0 is a multiple of 8
-                a0 = dd_fms(xr[lane][p], l[c][p], a0);
-                a1 = dd_fms(xr[lane][p + 1], l[c][p + 1], a1);
-                a2 = dd_fms(xr[lane][p + 2], l[c][p + 2], a2);
-                a3 = dd_fms(xr[lane][p + 3], l[c][p + 3], a3);
-            }
-            xr[lane][c] = dd_add(dd_add(a0, a1), dd_add(a2, a3));
-        }
-        __syncthreads();
-        if (warp == 0) {
-            const int c1 = min(w, c0 + TRSM_CB);
-            for (int cc = c0; cc < c1; cc++) {
-                dd v = xr[lane][cc];
-                for (int p = c0; p < cc; p++) v = dd_fms(xr[lane][p], l[cc][p], v);
-                xr[lane][cc] = dd_mul(v, rd[cc]);
-            }
-        }
-        __syncthreads();
-    }
-    if (row < n)
-        for (int c = warp; c < w; c += TRSM_CB) A[(size_t)(k0 + c) * n + row] = xr[lane][c];
-}
-
-// A(I, J) -= X_I X_J' for the tile pairs I >= J of the trailing matrix (K = w)
-// (column tiles jt0 + blockIdx.y: the first tile column of the trailing matrix is updated on the panel stream, the rest on a
-// second stream -- see lrn_dd_schur_factor)
-__global__ void __launch_bounds__(TS * TS) k_dd_syrk_tile(dd* __restrict__ A, int n, int k0, int w, int jt0) {
-    const int jt = jt0 + blockIdx.y;
-    if (jt > (int)blockIdx.x) return;
-    __shared__ dd xi[TS][TS + 1];
-    __shared__ dd xj[TS][TS + 1];
-    const int r = threadIdx.x, c = threadIdx.y;
-    const int base = k0 + w, i0 = base + blockIdx.x * TS, j0 = base + jt * TS;
-    // thread (r, c) loads column c of the panel for row r of both tiles
-    if (c < w) {
-        xi[r][c] = (i0 + r < n) ? A[(size_t)(k0 + c) * n + i0 + r] : dd_make(0.0);
-        xj[r][c] = (j0 + r < n) ? A[(size_t)(k0 + c) * n + j0 + r] : dd_make(0.0);
-    }
-    __syncthreads();
-    const int gi = i0 + r, gj = j0 + c;
-    if (gi < n && gj < n && gi >= gj) {
-        dd acc = A[(size_t)gj * n + gi];
-        for (int p = 0; p < w; p++) acc = dd_fms(xi[r][p], xj[c][p], acc);
-        A[(size_t)gj * n + gi] = acc;
-    }
+// sharded H: the diagonal entries of the rank's own row blocks only
+__global__ void k_dd_shift_own_diag(int n, dd* __restrict__ H, double delta, int rank, int world, int pw) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n && (i / pw) % world == rank) H[(size_t)i * n + i] = dd_add_d(H[(size_t)i * n + i], delta);
 }
 
 // ------------------------------------------------------------------------------------------------------------------------
@@ -585,6 +466,8 @@ void trsv(lrn_dd_solver* h, bool fwd, dd* x) {
     LRN_CHECK_LAUNCH();
 }
 
+lrn_dd_solver* dd_member0(lrn_dd_solver* facade) { return static_cast<GroupOf<lrn_dd_solver>*>(facade->group)->members[0]; }
+
 }  // namespace
 
 extern "C" {
@@ -638,6 +521,16 @@ int32_t lrn_dd_create(lrn_dd_handle_t* out, int64_t n_var, int64_t nlin, int32_t
 
 int32_t lrn_dd_destroy(lrn_dd_handle_t h) {
     if (!h) return LRN_OK;
+    if (h->group) {
+        auto* g = static_cast<GroupOf<lrn_dd_solver>*>(h->group);
+        // the communicators of one ncclCommInitAll clique are destroyed from concurrent threads (ncclCommDestroy may wait for peers)
+        std::vector<std::thread> th;
+        for (auto* m : g->members) th.emplace_back([m] { lrn_dd_destroy(m); });
+        for (auto& t : th) t.join();
+        delete g;
+        delete h;
+        return LRN_OK;
+    }
     cudaSetDevice(h->device);
     if (h->st) { cudaStreamSynchronize(h->st); cudaStreamDestroy(h->st); }
     if (h->st2) { cudaStreamSynchronize(h->st2); cudaStreamDestroy(h->st2); }
@@ -645,14 +538,19 @@ int32_t lrn_dd_destroy(lrn_dd_handle_t h) {
     if (h->evR) cudaEventDestroy(h->evR);
     if (h->ev0) cudaEventDestroy(h->ev0);
     if (h->ev1) cudaEventDestroy(h->ev1);
+    if (h->nccl) { delete static_cast<DistCtx*>(h->nccl); h->nccl = nullptr; }
     delete h;
     return LRN_OK;
 }
 
-const char* lrn_dd_last_error(lrn_dd_handle_t h) { return h ? h->err.c_str() : "null handle"; }
+const char* lrn_dd_last_error(lrn_dd_handle_t h) {
+    if (h && h->group && h->err.empty()) return dd_member0(h)->err.c_str();
+    return h ? h->err.c_str() : "null handle";
+}
 
 int32_t lrn_dd_set_lin(lrn_dd_handle_t h, const int64_t* colptr, const int64_t* rowval, const double* nz_hi, const double* nz_lo,
                        const double* d_hi, const double* d_lo) {
+    LRN_GROUP(h, lrn_dd_set_lin(m_, colptr, rowval, nz_hi, nz_lo, d_hi, d_lo));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(colptr && rowval && nz_hi && d_hi, "null argument");
         const int n = h->n, m = h->nlin;
@@ -694,6 +592,7 @@ int32_t lrn_dd_set_lin(lrn_dd_handle_t h, const int64_t* colptr, const int64_t* 
 }
 
 int32_t lrn_dd_set_b(lrn_dd_handle_t h, const double* b_hi, const double* b_lo) {
+    LRN_GROUP(h, lrn_dd_set_b(m_, b_hi, b_lo));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(b_hi, "null argument");
         upload_dd(h, h->b, b_hi, b_lo, (size_t)h->n);
@@ -703,6 +602,7 @@ int32_t lrn_dd_set_b(lrn_dd_handle_t h, const double* b_hi, const double* b_lo) 
 }
 
 int32_t lrn_dd_finalize(lrn_dd_handle_t h) {
+    LRN_GROUP(h, lrn_dd_finalize(m_));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(h->have_lin && h->have_b, "lrn_dd_set_lin and lrn_dd_set_b first");
         // norm(b), norm(d_lin) for the DIMACS denominators (src/Solvers.jl:499, :514)
@@ -718,6 +618,7 @@ int32_t lrn_dd_finalize(lrn_dd_handle_t h) {
 
 int32_t lrn_dd_set_iterate(lrn_dd_handle_t h, const double* y_hi, const double* y_lo, const double* x_hi, const double* x_lo,
                            const double* s_hi, const double* s_lo) {
+    LRN_GROUP(h, lrn_dd_set_iterate(m_, y_hi, y_lo, x_hi, x_lo, s_hi, s_lo));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(h->finalized, "lrn_dd_finalize first");
         LRN_REQUIRE(y_hi && x_hi && s_hi, "null argument");
@@ -733,6 +634,7 @@ int32_t lrn_dd_set_iterate(lrn_dd_handle_t h, const double* y_hi, const double* 
 }
 
 int32_t lrn_dd_get_solution(lrn_dd_handle_t h, double* y_hi, double* y_lo, double* x_hi, double* x_lo, double* s_hi, double* s_lo) {
+    if (h && h->group) return lrn_dd_get_solution(dd_member0(h), y_hi, y_lo, x_hi, x_lo, s_hi, s_lo);     // replicated
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(h->have_iterate, "no iterate");
         if (y_hi || y_lo) download_dd(h, h->y.p, y_hi, y_lo, (size_t)h->n);
@@ -743,6 +645,7 @@ int32_t lrn_dd_get_solution(lrn_dd_handle_t h, double* y_hi, double* y_lo, doubl
 }
 
 int32_t lrn_dd_find_mu(lrn_dd_handle_t h, double mu[2]) {
+    LRN_GROUP(h, lrn_dd_find_mu(m_, r_ == 0 ? mu : group_scratch().d));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(h->have_iterate && mu, "no iterate");
         Timed t(h, 3);
@@ -755,6 +658,7 @@ int32_t lrn_dd_find_mu(lrn_dd_handle_t h, double mu[2]) {
 }
 
 int32_t lrn_dd_prepare_W(lrn_dd_handle_t h) {
+    LRN_GROUP(h, lrn_dd_prepare_W(m_));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(h->have_iterate, "no iterate");
         Timed t(h, 3);
@@ -765,6 +669,7 @@ int32_t lrn_dd_prepare_W(lrn_dd_handle_t h) {
 }
 
 int32_t lrn_dd_residuals(lrn_dd_handle_t h) {
+    LRN_GROUP(h, lrn_dd_residuals(m_));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(h->have_iterate, "no iterate");
         Timed t(h, 3);
@@ -777,16 +682,26 @@ int32_t lrn_dd_residuals(lrn_dd_handle_t h) {
 }
 
 int32_t lrn_dd_schur_assemble(lrn_dd_handle_t h) {
+    LRN_GROUP(h, lrn_dd_schur_assemble(m_));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(h->have_iterate, "no iterate");
         Timed t(h, 0);
         const int n = h->n;
         k_dd_mul2<<<nblk(h->nlin), TB, 0, h->st>>>(h->nlin, h->x.p, h->si.p, h->w.p);
         LRN_CHECK_LAUNCH();
-        k_dd_lp_schur<<<n, TB, 0, h->st>>>(n, h->rptr.p, h->ridx.p, h->rval.p, h->cptr.p, h->cidx.p, h->cval.p, h->w.p, h->H.p);
-        LRN_CHECK_LAUNCH();
-        k_dd_mirror_lower<<<dim3(nblk(n), (unsigned)n), TB, 0, h->st>>>(n, h->H.p);
-        LRN_CHECK_LAUNCH();
+        if (dd_sharded(h)) {
+            // own rows of the lower triangle only (the upper mirror would mix the shards); lrn_dd_get_array(1) gathers them
+            k_dd_lp_schur<true><<<n, TB, 0, h->st>>>(n, h->rptr.p, h->ridx.p, h->rval.p, h->cptr.p, h->cidx.p, h->cval.p, h->w.p,
+                                                     h->H.p, h->rank, h->world, h->pw);
+            LRN_CHECK_LAUNCH();
+        } else {
+            k_dd_lp_schur<false><<<n, TB, 0, h->st>>>(n, h->rptr.p, h->ridx.p, h->rval.p, h->cptr.p, h->cidx.p, h->cval.p, h->w.p,
+                                                      h->H.p, 0, 1, 1);
+            LRN_CHECK_LAUNCH();
+            k_dd_mirror_lower<<<dim3(nblk(n), (unsigned)n), TB, 0, h->st>>>(n, h->H.p);
+            LRN_CHECK_LAUNCH();
+        }
+        h->H_gathered = false;
         h->have_H = true;
         h->have_factor = false;
         return LRN_OK;
@@ -794,19 +709,30 @@ int32_t lrn_dd_schur_assemble(lrn_dd_handle_t h) {
 }
 
 int32_t lrn_dd_schur_shift(lrn_dd_handle_t h, double delta) {
+    LRN_GROUP(h, lrn_dd_schur_shift(m_, delta));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(h->have_H, "lrn_dd_schur_assemble first");
-        k_dd_shift_diag<<<nblk(h->n), TB, 0, h->st>>>(h->n, h->H.p, delta);
+        if (dd_sharded(h) && !h->H_gathered)
+            k_dd_shift_own_diag<<<nblk(h->n), TB, 0, h->st>>>(h->n, h->H.p, delta, h->rank, h->world, h->pw);
+        else
+            k_dd_shift_diag<<<nblk(h->n), TB, 0, h->st>>>(h->n, h->H.p, delta);
         LRN_CHECK_LAUNCH();
         return LRN_OK;
     });
 }
 
 int32_t lrn_dd_schur_factor(lrn_dd_handle_t h) {
+    LRN_GROUP(h, lrn_dd_schur_factor(m_));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(h->have_H, "lrn_dd_schur_assemble first");
         int info = 0;
-        {
+        if (dd_sharded(h)) {
+            // a handle sharded through lrn_dd_dbg_set_shard holds one shard of H: it must not factor it
+            if (!h->nccl) throw std::runtime_error("the Schur rows are sharded but the handle has no NCCL communicator "
+                                                   "(lrn_dd_dist_init / lrn_dd_create_multi)");
+            Timed t(h, 1);
+            info = dd_factor_dist(h);
+        } else {
             Timed t(h, 1);
             const int n = h->n;
             // (replaying the factorisation as a CUDA graph was measured: 6.85 ms against 6.24 ms eager at n = 2000 -- the chain
@@ -852,6 +778,7 @@ int32_t lrn_dd_schur_factor(lrn_dd_handle_t h) {
 }
 
 int32_t lrn_dd_rhs_predictor(lrn_dd_handle_t h) {
+    LRN_GROUP(h, lrn_dd_rhs_predictor(m_));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(h->have_iterate, "no iterate");
         Timed t(h, 3);
@@ -863,6 +790,7 @@ int32_t lrn_dd_rhs_predictor(lrn_dd_handle_t h) {
 }
 
 int32_t lrn_dd_rhs_corrector(lrn_dd_handle_t h, const double sigma[2], const double mu[2]) {
+    LRN_GROUP(h, lrn_dd_rhs_corrector(m_, sigma, mu));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(h->have_iterate && sigma && mu, "no iterate");
         Timed t(h, 3);
@@ -876,6 +804,7 @@ int32_t lrn_dd_rhs_corrector(lrn_dd_handle_t h, const double sigma[2], const dou
 }
 
 int32_t lrn_dd_schur_solve(lrn_dd_handle_t h, int32_t which) {
+    LRN_GROUP(h, lrn_dd_schur_solve(m_, which));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(h->have_factor, "lrn_dd_schur_factor first");
         LRN_REQUIRE(which == 3 || which == 6, "which must be 3 or 6");
@@ -898,6 +827,8 @@ int32_t lrn_dd_schur_solve(lrn_dd_handle_t h, int32_t which) {
 
 int32_t lrn_dd_find_step(lrn_dd_handle_t h, int32_t predict, const double sigma[2], const double mu[2], double tau,
                          double alpha_lin[2], double beta_lin[2]) {
+    LRN_GROUP(h, lrn_dd_find_step(m_, predict, sigma, mu, tau, r_ == 0 ? alpha_lin : group_scratch().d,
+                                  r_ == 0 ? beta_lin : group_scratch().d + 2));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(h->have_iterate && sigma && mu && alpha_lin && beta_lin, "no iterate");
         Timed t(h, 3);
@@ -929,6 +860,7 @@ int32_t lrn_dd_find_step(lrn_dd_handle_t h, int32_t predict, const double sigma[
 }
 
 int32_t lrn_dd_sigma_trace(lrn_dd_handle_t h, double dot_lin[2]) {
+    LRN_GROUP(h, lrn_dd_sigma_trace(m_, r_ == 0 ? dot_lin : group_scratch().d));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(h->have_iterate && dot_lin, "no iterate");
         Timed t(h, 3);
@@ -940,6 +872,8 @@ int32_t lrn_dd_sigma_trace(lrn_dd_handle_t h, double dot_lin[2]) {
 }
 
 int32_t lrn_dd_dimacs(lrn_dd_handle_t h, double err6[12], double by[2], double dx[2]) {
+    LRN_GROUP(h, r_ == 0 ? lrn_dd_dimacs(m_, err6, by, dx)
+                       : lrn_dd_dimacs(m_, group_scratch().d, group_scratch().d + 12, group_scratch().d + 14));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(h->have_iterate && err6 && by && dx, "no iterate");
         Timed t(h, 3);
@@ -961,11 +895,25 @@ int32_t lrn_dd_dimacs(lrn_dd_handle_t h, double err6[12], double by[2], double d
 }
 
 int32_t lrn_dd_get_array(lrn_dd_handle_t h, int32_t which, double* hi, double* lo) {
+    // H is a collective on a facade (every member contributes its row shard); everything else is replicated -> member 0
+    if (h && h->group && which != 1) return lrn_dd_get_array(dd_member0(h), which, hi, lo);
+    LRN_GROUP(h, lrn_dd_get_array(m_, which, r_ == 0 ? hi : nullptr, r_ == 0 ? lo : nullptr));
     return guarded(h, [&]() -> int32_t {
-        LRN_REQUIRE(hi, "null argument");
+        // (a null output is allowed for H on a sharded handle: ranks other than the caller's only take part in the gather)
+        LRN_REQUIRE(hi || (which == 1 && dd_sharded(h)), "null argument");
         const size_t n = (size_t)h->n, m = (size_t)h->nlin;
         switch (which) {
-            case 1: LRN_REQUIRE(h->have_H, "no Schur matrix"); download_dd(h, h->H.p, hi, lo, n * n); break;
+            case 1:
+                LRN_REQUIRE(h->have_H, "no Schur matrix");
+                if (h->nccl && !h->H_gathered) {
+                    // every rank holds its own rows of the lower triangle, zeros elsewhere: the sum is exact
+                    dd_gather_H(h);
+                    k_dd_mirror_lower<<<dim3(nblk((long long)n), (unsigned)n), TB, 0, h->st>>>((int)n, h->H.p);
+                    LRN_CHECK_LAUNCH();
+                    h->H_gathered = true;
+                }
+                if (hi) download_dd(h, h->H.p, hi, lo, n * n);
+                break;
             case 2: LRN_REQUIRE(h->have_factor, "no factor"); download_dd(h, h->L.p, hi, lo, n * n); break;
             case 3: download_dd(h, h->rp.p, hi, lo, n); break;
             case 4: download_dd(h, h->rd.p, hi, lo, m); break;
@@ -984,6 +932,9 @@ int32_t lrn_dd_get_array(lrn_dd_handle_t h, int32_t which, double* hi, double* l
 }
 
 int32_t lrn_dd_timers(lrn_dd_handle_t h, double ms[4], int32_t reset) {
+    // a facade reports member 0's device times; a reset resets every member
+    if (h && h->group && !reset) return lrn_dd_timers(dd_member0(h), ms, 0);
+    LRN_GROUP(h, lrn_dd_timers(m_, r_ == 0 ? ms : group_scratch().d, reset));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(ms, "null argument");
         for (int k = 0; k < 4; k++) { ms[k] = h->t_ms[k]; if (reset) h->t_ms[k] = 0.0; }

@@ -4,19 +4,23 @@
 // runs the same entry point on its own device from its own short-lived host thread (rank 0 on the caller's thread), exactly
 // as the ranks of a one-process-per-GPU launch would, so the sharded Schur assembly / row-block-cyclic Cholesky code is the
 // same in both modes.  Host-visible outputs are taken from member 0; the other members write into thread-local scratch.
+// The facade is generic over the handle type: lrn_create_multi (Float64, lrn_solver) and lrn_dd_create_multi (double-double
+// LP path, lrn_dd_solver) share it.  A handle type needs `void* group` and `std::string err`.
 #pragma once
 #include "solver.cuh"
 #include <thread>
 
 namespace lrn {
 
-struct Group {
-    std::vector<lrn_solver*> members;
+template <typename Hd>
+struct GroupOf {
+    std::vector<Hd*> members;
 };
+using Group = GroupOf<lrn_solver>;
 
-template <typename F>
-int32_t group_call(lrn_solver* facade, F&& f) {
-    Group* g = static_cast<Group*>(facade->group);
+template <typename Hd, typename F>
+int32_t group_call(Hd* facade, F&& f) {
+    GroupOf<Hd>* g = static_cast<GroupOf<Hd>*>(facade->group);
     const int N = (int)g->members.size();
     facade->err.clear();
     std::vector<int32_t> rc(N, 0);
@@ -35,7 +39,7 @@ int32_t group_call(lrn_solver* facade, F&& f) {
 
 // scratch outputs of the members with rank > 0
 struct GroupScratch {
-    double d[8];
+    double d[16];
     int32_t i32[4];
     int64_t i64[4];
     std::vector<double> a, b;
@@ -51,5 +55,5 @@ inline GroupScratch& group_scratch() {
 #define LRN_GROUP(h, CALL)                                                                          \
     do {                                                                                            \
         if ((h) && (h)->group)                                                                      \
-            return lrn::group_call((h), [&](lrn_solver* m_, int r_) -> int32_t { (void)r_; return CALL; }); \
+            return lrn::group_call((h), [&](auto* m_, int r_) -> int32_t { (void)r_; return CALL; }); \
     } while (0)

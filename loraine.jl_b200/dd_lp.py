@@ -62,6 +62,7 @@ class DDSolver:
         self.initpoint = int(o["initpoint"])
         self.verb = int(o["verb"])
         self.device = int(o.get("device", -1))
+        self.ngpus = int(o.get("ngpus", 1))        # 1: one device; otherwise lrn_dd_create_multi (<= 0: every visible device)
         self.lib = _lib.lib()
         self.h = C.c_void_p()
         self.status = 0
@@ -110,9 +111,15 @@ def setup_solver(s: DDSolver):
     md = s.model
     if s.h:
         s.close()
-    rc = s.lib.lrn_dd_create(C.byref(s.h), md.n, md.nlin, s.device)
-    if rc != 0:
-        raise LoraineB200DDError(f"lrn_dd_create failed ({rc}): no usable sm_100 CUDA device; there is no CPU fallback")
+    if s.ngpus != 1:                           # one host thread, N devices: the library owns the NCCL communicator
+        rc = s.lib.lrn_dd_create_multi(C.byref(s.h), md.n, md.nlin, s.ngpus, None)
+        if rc != 0:
+            raise LoraineB200DDError(f"lrn_dd_create_multi(ngpus={s.ngpus}) failed ({rc}): not enough usable sm_100 CUDA devices "
+                                     "or no NCCL; there is no CPU fallback")
+    else:
+        rc = s.lib.lrn_dd_create(C.byref(s.h), md.n, md.nlin, s.device)
+        if rc != 0:
+            raise LoraineB200DDError(f"lrn_dd_create failed ({rc}): no usable sm_100 CUDA device; there is no CPU fallback")
     M = sp.csc_matrix(md.C_lin)
     M.sum_duplicates()
     M.sort_indices()

@@ -19,6 +19,11 @@ def block_rows(n_var: int) -> int:
     return 512 if n_var >= 16384 else (256 if n_var >= 4096 else 128)
 
 
+def dd_block_rows(n_var: int) -> int:
+    """height of a row block of the double-double LP path (mirrors lrn::dd_block_rows in csrc/ddlp.cuh)"""
+    return 256 if n_var >= 4096 else (128 if n_var >= 1024 else 64)
+
+
 def first_block(p: int, rank: int, world: int) -> int:
     """first row block >= p owned by `rank` (mirrors first_block in csrc/dist.cu)"""
     return p + ((rank - p % world + world) % world)
@@ -59,6 +64,29 @@ def init_distributed(solver) -> bool:
     uid = exchange_unique_id(make_id, rank, world)
     buf = C.create_string_buffer(uid, 128)
     solver._call("lrn_dist_init", rank, world, buf)
+    solver.dist_rank, solver.dist_world = rank, world
+    return True
+
+
+def init_distributed_dd(solver) -> bool:
+    """The double-double counterpart of init_distributed for a dd_lp.DDSolver (call after dd_lp.setup_solver, before the first
+    iteration): attaches the handle to the job's NCCL communicator with lrn_dd_dist_init.  Every rank then runs the whole
+    solve; the Schur assembly and factorisation are sharded, everything else is replicated.  Returns True when the job has
+    more than one rank."""
+    import torch.distributed as dist
+    if not dist.is_available() or not dist.is_initialized() or dist.get_world_size() <= 1:
+        return False
+    rank, world = dist.get_rank(), dist.get_world_size()
+    lib = solver.lib
+
+    def make_id():
+        buf = C.create_string_buffer(128)
+        rc = lib.lrn_dist_unique_id(buf)
+        if rc != 0:
+            raise RuntimeError(f"lrn_dist_unique_id failed ({rc})")
+        return buf.raw
+    uid = exchange_unique_id(make_id, rank, world)
+    solver._call("lrn_dd_dist_init", rank, world, C.create_string_buffer(uid, 128))
     solver.dist_rank, solver.dist_world = rank, world
     return True
 
