@@ -62,7 +62,8 @@ int32_t lrn_dd_rhs_corrector(lrn_dd_handle_t h, const double sigma[2], const dou
 int32_t lrn_dd_schur_factor(lrn_dd_handle_t h);
 /* BBBB += delta I, src/predictor_corrector.jl:74 */
 int32_t lrn_dd_schur_shift(lrn_dd_handle_t h, double delta);
-/* dely = L' \ (L \ h) (which = 3) or (L L')^-1 (L L')^-1 h (which = 6, the regularised-path quirk), src/predictor_corrector.jl:85-90,199 */
+/* dely = L' \ (L \ h) (which = 3) or (L L')^-1 (L L')^-1 h (which = 6, the regularised-path quirk), src/predictor_corrector.jl:85-90,199.
+ * LRN_ERR_STATE when there is no valid factor (no lrn_dd_schur_factor since the Schur matrix changed, or it failed). */
 int32_t lrn_dd_schur_solve(lrn_dd_handle_t h, int32_t which);
 /* find_step_lin, src/predictor_corrector.jl:329-364.  predict != 0: Xn_lin, Sn_lin, RNT_lin; else the iterate is updated. */
 int32_t lrn_dd_find_step(lrn_dd_handle_t h, int32_t predict, const double sigma[2], const double mu[2], double tau,

@@ -52,6 +52,18 @@ int32_t lrn_dbg_set_shard(lrn_handle_t h, int32_t rank, int32_t world, int32_t b
  * lrn_dd_schur_assemble then writes the owned rows of the lower triangle only (zeros elsewhere, no upper mirror),
  * lrn_dd_get_array(h, 1, ...) returns that shard, and lrn_dd_schur_factor fails with LRN_ERR_STATE. */
 int32_t lrn_dd_dbg_set_shard(lrn_dd_handle_t h, int32_t rank, int32_t world, int32_t block_rows);
+/* test hook: load an array of a double-double LP handle directly, so that the factorisation and the solves can be checked on
+ * matrices whose factor is known exactly.  Ids as in lrn_dd_get_array; lo may be NULL (exact doubles).
+ *   which = 1: the Schur matrix H (n_var x n_var, symmetric, column-major, full).  No iterate is needed; the handle then holds
+ *              a Schur matrix and no factor.  A sharded handle keeps only its own rows of the lower triangle (zeros
+ *              elsewhere), the state lrn_dd_schur_assemble leaves, so lrn_dd_schur_factor runs the distributed path.
+ *   which = 5: the right-hand side h of lrn_dd_schur_solve (n_var).
+ * On a lrn_dd_create_multi handle every device receives the same array.  Any other id: LRN_ERR_ARG. */
+int32_t lrn_dd_dbg_set_array(lrn_dd_handle_t h, int32_t which, const double* hi, const double* lo);
+/* test hook: the number of CTAs of the multi-CTA triangular solves of lrn_dd_schur_solve.  0 = the single-CTA kernels,
+ * -1 = the value lrn_dd_create chose, >= 1 = that many, clamped to the lrn_dd_create value (every CTA must stay resident:
+ * the CTAs wait on each other's results).  Fewer CTAs than row tiles make one CTA solve several tiles. */
+int32_t lrn_dd_dbg_set_trsv_ctas(lrn_dd_handle_t h, int32_t ctas);
 /* relative Frobenius distance ||A_a - A_b||_F / ||A_b||_F over the LOWER triangles of the n_var x n_var Schur matrices
  * (which = LRN_ARR_H) or Cholesky factors (LRN_ARR_L) of two handles living on the same device; computed on the device
  * (bench.py's dist_parity: sharded handle against a single-GPU handle at n_var = 40000 without a 12.8 GB download) */

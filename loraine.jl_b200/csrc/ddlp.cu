@@ -12,6 +12,8 @@
 #include "group.cuh"
 #include "dist.cuh"
 
+#include "../../include/loraine_b200_debug.h"
+
 using namespace lrn;
 
 namespace {
@@ -70,6 +72,11 @@ __global__ void k_dd_mirror_lower(int n, dd* __restrict__ H) {      // Hermitian
 __global__ void k_dd_shift_diag(int n, dd* __restrict__ H, double delta) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) H[(size_t)i * n + i] = dd_add_d(H[(size_t)i * n + i], delta);
+}
+// sharded H: keep the rank's own rows of the lower triangle, zero everything else (what k_dd_lp_schur<true> leaves)
+__global__ void k_dd_keep_own_lower(int n, dd* __restrict__ H, int rank, int world, int pw) {
+    const int j = blockIdx.y, i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n && (i < j || (i / pw) % world != rank)) H[(size_t)j * n + i] = dd_make(0.0);
 }
 // sharded H: the diagonal entries of the rank's own row blocks only
 __global__ void k_dd_shift_own_diag(int n, dd* __restrict__ H, double delta, int rank, int world, int pw) {
@@ -507,7 +514,7 @@ int32_t lrn_dd_create(lrn_dd_handle_t* out, int64_t n_var, int64_t nlin, int32_t
         int per_sm = 0, coop = 0;
         LRN_CUDA(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, h->device));
         LRN_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_dd_trsv_multi, TRSV_T, 0));
-        h->trsv_ctas = (coop && per_sm > 0) ? std::min(prop.multiProcessorCount, 128) : 0;
+        h->trsv_ctas = h->trsv_ctas_max = (coop && per_sm > 0) ? std::min(prop.multiProcessorCount, 128) : 0;
         return LRN_OK;
     });
     if (rc != LRN_OK) {
@@ -806,8 +813,9 @@ int32_t lrn_dd_rhs_corrector(lrn_dd_handle_t h, const double sigma[2], const dou
 int32_t lrn_dd_schur_solve(lrn_dd_handle_t h, int32_t which) {
     LRN_GROUP(h, lrn_dd_schur_solve(m_, which));
     return guarded(h, [&]() -> int32_t {
-        LRN_REQUIRE(h->have_factor, "lrn_dd_schur_factor first");
         LRN_REQUIRE(which == 3 || which == 6, "which must be 3 or 6");
+        // a call-order error, not a bad argument: no factor, or the last factorisation failed
+        if (!h->have_factor) throw std::runtime_error("no valid Cholesky factor (lrn_dd_schur_factor first, and it must return 0)");
         Timed t(h, 2);
         LRN_CUDA(cudaMemcpyAsync(h->dely.p, h->rhs.p, (size_t)h->n * sizeof(dd), cudaMemcpyDeviceToDevice, h->st));
         for (int rep = 0; rep < (which == 6 ? 2 : 1); rep++) {
@@ -940,6 +948,38 @@ int32_t lrn_dd_timers(lrn_dd_handle_t h, double ms[4], int32_t reset) {
         for (int k = 0; k < 4; k++) { ms[k] = h->t_ms[k]; if (reset) h->t_ms[k] = 0.0; }
         return LRN_OK;
     });
+}
+
+// ---- test hooks (loraine_b200_debug.h) -----------------------------------------------------------------------------------
+int32_t lrn_dd_dbg_set_array(lrn_dd_handle_t h, int32_t which, const double* hi, const double* lo) {
+    if (which != 1 && which != 5) return LRN_ERR_ARG;
+    LRN_GROUP(h, lrn_dd_dbg_set_array(m_, which, hi, lo));
+    return guarded(h, [&]() -> int32_t {
+        LRN_REQUIRE(hi, "null argument");
+        const int n = h->n;
+        if (which == 5) {
+            upload_dd(h, h->rhs, hi, lo, (size_t)n);
+            return LRN_OK;
+        }
+        upload_dd(h, h->H, hi, lo, (size_t)n * n);
+        if (dd_sharded(h)) {
+            k_dd_keep_own_lower<<<dim3(nblk(n), (unsigned)n), TB, 0, h->st>>>(n, h->H.p, h->rank, h->world, h->pw);
+            LRN_CHECK_LAUNCH();
+            LRN_CUDA(cudaStreamSynchronize(h->st));
+        }
+        h->H_gathered = false;
+        h->have_H = true;
+        h->have_factor = false;
+        return LRN_OK;
+    });
+}
+
+int32_t lrn_dd_dbg_set_trsv_ctas(lrn_dd_handle_t h, int32_t ctas) {
+    if (ctas < -1) return LRN_ERR_ARG;
+    LRN_GROUP(h, lrn_dd_dbg_set_trsv_ctas(m_, ctas));
+    if (!h) return LRN_ERR_ARG;
+    h->trsv_ctas = ctas < 0 ? h->trsv_ctas_max : std::min(ctas, h->trsv_ctas_max);
+    return LRN_OK;
 }
 
 }  // extern "C"

@@ -21,7 +21,7 @@ struct lrn_dd_solver {
     lrn::DevBuf<lrn::dd> d, b, x, s, si, y, rp, rd, rhs, dely, dx, ds, xn, sn, rnt, w, tl, tn;
     lrn::DevBuf<lrn::dd> H, L, red, rdiag;
     lrn::DevBuf<int> info, flags;      // info[0]: Cholesky pivot, info[1]: time-out of the flag wait in the multi-CTA solves
-    int trsv_ctas = 0, trsv_epoch = 0;
+    int trsv_ctas = 0, trsv_ctas_max = 0, trsv_epoch = 0;     // (trsv_ctas_max: the lrn_dd_create value)
     bool have_lin = false, have_b = false, finalized = false, have_iterate = false, have_H = false, have_factor = false;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     double t_ms[4] = {0, 0, 0, 0};
