@@ -56,6 +56,10 @@ typedef struct lrn_options {
 void lrn_default_options(lrn_options_t* opt);
 
 /* ---- construction: replaces MyModel / MySolver storage (src/model.jl:34-87, src/Solvers.jl:18-147, :363-446) ---- */
+/* Limits on n_var: kit = 0 forms the dense n_var x n_var Schur matrix and its factor, so 1 <= n_var <= 140 000
+ * (LRN_ERR_ARG "n_var out of range (1..140000)").  kit = 1 forms neither: 1 <= n_var <= 2^31 - 1, and lrn_finalize returns
+ * LRN_ERR_ARG, naming the bytes needed and the bytes free, when the CG state does not fit the device's free memory.  With an
+ * LP block and n_var > 140 000, lrn_prec_prepare(h, 1) (H_alpha) returns LRN_ERR_UNSUPPORTED; kinds 2 and 4 run. */
 int32_t lrn_create(lrn_handle_t* out, int64_t n_var, int64_t nlmi, const int64_t* msizes, int64_t nlin,
                    const lrn_options_t* opt);
 /* AA[i] (n_var x m_i^2, row k = vec(calA_{i,k}), math sign), as built by prep_AA! (src/model.jl:199-229) */

@@ -64,6 +64,12 @@ int32_t lrn_dd_dbg_set_array(lrn_dd_handle_t h, int32_t which, const double* hi,
  * -1 = the value lrn_dd_create chose, >= 1 = that many, clamped to the lrn_dd_create value (every CTA must stay resident:
  * the CTAs wait on each other's results).  Fewer CTAs than row tiles make one CTA solve several tiles. */
 int32_t lrn_dd_dbg_set_trsv_ctas(lrn_dd_handle_t h, int32_t ctas);
+/* test hook for the kit = 1 H_alpha preconditioner, whose build forms T (n_var x erank sum m_i) and A_j u_r (n_var x max m_i)
+ * `rows` rows at a time: set_rows > 0 forces that slab height (clamped to n_var; 1 and odd heights are allowed), 0 restores the
+ * automatic height (n_var when both whole arrays fit 2 GiB, otherwise the largest multiple of 8 that does).  *rows_used
+ * (optional) receives the height the last lrn_prec_prepare(h, 1) used (0 before the first).  A lrn_create_multi handle sets
+ * every member and reports member 0. */
+int32_t lrn_dbg_prec_slab(lrn_handle_t h, int64_t set_rows, int64_t* rows_used);
 /* relative Frobenius distance ||A_a - A_b||_F / ||A_b||_F over the LOWER triangles of the n_var x n_var Schur matrices
  * (which = LRN_ARR_H) or Cholesky factors (LRN_ARR_L) of two handles living on the same device; computed on the device
  * (bench.py's dist_parity: sharded handle against a single-GPU handle at n_var = 40000 without a 12.8 GB download) */

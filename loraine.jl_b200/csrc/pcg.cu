@@ -6,6 +6,7 @@
 // The whole recurrence keeps its scalars on the device; the host reads one residual norm per iteration.
 #include "solver.cuh"
 #include "group.cuh"
+#include "../../include/loraine_b200_debug.h"
 #include <algorithm>
 #include <cmath>
 
@@ -48,14 +49,16 @@ __global__ void k_set_diag(int n, double* A, int lda, const double* d) {
     int i = blockIdx.x * TBK + threadIdx.x;
     if (i < n) A[(size_t)i * lda + i] = d[i];
 }
-// AU[j,p] = rowscale[j] * sum_q calA_j[p,q] U[q]        (prec_alpha_S!, src/Solvers.jl:833-841)
-__global__ void k_build_AU(int n_var, const int* __restrict__ rowptr, const int* __restrict__ ep, const int* __restrict__ eq,
+// AU[j - r0, p] = rowscale[j] * sum_q calA_j[p,q] U[q] for the constraints j of the slab [r0, r0 + rows)
+//                                                        (prec_alpha_S!, src/Solvers.jl:833-841)
+__global__ void k_build_AU(int r0, int rows, const int* __restrict__ rowptr, const int* __restrict__ ep, const int* __restrict__ eq,
                            const double* __restrict__ ev, const double* __restrict__ U, const double* __restrict__ rowscale,
                            double* __restrict__ AU, int ld) {
-    int j = blockIdx.x * TBK + threadIdx.x;
-    if (j >= n_var) return;
+    const int i = blockIdx.x * TBK + threadIdx.x;
+    if (i >= rows) return;
+    const int j = r0 + i;
     const double sc = rowscale ? rowscale[j] : 1.0;
-    for (int e = rowptr[j]; e < rowptr[j + 1]; e++) AU[(size_t)ep[e] * ld + j] += sc * ev[e] * U[eq[e]];
+    for (int e = rowptr[j]; e < rowptr[j + 1]; e++) AU[(size_t)ep[e] * ld + i] += sc * ev[e] * U[eq[e]];
 }
 // Thin products of the H_alpha apply (k = erank <= 8 columns): the DMMA tiles would be 1/64 full, these are plain
 // bandwidth-bound kernels instead.
@@ -207,13 +210,11 @@ int32_t prec_alpha(lrn_solver* h) {
     if (!h->pDiag.p) { h->pDiag.alloc(n); h->pDsq.alloc(n); }
     int kS = 0, maxm = 1;
     for (auto& B : h->blk) { kS += k * B.m; maxm = std::max(maxm, B.m); }
-    const int ldt = pad_ld(n);
-    if (h->kS != kS || !h->pT.p) {
+    if (h->kS != kS || !h->pS.p) {
         h->kS = kS;
-        h->pT.alloc((size_t)ldt * kS);
         h->pS.alloc((size_t)pad_ld(kS) * kS);
         h->pY.alloc(kS);
-        h->pAU.alloc((size_t)ldt * maxm);
+        h->pYw.alloc(kS);
     }
     double shift = 0.0;
     std::vector<double> tv, sc(k);
@@ -256,21 +257,32 @@ int32_t prec_alpha(lrn_solver* h) {
     vec_op(st, n, VEC_RSQRT, h->pDsq.p, h->pDiag.p, nullptr);
     // t = [AA_i kron(U_i, Z_i)]_i ; fast formula scales rows by diag(AAAATtau)^{-1/2}   (src/Solvers.jl:752-801, :819-864)
     const bool fast = (!h->pDense) || k == 1;
-    int off = 0;
-    for (auto& B : h->blk) {
-        const int m = B.m;
-        for (int r = 0; r < k; r++) {
-            LRN_CUDA(cudaMemsetAsync(h->pAU.p, 0, (size_t)ldt * m * sizeof(double), st));
-            k_build_AU<<<nb(n), TBK, 0, st>>>(n, B.sp.rowptr.p, B.sp.ep.p, B.sp.eq.p, B.sp.ev.p, B.U.p() + (size_t)r * B.U.ld,
-                                              fast ? h->pDsq.p : nullptr, h->pAU.p, ldt);
-            gemm_nn(st, n, m, m, 1.0, h->pAU.p, ldt, B.Zf.p(), B.ld, 0.0, h->pT.p + (size_t)(off + r * m) * ldt, ldt);
-        }
-        off += k * m;
+    // The fast formula needs T only through S = T'T, so T and A_j u_r are built `R` rows at a time and S accumulates the slab
+    // products.  The other formula needs whole columns of T (only reachable with an LP block, i.e. below KIT0_MAX_NVAR).
+    const int R = fast ? prec_slab_rows(n, kS, maxm, h->slab_force) : n;
+    const int ldt = pad_ld(R);
+    if (h->slab_rows != R || h->pT.n != (size_t)ldt * kS) {
+        h->pT.alloc((size_t)ldt * kS);
+        h->pAU.alloc((size_t)ldt * maxm);
+        h->slab_rows = R;
     }
     const int lds = pad_ld(kS);
-    if (fast) {
-        gemm_tn(st, kS, kS, n, 1.0, h->pT.p, ldt, h->pT.p, ldt, 0.0, h->pS.p, lds);
-    } else {
+    for (int r0 = 0; r0 < n; r0 += R) {
+        const int rows = std::min(R, n - r0);
+        int off = 0;
+        for (auto& B : h->blk) {
+            const int m = B.m;
+            for (int r = 0; r < k; r++) {
+                LRN_CUDA(cudaMemsetAsync(h->pAU.p, 0, (size_t)ldt * m * sizeof(double), st));
+                k_build_AU<<<nb(rows), TBK, 0, st>>>(r0, rows, B.sp.rowptr.p, B.sp.ep.p, B.sp.eq.p, B.sp.ev.p,
+                                                     B.U.p() + (size_t)r * B.U.ld, fast ? h->pDsq.p : nullptr, h->pAU.p, ldt);
+                gemm_nn(st, rows, m, m, 1.0, h->pAU.p, ldt, B.Zf.p(), B.ld, 0.0, h->pT.p + (size_t)(off + r * m) * ldt, ldt);
+            }
+            off += k * m;
+        }
+        if (fast) gemm_tn(st, kS, kS, rows, 1.0, h->pT.p, ldt, h->pT.p, ldt, r0 > 0 ? 1.0 : 0.0, h->pS.p, lds);
+    }
+    if (!fast) {
         // S = t' * (AAAATtau \ t), column by column (only for erank > 1 together with an LP block)
         DevBuf<double> DT((size_t)ldt * kS);
         for (int c = 0; c < kS; c++) d_solve(h, h->pT.p + (size_t)c * ldt, DT.p + (size_t)c * ldt);
@@ -308,8 +320,7 @@ void apply_alpha(lrn_solver* h, const double* x, double* out) {
         AtB_thin(st, B.Zf.p(), ld, m, m, B.MU.p(), B.MU.ld, k, h->pY.p + off, m);
         off += k * m;
     }
-    chol_solve(h->pS.p, h->kS, pad_ld(h->kS), h->cholS, h->pY.p, h->pT.p /* scratch: t is only needed while S is being built */,
-               3, st);
+    chol_solve(h->pS.p, h->kS, pad_ld(h->kS), h->cholS, h->pY.p, h->pYw.p, 3, st);
     double* yy2 = h->cg_Ap.p;     // free while the preconditioner runs
     LRN_CUDA(cudaMemsetAsync(yy2, 0, n * sizeof(double), st));
     off = 0;
@@ -338,12 +349,32 @@ void ensure_cg(lrn_solver* h) {
 
 }  // namespace
 
+namespace lrn {
+// Above this many bytes for the whole T and A_j u_r the H_alpha build runs in row slabs.
+constexpr size_t PREC_SLAB_BUDGET = (size_t)2 << 30;
+
+size_t prec_slab_bytes(int rows, int kS, int maxm) { return (size_t)pad_ld(rows) * ((size_t)kS + (size_t)maxm) * sizeof(double); }
+
+int prec_slab_rows(int n_var, int kS, int maxm, int64_t force) {
+    if (force > 0) return (int)std::min<int64_t>(force, n_var);
+    if (prec_slab_bytes(n_var, kS, maxm) <= PREC_SLAB_BUDGET) return n_var;
+    const size_t per_row = ((size_t)kS + (size_t)maxm) * sizeof(double);
+    const size_t R = (PREC_SLAB_BUDGET / per_row) & ~(size_t)7;
+    return (int)std::max<size_t>(R, 8);
+}
+}  // namespace lrn
+
 extern "C" {
 
 int32_t lrn_prec_prepare(lrn_handle_t h, int32_t kind) {
     LRN_GROUP(h, lrn_prec_prepare(m_, kind));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(h->finalized && h->nlmi > 0, "preconditioners need at least one PSD block");
+        if (kind == 1 && h->nlin > 0 && h->n_var > KIT0_MAX_NVAR) {
+            h->err = "H_alpha with an LP block forms the dense n_var x n_var matrix AAAATtau and factors it; above n_var = " +
+                     std::to_string(KIT0_MAX_NVAR) + " it does not fit one GPU (use preconditioner 2, H_beta, which needs only its diagonal)";
+            return LRN_ERR_UNSUPPORTED;
+        }
         PhaseT ph(h, LRN_T_PREC);
         for (auto& Bk : h->blk) Bk.ud_valid = false;
         ensure_cg(h);
@@ -471,6 +502,21 @@ int32_t lrn_apply_operator(lrn_handle_t h, int32_t kind, const double* x, double
         LRN_CUDA(cudaStreamSynchronize(st));
         return LRN_OK;
     });
+}
+
+int32_t lrn_dbg_prec_slab(lrn_handle_t h, int64_t set_rows, int64_t* rows_used) {
+    if (h && h->group) {
+        Group* g = static_cast<Group*>(h->group);
+        for (auto* m : g->members) {
+            const int32_t rc = lrn_dbg_prec_slab(m, set_rows, nullptr);
+            if (rc != LRN_OK) return rc;
+        }
+        return lrn_dbg_prec_slab(g->members[0], set_rows, rows_used);
+    }
+    if (!h || set_rows < 0) return LRN_ERR_ARG;
+    h->slab_force = set_rows;
+    if (rows_used) *rows_used = h->slab_rows;
+    return LRN_OK;
 }
 
 }  // extern "C"

@@ -252,7 +252,7 @@ void build_block(lrn_solver* h, Block& B) {
         }
     }
     sp.nF1 = nF1;
-    sp_build_pair_plan(sp, rowptr, ep, eq, ev, h->st);      // staged pair kernel when every matrix goes through the F3 formula
+    if (h->opt.kit == 0) sp_build_pair_plan(sp, rowptr, ep, eq, ev, h->st);   // staged pair kernel of the Schur assembly
     sp.h_rowptr = rowptr;
     sp.h_part = part;
     sp.rowptr.upload(rowptr, h->st); sp.ep.upload(ep, h->st); sp.eq.upload(eq, h->st); sp.ev.upload(ev, h->st);
@@ -480,8 +480,10 @@ int32_t lrn_create(lrn_handle_t* out, int64_t n_var, int64_t nlmi, const int64_t
             h->err = "loraine_b200 requires an sm_100 (Blackwell) GPU; there is no fallback path";
             return LRN_ERR_NO_DEVICE;
         }
-        // the Schur matrix and its factor are dense n_var x n_var FP64 (2 x 8 n_var^2 bytes): 140 000 is what 180 GB of HBM holds
-        LRN_REQUIRE(n_var >= 1 && n_var <= 140000, "n_var out of range (1..140000)");
+        // kit = 0: the Schur matrix and its factor are dense n_var x n_var FP64 (2 x 8 n_var^2 bytes): 140 000 is what 180 GB
+        // of HBM holds.  kit = 1 forms neither; its limit is the device memory lrn_finalize checks (indices stay int).
+        if (h->opt.kit == 1) LRN_REQUIRE(n_var >= 1 && n_var <= INT32_MAX, "n_var out of range (1..2147483647 for kit = 1)");
+        else LRN_REQUIRE(n_var >= 1 && n_var <= KIT0_MAX_NVAR, "n_var out of range (1..140000)");
         LRN_REQUIRE(nlmi >= 0 && nlin >= 0 && nlin < 2000000000LL, "nlmi/nlin out of range");
         LRN_REQUIRE(nlmi == 0 || msizes, "msizes is null");
         h->n_var = (int)n_var; h->nlmi = (int)nlmi; h->nlin = (int)nlin;
@@ -553,11 +555,43 @@ int32_t lrn_set_b(lrn_handle_t h, const double* b) {
     });
 }
 
+// Device bytes of the kit = 1 state, from the staged model: model data, the n_var-long vectors, the m x m block arrays, and
+// for H_alpha the kS x kS matrix S and one slab of its row-slab build (the dense AAAATtau of an LP block below KIT0_MAX_NVAR).
+static size_t cg_footprint(const lrn_solver* h) {
+    const size_t n = (size_t)h->n_var, d = sizeof(double), ix = sizeof(int);
+    size_t bytes = 14 * n * d;                                    // y, dely, rhs, Rp, tn1, tn2, ones, b, 4 CG vectors, pDiag, pDsq
+    int kS = 0, maxm = 1;
+    for (const auto& B : h->blk) {
+        const size_t nnz = B.hAA.rowval.size(), nnzB = B.hB.rowval.size(), mm = (size_t)pad_ld(B.m) * B.m;
+        bytes += nnz * (3 * ix + 3 * d) + nnz * (3 * ix + d);     // by-constraint (p, q, v, values), by-position lists
+        bytes += 2 * (n + 1) * ix + nnzB * (ix + d);              // row pointers, constraint order, rank-one factors
+        bytes += 24 * mm * d;                                     // X, S, W, G, ... T1-T4, C, Z, work of the m x m kernels
+        kS += h->opt.erank * B.m;
+        maxm = std::max(maxm, B.m);
+    }
+    if (h->nlin > 0) bytes += 2 * h->hClin.rowval.size() * (ix + d) + (n + h->nlin + 2) * ix + 12 * (size_t)h->nlin * d;
+    if (h->opt.preconditioner == 1 || h->opt.preconditioner == 4) {
+        bytes += ((size_t)pad_ld(kS) * kS + 2 * (size_t)kS) * d;
+        bytes += prec_slab_bytes(prec_slab_rows(h->n_var, kS, maxm, h->slab_force), kS, maxm);
+        if (h->nlin > 0 && h->n_var <= KIT0_MAX_NVAR) bytes += (size_t)pad_ld(h->n_var) * n * d;
+    }
+    return bytes;
+}
+
 int32_t lrn_finalize(lrn_handle_t h) {
     LRN_GROUP(h, lrn_finalize(m_));
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(!h->finalized, "already finalized");
         LRN_REQUIRE(h->b.p, "lrn_set_b was not called");
+        if (h->opt.kit == 1) {
+            // refuse a model whose CG state cannot fit before anything is allocated, instead of failing partway through a solve
+            size_t free_b = 0, total_b = 0;
+            LRN_CUDA(cudaMemGetInfo(&free_b, &total_b));
+            const size_t need = cg_footprint(h);
+            if (need > free_b)
+                throw std::invalid_argument("kit = 1 state needs " + std::to_string(need) + " bytes of device memory, " +
+                                            std::to_string(free_b) + " bytes are free");
+        }
         const int n = h->n_var;
         int maxm = 1;
         record_model_norms(h, h->hb);          // norms of AA_i, b, C_lin rows for lrn_initial_point (host copies still exist)

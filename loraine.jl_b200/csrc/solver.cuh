@@ -52,6 +52,15 @@ struct PhaseEvt {
     int phase;
 };
 
+// Largest n_var of the direct (kit = 0) path: its Schur matrix and factor are dense n_var x n_var FP64 (2 x 8 n_var^2 bytes),
+// and 140 000 is what 180 GB of HBM holds.  The CG path (kit = 1) forms neither.
+constexpr int64_t KIT0_MAX_NVAR = 140000;
+// Row-slab height of the H_alpha build (pcg.cu): n_var when the whole T (n_var x kS) and A_j u_r (n_var x maxm) fit the slab
+// budget, otherwise the largest multiple of 8 that does; force > 0 is used as given (clamped to n_var).
+int prec_slab_rows(int n_var, int kS, int maxm, int64_t force);
+// device bytes of one slab pair (T and A_j u_r) of height `rows`
+size_t prec_slab_bytes(int rows, int kS, int maxm);
+
 }  // namespace lrn
 
 struct lrn_solver {
@@ -104,11 +113,15 @@ struct lrn_solver {
     long long stat_svd_sweeps = 0, stat_lanczos_iters = 0, stat_lanczos_fail = 0;
     // CG / preconditioner state
     lrn::DevBuf<double> cg_r, cg_z, cg_p, cg_Ap, cg_scal;
-    lrn::DevBuf<double> pDiag, pDsq, pT, pS, pY, pAU;
+    lrn::DevBuf<double> pDiag, pDsq, pT, pS, pY, pYw, pAU;
     lrn::DMat pDd;                     // dense AAAATtau when nlin > 0
     lrn::CholWork cholS, cholD;
     bool pDense = false;
     int kS = 0;
+    // H_alpha build in row slabs: pT (pad_ld(slab_rows) x kS) and pAU (pad_ld(slab_rows) x max m) hold slab_rows rows of T
+    // and of A_j u_r
+    int slab_rows = 0;
+    int64_t slab_force = 0;            // debug hook: forced slab height (0 = automatic)
     int prec_ready = 0;                // kind prepared (0 none)
     // distributed
     int rank = 0, world = 1;

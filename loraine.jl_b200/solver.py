@@ -115,6 +115,8 @@ class MySolver:
     def get_array(self, name, iblk=0):
         md = self.model
         which = _lib.ARR[name]
+        if which in (1, 2) and self.kit != 0:      # before allocating an n x n host array: kit = 1 has no Schur matrix
+            raise LoraineB200Error(f"{name} (the Schur matrix or its factor) exists only for kit = 0")
         if which < 10:
             shape = (md.n, md.n) if which in (1, 2) else (md.n,)
         elif which in (14, 15):
