@@ -19,6 +19,15 @@ int32_t lrn_dbg_gemm(int32_t M, int32_t N, int32_t K, int32_t transA, int32_t tr
                      int32_t misalign, int32_t reps, double* ms_per_launch);
 /* A (n x n, symmetric, lower used) -> L in the lower triangle (upper zeroed); x (n) <- solve per `which` (0 = skip) */
 int32_t lrn_dbg_cholesky(int32_t n, double* A, double* x, int32_t which, int32_t* info, int32_t reps, double* ms_factor);
+/* trailing updates of lrn_dbg_cholesky: 0 = DMMA (default), 1 = Ozaki INT8 products when the panels are 1024 wide (n >= 16384;
+ * the Schur factor's default, off under LRN_CHOL_INT8=0), 2 = Ozaki INT8 products at every panel width (n >= 1024) */
+int32_t lrn_dbg_chol_int8(int32_t mode);
+/* the Ozaki INT8 product alone: P (rows x K, K <= 1024) is sliced into digit planes and C (M x N) -= P[a_row0 + i, :] P[b_row0 + j, :]^T
+ * (a_row0, b_row0 multiples of 8; rows beyond `rows` read as zero).  lower != 0: only 128 x 64 tiles that meet the lower triangle
+ * of a symmetric matrix in which C(0, 0) sits at (row0, col0).  sigma (optional, rows) receives the row scales.  reps > 0: the
+ * update is timed over `reps` further launches (they keep subtracting from the device copy of C) into *ms_per_launch. */
+int32_t lrn_dbg_syrk_i8(int32_t rows, int32_t K, const double* P, int32_t a_row0, int32_t b_row0, int32_t M, int32_t N, int64_t row0,
+                        int64_t col0, int32_t lower, double* C, double* sigma, int32_t reps, double* ms_per_launch);
 /* symmetric n <= 64: eigenvalues (descending) and eigenvectors */
 int32_t lrn_dbg_eig_small(int32_t n, const double* A, double* evals, double* V, int32_t relative);
 /* one-sided block Jacobi SVD of the m x m matrix A: UD = U*diag(sigma), V (NULL: not accumulated), sigma (descending) */

@@ -80,6 +80,8 @@ def lib():
         "lrn_dbg_model_block": (i64, [i64, i64, pi64, i64, pi64, pi64, pi64, pi64, pdbl, pdbl, i32, i64, i32, i64, pi64, pi64, pdbl,
                                       pdbl]),
         "lrn_dbg_compare": (i32, [vp, vp, i32, pdbl]),
+        "lrn_dbg_chol_int8": (i32, [i32]),
+        "lrn_dbg_syrk_i8": (i32, [i32, i32, pdbl, i32, i32, i32, i32, i64, i64, i32, pdbl, pdbl, i32, pdbl]),
         "lrn_dbg_gather_H": (i32, [vp]),
         "lrn_dist_unique_id": (i32, [C.c_char_p]),
         "lrn_dist_init": (i32, [vp, i32, i32, C.c_char_p]),
@@ -136,4 +138,5 @@ DD_ARR = dict(H=1, L=2, RP=3, RD=4, RHS=5, DELY=6, DELX=7, DELS=8, XN=9, SN=10, 
 
 DEBUG_SYMBOLS = ["lrn_dbg_gemm", "lrn_dbg_cholesky", "lrn_dbg_eig_small", "lrn_dbg_svd", "lrn_dbg_lanczos",
                  "lrn_dbg_batched_lambda_min", "lrn_dbg_peak", "lrn_dbg_gemm_profile", "lrn_dbg_set_shard", "lrn_dbg_compare",
-                 "lrn_dbg_gather_H", "lrn_dbg_model_block", "lrn_dd_dbg_set_shard", "lrn_dbg_prec_slab"]
+                 "lrn_dbg_gather_H", "lrn_dbg_model_block", "lrn_dd_dbg_set_shard", "lrn_dbg_prec_slab",
+                 "lrn_dbg_chol_int8", "lrn_dbg_syrk_i8"]

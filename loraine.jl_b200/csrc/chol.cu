@@ -723,6 +723,18 @@ void chol_lookahead(double* A, int n, int lda, CholWork& work, cudaStream_t st) 
     cudaEvent_t evStart = work.ev[0], evP[2] = {work.ev[1], work.ev[2]}, evR[2] = {work.ev[3], work.ev[4]};
     int* info = work.info_ptr();
     const int NB = pick_nb(n), npan = (int)cdiv(n, NB), gcap = panel_grid_cap(n);
+    // the two trailing-update products of a panel run as Ozaki INT8 products (chol_i8.cu) when the caller opted in: the solved
+    // panel is sliced into digit planes once, on the panel stream, and both products read the planes
+    static const bool env_off = [] { const char* e = getenv("LRN_CHOL_INT8"); return e && atoi(e) == 0; }();
+    const bool i8 = n > NB && (work.int8 == 2 || (work.int8 == 1 && NB == 1024 && !env_off));
+    const auto slice_rows = [](int rows) { return round_up(rows, 128) + 128; };   // room for the 128-row tiles at row offset wq
+    if (i8) {
+        const int r0 = slice_rows(n - NB);
+        for (int b = 0; b < 2; b++) {
+            if (work.i8_slices[b].n < i8_slice_bytes(r0, NB)) work.i8_slices[b].alloc(i8_slice_bytes(r0, NB));
+            if (work.i8_sigma[b].n < (size_t)r0) work.i8_sigma[b].alloc((size_t)r0);
+        }
+    }
     LRN_CUDA(cudaEventRecord(evStart, st));
     LRN_CUDA(cudaStreamWaitEvent(sp, evStart, 0));
     int last = 0;
@@ -731,26 +743,37 @@ void chol_lookahead(double* A, int n, int lda, CholWork& work, cudaStream_t st) 
         double* Ap = A + (size_t)c0 * lda + c0;
         double* dk = work.dinv.p + (size_t)(c0 / DB) * DB * DB;
         factor_panel(Ap, w, rows - w, lda, dk, info, c0, gcap, sp);
+        const int q0 = c0 + w;
+        const double* P = Ap + w;                                           // rows below the diagonal block, lda
+        // set p & 1 was last read by the products of panel p - 2; the next-columns update of panel p - 1, which precedes this
+        // slicing on the panel stream, waited for rest(p - 2)
+        const int rpad = slice_rows(n - q0);
+        int8_t* sl = work.i8_slices[p & 1].p;
+        const double* sg = work.i8_sigma[p & 1].p;
+        if (i8 && q0 < n) i8_slice(P, lda, n - q0, w, rpad, sl, work.i8_sigma[p & 1].p, sp);
         LRN_CUDA(cudaEventRecord(evP[p & 1], sp));
         last = p & 1;
-        const int q0 = c0 + w;
         if (q0 >= n) break;
         const int wq = (n - q0 < NB) ? (n - q0) : NB;
-        const double* P = Ap + w;                                           // rows below the diagonal block, lda
         const int q1 = q0 + wq;
         // rest of the trailing matrix (lower triangle, columns behind the next panel) on the main stream
         LRN_CUDA(cudaStreamWaitEvent(st, evP[p & 1], 0));
         if (q1 < n) {
-            GemmParams g;
-            g.A = P + wq; g.B = P + wq; g.C = A + (size_t)q1 * lda + q1;
-            g.M = n - q1; g.N = n - q1; g.K = w; g.lda = lda; g.ldb = lda; g.ldc = lda;
-            g.transB = true; g.alpha = -1.0; g.beta = 1.0; g.lower = 1;
-            gemm(g, st);
+            if (i8) {
+                syrk_update_i8(sl, sg, rpad, w, wq, wq, n - q1, n - q1, A + (size_t)q1 * lda + q1, lda, 0, 0, true, st);
+            } else {
+                GemmParams g;
+                g.A = P + wq; g.B = P + wq; g.C = A + (size_t)q1 * lda + q1;
+                g.M = n - q1; g.N = n - q1; g.K = w; g.lda = lda; g.ldb = lda; g.ldc = lda;
+                g.transB = true; g.alpha = -1.0; g.beta = 1.0; g.lower = 1;
+                gemm(g, st);
+            }
         }
         LRN_CUDA(cudaEventRecord(evR[p & 1], st));
         // the next panel's columns on the panel stream (they also received rest(p-1), which must have completed)
         if (p >= 1) LRN_CUDA(cudaStreamWaitEvent(sp, evR[(p - 1) & 1], 0));
-        gemm_nt(sp, n - q0, wq, w, -1.0, P, lda, P, lda, 1.0, A + (size_t)q0 * lda + q0, lda);
+        if (i8) syrk_update_i8(sl, sg, rpad, w, 0, 0, n - q0, wq, A + (size_t)q0 * lda + q0, lda, 0, 0, true, sp);
+        else gemm_nt(sp, n - q0, wq, w, -1.0, P, lda, P, lda, 1.0, A + (size_t)q0 * lda + q0, lda);
     }
     LRN_CUDA(cudaStreamWaitEvent(st, evP[last], 0));
 }

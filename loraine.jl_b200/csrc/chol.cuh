@@ -27,6 +27,13 @@ struct CholWork {
     cudaStream_t aux = nullptr;   // high-priority side stream (panel factorisation + broadcast look-ahead in multi-GPU runs)
     cudaStream_t aux2 = nullptr;  // second high-priority stream (distributed path: early factorisation of the next diagonal block)
     cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    // trailing updates as Ozaki INT8 products (chol_i8.cu): 0 never (DMMA), 1 when the panels are 1024 wide (n >= 16384) unless the
+    // environment sets LRN_CHOL_INT8=0, 2 at every panel width (tests).  Only the Schur factor opts in.
+    int int8 = 0;
+    // digit planes + row scales of the solved panel, two sets: panel p + 1 is sliced while the rest update of panel p still
+    // reads panel p's set
+    DevBuf<int8_t> i8_slices[2];
+    DevBuf<double> i8_sigma[2];
     int n = 0;
     void ensure(int n_) {
         if (n_ > n || !dinv.p) { dinv.alloc((size_t)cdiv(n_, CHOL_DB) * CHOL_DB * CHOL_DB); n = n_; }
@@ -57,5 +64,17 @@ void trsm_left_lower_trans(const double* L, int n, int lda, const CholWork& work
 
 // Zero the strict upper triangle (so the factor can be used as a dense GEMM operand).
 void zero_strict_upper(double* A, int n, int lda, cudaStream_t st);
+
+// ---- Ozaki INT8 products (chol_i8.cu) ----
+// bytes of the digit planes of rows_pad rows x K columns
+size_t i8_slice_bytes(int rows_pad, int K);
+// slice P (rows x K, leading dimension ldp, 1 <= K <= 1024) into 8 int8 digit planes and per-row power-of-two scales sigma;
+// rows [rows, rows_pad) get zero digits and sigma 0 (rows_pad % 8 == 0)
+void i8_slice(const double* P, int ldp, int rows, int K, int rows_pad, int8_t* slices, double* sigma, cudaStream_t st);
+// C (M x N, ldc) -= P[a_row0 + i, :] P[b_row0 + j, :]^T from the slices (a_row0, b_row0 multiples of 8).  lower: only tiles
+// (128 x 64) that meet the lower triangle, with (row0, col0) the position of C(0, 0) in the symmetric matrix; entries above the
+// diagonal inside such tiles are updated too (don't-care for the factorisation)
+void syrk_update_i8(const int8_t* slices, const double* sigma, int rows_pad, int K, int a_row0, int b_row0, int M, int N, double* C,
+                    int ldc, long long row0, long long col0, bool lower, cudaStream_t st);
 
 }  // namespace lrn

@@ -113,10 +113,49 @@ int32_t lrn_dbg_gemm(int32_t M, int32_t N, int32_t K, int32_t transA, int32_t tr
     });
 }
 
+static int g_dbg_chol_int8 = 0;
+
+int32_t lrn_dbg_chol_int8(int32_t mode) {
+    if (mode < 0 || mode > 2) return LRN_ERR_ARG;
+    g_dbg_chol_int8 = mode;
+    return LRN_OK;
+}
+
+int32_t lrn_dbg_syrk_i8(int32_t rows, int32_t K, const double* P, int32_t a_row0, int32_t b_row0, int32_t M, int32_t N, int64_t row0,
+                        int64_t col0, int32_t lower, double* C, double* sigma, int32_t reps, double* ms_per_launch) {
+    return guard([&]() -> int32_t {
+        HostMat dP(P, rows, K), dC(C, M, N);
+        const int rows_pad = round_up(std::max(rows, std::max(a_row0 + round_up(M, 128), b_row0 + round_up(N, 64))), 8);
+        DevBuf<int8_t> sl(i8_slice_bytes(rows_pad, K));
+        DevBuf<double> sg(rows_pad);
+        cudaStream_t st = 0;
+        i8_slice(dP.p, dP.ld, rows, K, rows_pad, sl.p, sg.p, st);
+        syrk_update_i8(sl.p, sg.p, rows_pad, K, a_row0, b_row0, M, N, dC.p, dC.ld, row0, col0, lower != 0, st);
+        LRN_CUDA(cudaDeviceSynchronize());
+        dC.download(C);
+        if (sigma) LRN_CUDA(cudaMemcpy(sigma, sg.p, (size_t)rows * sizeof(double), cudaMemcpyDeviceToHost));
+        if (reps > 0 && ms_per_launch) {
+            cudaEvent_t e0, e1;
+            LRN_CUDA(cudaEventCreate(&e0)); LRN_CUDA(cudaEventCreate(&e1));
+            for (int r = 0; r < 2; r++) syrk_update_i8(sl.p, sg.p, rows_pad, K, a_row0, b_row0, M, N, dC.p, dC.ld, row0, col0, lower != 0, st);
+            LRN_CUDA(cudaEventRecord(e0, st));
+            for (int r = 0; r < reps; r++) syrk_update_i8(sl.p, sg.p, rows_pad, K, a_row0, b_row0, M, N, dC.p, dC.ld, row0, col0, lower != 0, st);
+            LRN_CUDA(cudaEventRecord(e1, st));
+            LRN_CUDA(cudaEventSynchronize(e1));
+            float ms = 0;
+            LRN_CUDA(cudaEventElapsedTime(&ms, e0, e1));
+            *ms_per_launch = ms / reps;
+            cudaEventDestroy(e0); cudaEventDestroy(e1);
+        }
+        return LRN_OK;
+    });
+}
+
 int32_t lrn_dbg_cholesky(int32_t n, double* A, double* x, int32_t which, int32_t* info, int32_t reps, double* ms_factor) {
     return guard([&]() -> int32_t {
         HostMat dA(A, n, n), dA0(A, n, n);
         CholWork w;
+        w.int8 = g_dbg_chol_int8;
         cudaStream_t st = 0;
         cholesky_lower(dA.p, n, dA.ld, w, st);
         int inf = 0;

@@ -430,9 +430,11 @@ __global__ void __launch_bounds__(288) panel_rotate_kernel(const PanelRotatePara
 std::atomic<long long> g_launches{0};
 
 // optional per-launch profiling (bench roofline): CUDA events around every DMMA GEMM launch on its own stream
-struct ProfRec { cudaEvent_t a, b; double flops; int fam = 0; };   // fam: 0 cp.async kernel, 1 TMA-fed kernel, 2 panel rotation
-double g_fam_ms[3] = {0, 0, 0}, g_fam_flops[3] = {0, 0, 0};
-long long g_fam_n[3] = {0, 0, 0};
+// fam: 0 cp.async kernel, 1 TMA-fed kernel, 2 panel rotation, 3 INT8 Ozaki update (chol_i8.cu; not a DMMA kernel)
+struct ProfRec { cudaEvent_t a, b; double flops; int fam = 0; };
+constexpr int NFAM = 4, NFAM_DMMA = 3;
+double g_fam_ms[NFAM] = {}, g_fam_flops[NFAM] = {};
+long long g_fam_n[NFAM] = {};
 bool g_prof_on = false;
 std::vector<ProfRec> g_prof;
 constexpr size_t PROF_CAP = 60000;
@@ -621,6 +623,23 @@ long long gemm_launch_count() { return g_launches.load(); }
 
 bool gemm_profile_active() { return g_prof_on; }
 
+bool gemm_prof_begin(cudaStream_t st, cudaEvent_t& start) {
+    if (!g_prof_on || g_prof.size() >= PROF_CAP) return false;
+    LRN_CUDA(cudaEventCreate(&start));
+    LRN_CUDA(cudaEventRecord(start, st));
+    return true;
+}
+
+void gemm_prof_end(cudaEvent_t start, cudaStream_t st, double flops, int fam) {
+    ProfRec rec;
+    rec.a = start;
+    LRN_CUDA(cudaEventCreate(&rec.b));
+    LRN_CUDA(cudaEventRecord(rec.b, st));
+    rec.flops = flops;
+    rec.fam = fam;
+    g_prof.push_back(rec);
+}
+
 void gemm_profile(int mode, double* ms, double* flops, long long* launches) {
     if (mode == 1) {
         for (auto& r : g_prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
@@ -628,7 +647,7 @@ void gemm_profile(int mode, double* ms, double* flops, long long* launches) {
         g_prof_on = true;
         return;
     }
-    if (mode >= 10 && mode <= 12) {          // per-kernel totals of the last stopped profile
+    if (mode >= 10 && mode < 10 + NFAM) {    // per-kernel totals of the last stopped profile
         const int f = mode - 10;
         if (ms) *ms = g_fam_ms[f];
         if (flops) *flops = g_fam_flops[f];
@@ -638,18 +657,20 @@ void gemm_profile(int mode, double* ms, double* flops, long long* launches) {
     g_prof_on = false;
     LRN_CUDA(cudaDeviceSynchronize());
     double t = 0.0, f = 0.0;
-    for (int k = 0; k < 3; k++) { g_fam_ms[k] = 0.0; g_fam_flops[k] = 0.0; g_fam_n[k] = 0; }
+    long long n = 0;
+    for (int k = 0; k < NFAM; k++) { g_fam_ms[k] = 0.0; g_fam_flops[k] = 0.0; g_fam_n[k] = 0; }
     for (auto& r : g_prof) {
         float e = 0.f;
         if (cudaEventElapsedTime(&e, r.a, r.b) == cudaSuccess) {
-            t += e; f += r.flops;
+            if (r.fam < NFAM_DMMA) { t += e; f += r.flops; }
             g_fam_ms[r.fam] += e; g_fam_flops[r.fam] += r.flops; g_fam_n[r.fam]++;
         }
+        if (r.fam < NFAM_DMMA) n++;
         cudaEventDestroy(r.a); cudaEventDestroy(r.b);
     }
     if (ms) *ms = t;
     if (flops) *flops = f;
-    if (launches) *launches = (long long)g_prof.size();
+    if (launches) *launches = n;
     g_prof.clear();
 }
 

@@ -78,7 +78,13 @@ struct PanelRotateParams {
 };
 void panel_rotate(const PanelRotateParams& p, cudaStream_t stream);
 // mode 1: start recording one CUDA-event pair per GEMM launch; mode 0: stop, synchronise and report the totals
+// modes 10 / 11 / 12 / 13 return the totals of one kernel family of the last stopped profile; family 3 (the INT8 Ozaki update of
+// chol_i8.cu) is kept out of the mode 0 totals, which describe the DMMA kernels only
 void gemm_profile(int mode, double* ms, double* flops, long long* launches);
 bool gemm_profile_active();   // per-launch event timing is on (stream capture must not be used meanwhile)
+// per-launch records of kernels outside gemm.cu: begin records a start event on `st` when the profile is on (returns false
+// otherwise); end records the stop event and files the launch under family `fam` with its algorithmic flops
+bool gemm_prof_begin(cudaStream_t st, cudaEvent_t& start);
+void gemm_prof_end(cudaEvent_t start, cudaStream_t st, double flops, int fam);
 
 }  // namespace lrn

@@ -1068,8 +1068,10 @@ int32_t lrn_schur_factor(lrn_handle_t h) {
                         "the Schur rows are sharded but the handle has no NCCL communicator (lrn_dist_init / lrn_create_multi)");
             if (h->nccl && static_cast<DistCtx*>(h->nccl)->comm)
                 cholesky_dist(h->L.p(), h->n_var, h->L.ld, h->cholH, *static_cast<DistCtx*>(h->nccl), h->dist_pw, st);
-            else
+            else {
+                h->cholH.int8 = h->chol_int8;
                 cholesky_lower(h->L.p(), h->n_var, h->L.ld, h->cholH, st);
+            }
             LRN_CUDA(cudaMemcpyAsync(&info, h->cholH.info_ptr(), sizeof(int), cudaMemcpyDeviceToHost, st));
             LRN_CUDA(cudaStreamSynchronize(st));
         }
@@ -1460,6 +1462,7 @@ int32_t lrn_set_option(lrn_handle_t h, const char* name, double value) {
         else if (n == "svd_tol") h->opt.svd_tol = value;
         else if (n == "lanczos_tol") h->opt.lanczos_tol = value;
         else if (n == "lanczos_kmax") h->lanczos_kmax = std::max(4, (int)value);   // test hook: forces the bisection fallback
+        else if (n == "chol_int8") h->chol_int8 = value != 0 ? 1 : 0;
         else if (n == "pair_kernel") h->use_staged_pairs = (int)value;   // 0: gather kernel (one thread per pair), 1: staged kernel, -1: auto
         else if (n == "sparse_op") {
             // 0: dense W M W operator, 1: sparse-aware operator wherever the data allows it, -1: automatic (density rule)

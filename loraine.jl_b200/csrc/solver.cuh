@@ -129,6 +129,8 @@ struct lrn_solver {
     int dist_pw = 512;                 // row block height of the block-cyclic Schur distribution
     int use_staged_pairs = -1;         // sparse-pair Schur term: 1 staged kernel (pairs.cu) when the block has a plan, 0 gather kernel,
                                        // -1 automatic (staged from 1024 participating constraints per block on)
+    int chol_int8 = 1;                 // Schur factor: trailing updates as Ozaki INT8 products for n_var >= 16384 (CholWork::int8;
+                                       // lrn_set_option("chol_int8", 0) keeps them on DMMA)
     bool H_gathered = false;           // the row-block shards of H have already been summed over the ranks (parity hooks)
     void* group = nullptr;             // lrn::Group*: this handle is the facade of an in-process multi-GPU group (group.cuh)
 };
