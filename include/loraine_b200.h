@@ -56,8 +56,10 @@ typedef struct lrn_options {
 void lrn_default_options(lrn_options_t* opt);
 
 /* ---- construction: replaces MyModel / MySolver storage (src/model.jl:34-87, src/Solvers.jl:18-147, :363-446) ---- */
-/* Limits on n_var: kit = 0 forms the dense n_var x n_var Schur matrix and its factor, so 1 <= n_var <= 140 000
- * (LRN_ERR_ARG "n_var out of range (1..140000)").  kit = 1 forms neither: 1 <= n_var <= 2^31 - 1, and lrn_finalize returns
+/* Limits on n_var: kit = 0 forms the dense n_var x n_var Schur matrix and its factor on every GPU, so 1 <= n_var <= 140 000
+ * (LRN_ERR_ARG "n_var out of range (1..140000)"), and lrn_finalize returns LRN_ERR_ARG, naming the bytes needed and the bytes
+ * free, when they, the Cholesky workspace and the model do not fit the device's free memory (near n_var = 100 000 on a
+ * 180 GB B200, for any number of GPUs).  kit = 1 forms neither: 1 <= n_var <= 2^31 - 1, and lrn_finalize returns
  * LRN_ERR_ARG, naming the bytes needed and the bytes free, when the CG state does not fit the device's free memory.  With an
  * LP block and n_var > 140 000, lrn_prec_prepare(h, 1) (H_alpha) returns LRN_ERR_UNSUPPORTED; kinds 2 and 4 run. */
 int32_t lrn_create(lrn_handle_t* out, int64_t n_var, int64_t nlmi, const int64_t* msizes, int64_t nlin,
@@ -196,6 +198,9 @@ int32_t lrn_create_multi(lrn_handle_t* out, int64_t n_var, int64_t nlmi, const i
 /* ---- multi-GPU (one process per GPU; NCCL over NVLink) ---- */
 /* unique id: 128 bytes generated on rank 0 with lrn_dist_unique_id and broadcast by the host (torch.distributed / MPI) */
 int32_t lrn_dist_unique_id(void* out128);
+/* Collective.  On a finalized kit = 0 handle every rank also checks that the exchange buffers of the distributed
+ * factorisation fit its free device memory; if any rank is short, every rank returns LRN_ERR_ARG (lrn_last_error names
+ * the byte counts) and the handle stays single-GPU. */
 int32_t lrn_dist_init(lrn_handle_t h, int32_t rank, int32_t world, const void* unique_id128);
 
 #ifdef __cplusplus

@@ -712,6 +712,15 @@ void ensure_aux(CholWork& work) {
     for (auto& e : work.ev) LRN_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
 }
 
+// the two trailing-update products of a panel run as Ozaki INT8 products (chol_i8.cu) when the caller opted in: the solved
+// panel is sliced into digit planes once, on the panel stream, and both products read the planes
+static bool lookahead_i8(int n, int int8) {
+    static const bool env_off = [] { const char* e = getenv("LRN_CHOL_INT8"); return e && atoi(e) == 0; }();
+    const int NB = pick_nb(n);
+    return n > NB && (int8 == 2 || (int8 == 1 && NB == 1024 && !env_off));
+}
+static int slice_rows(int rows) { return round_up(rows, 128) + 128; }   // room for the 128-row tiles at row offset wq
+
 // Right-looking factorisation with one-step look-ahead on two streams.  The high-priority panel stream runs the whole
 // dependency chain -- panel p (one cooperative launch: diagonal block + rows below), then the update of the NEXT panel's
 // columns -- while the main stream applies the rest of the trailing update of panel p (columns behind the next panel) on the
@@ -723,11 +732,7 @@ void chol_lookahead(double* A, int n, int lda, CholWork& work, cudaStream_t st) 
     cudaEvent_t evStart = work.ev[0], evP[2] = {work.ev[1], work.ev[2]}, evR[2] = {work.ev[3], work.ev[4]};
     int* info = work.info_ptr();
     const int NB = pick_nb(n), npan = (int)cdiv(n, NB), gcap = panel_grid_cap(n);
-    // the two trailing-update products of a panel run as Ozaki INT8 products (chol_i8.cu) when the caller opted in: the solved
-    // panel is sliced into digit planes once, on the panel stream, and both products read the planes
-    static const bool env_off = [] { const char* e = getenv("LRN_CHOL_INT8"); return e && atoi(e) == 0; }();
-    const bool i8 = n > NB && (work.int8 == 2 || (work.int8 == 1 && NB == 1024 && !env_off));
-    const auto slice_rows = [](int rows) { return round_up(rows, 128) + 128; };   // room for the 128-row tiles at row offset wq
+    const bool i8 = lookahead_i8(n, work.int8);
     if (i8) {
         const int r0 = slice_rows(n - NB);
         for (int b = 0; b < 2; b++) {
@@ -785,6 +790,17 @@ void cholesky_lower(double* A, int n, int lda, CholWork& work, cudaStream_t st) 
     if (n <= 0) return;
     if (n >= 1024) chol_lookahead(A, n, lda, work, st);
     else chol_rec(A, n, lda, work.dinv.p, work.info_ptr(), 0, work, st);
+}
+
+size_t chol_work_bytes(int n, int int8) {
+    const size_t d = sizeof(double);
+    size_t bytes = (size_t)cdiv(n, DB) * DB * DB * d + sizeof(int);             // dinv, info
+    bytes += (size_t)cdiv(n, SW) * (SW * SW + DB * DB) * d;                     // tinv, tscr (chol_build_tinv)
+    if (n >= 1024 && lookahead_i8(n, int8)) {                                   // two slice sets (chol_lookahead)
+        const int r0 = slice_rows(n - pick_nb(n));
+        bytes += 2 * (i8_slice_bytes(r0, pick_nb(n)) + (size_t)r0 * d);
+    }
+    return bytes;
 }
 
 // inverses of the 256 x 256 diagonal blocks of L: X_ii = D_i, X_ij = -D_i (L[i, j:i] X[j:i, j]) for sub-blocks i > j

@@ -45,6 +45,8 @@ struct CholWork {
 // Factor the lower triangle of A (n x n, column-major, lda) in place: A = L L^T. The strict upper triangle is ignored
 // (inside diagonal 128-tiles it may be overwritten with don't-care values). Enqueues only; read `work.info` after a sync.
 void cholesky_lower(double* A, int n, int lda, CholWork& work, cudaStream_t st);
+// device bytes a CholWork holds once cholesky_lower (with work.int8 = int8) and chol_solve have run at size n
+size_t chol_work_bytes(int n, int int8);
 
 // Factor ONE diagonal block (w <= 512) in place with a single launch; `dinv` receives its inverted 64 x 64 diagonal blocks and
 // X (w x w, leading dimension ldx, optional) the full inverse of the factor (lower triangular, zero above the diagonal);

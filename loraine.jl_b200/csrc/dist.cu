@@ -6,6 +6,7 @@
 #include <algorithm>
 #include <vector>
 #include <unistd.h>
+#include <memory>
 #include <mutex>
 
 namespace lrn {
@@ -299,6 +300,27 @@ void syrk_sq_row_blocks(const double* BG, int ldbg, int n, int K, double* H, int
     row_block_gemm(st, n, pw, rank, world, 0, BG, ldbg, BG, ldbg, H, ldh, 0, n, K, 1.0, 1.0, 1, true);
 }
 
+namespace {
+// buffer sizes (doubles) of cholesky_dist
+struct DistBufs {
+    size_t xb, send, recv;
+    DistBufs(int n, int pw, int world) {
+        const size_t blk = (size_t)pw * pw, ndmax = (size_t)(pw / CHOL_DB) * CHOL_DB * CHOL_DB;
+        const size_t maxcnt0 = (size_t)cdiv(cdiv(n, pw), world);
+        // two inverse buffers of X | 64 x 64 inverse blocks | scratch of the inversion (step parity: X(p+1) is produced while
+        // X(p) is still being used) + flag words of the peer exchange
+        xb = 2 * (2 * blk + ndmax) + 64;
+        send = maxcnt0 * blk;
+        recv = send * world;
+    }
+};
+}  // namespace
+
+size_t dist_work_bytes(int n, int pw, int world) {
+    const DistBufs b(n, pw, world);
+    return (b.xb + b.send + b.recv) * sizeof(double) + (size_t)world * sizeof(int);
+}
+
 void cholesky_dist(double* A, int n, int lda, CholWork& work, DistCtx& ctx, int pw, cudaStream_t st) {
     work.tinv_for = nullptr;   // the triangular solves rebuild their diagonal-block inverses from the new factor
     work.ensure(n);
@@ -306,13 +328,12 @@ void cholesky_dist(double* A, int n, int lda, CholWork& work, DistCtx& ctx, int 
     LRN_REQUIRE(ctx.comm, "no NCCL communicator (lrn_dist_init)");
     const int world = ctx.world, rank = ctx.rank;
     const int nblk = (int)cdiv(n, pw);
-    const int maxcnt0 = (int)cdiv(nblk, world);
     const size_t blk = (size_t)pw * pw, ndmax = (size_t)(pw / CHOL_DB) * CHOL_DB * CHOL_DB;
     const size_t xhalf = 2 * blk + ndmax;            // one inverse buffer: X | 64 x 64 inverse blocks | scratch of the inversion
-    // two inverse buffers (step parity: X(p+1) is produced while X(p) is still being used) + flag words of the peer exchange
-    if (ctx.xb.n < 2 * xhalf + 64) { ctx.xb.alloc(2 * xhalf + 64); ctx.flags_off = 2 * xhalf; ctx.p2p = -1; }
-    if (ctx.sendbuf.n < (size_t)maxcnt0 * blk) ctx.sendbuf.alloc((size_t)maxcnt0 * blk);
-    if (ctx.recvbuf.n < (size_t)maxcnt0 * blk * world) ctx.recvbuf.alloc((size_t)maxcnt0 * blk * world);
+    const DistBufs bufs(n, pw, world);
+    if (ctx.xb.n < bufs.xb) { ctx.xb.alloc(bufs.xb); ctx.flags_off = 2 * xhalf; ctx.p2p = -1; }
+    if (ctx.sendbuf.n < bufs.send) ctx.sendbuf.alloc(bufs.send);
+    if (ctx.recvbuf.n < bufs.recv) ctx.recvbuf.alloc(bufs.recv);
     if (ctx.infos.n < (size_t)world) ctx.infos.alloc(world);
     if (ctx.p2p < 0 || (ctx.p2p >= 1 && ctx.L_mapped != A)) setup_p2p(ctx, A, st);     // collective, once per factor matrix
     // exchange mode: 0 NCCL only; 1 (default) the 2 MB inverse travels over peer memory (latency-bound), the solved panel through
@@ -553,15 +574,36 @@ int32_t lrn_dist_init(lrn_handle_t h, int32_t rank, int32_t world, const void* u
         LRN_CUDA(cudaSetDevice(h->device));
         ncclUniqueId id;
         std::memcpy(&id, unique_id128, sizeof id);
-        auto* ctx = new DistCtx();
+        std::unique_ptr<DistCtx> ctx(new DistCtx());
         ctx->rank = rank;
         ctx->world = world;
         LRN_NCCL(nccl_api().CommInitRank(&ctx->comm, world, id, rank));
+        const int pw = (h->n_var >= 16384) ? 512 : (h->n_var >= 4096 ? 256 : 128);
+        if (h->finalized && h->H.p()) {
+            // lrn_finalize counted no exchange buffers (it ran without a communicator): refuse now if the buffers the
+            // distributed factorisation will allocate do not fit, with the same decision on every rank
+            size_t free_b = 0, total_b = 0;
+            LRN_CUDA(cudaMemGetInfo(&free_b, &total_b));
+            const size_t need = dist_work_bytes(h->n_var, pw, world);
+            const int mine = need > free_b ? 1 : 0;
+            DevBuf<int> flag(1);
+            LRN_CUDA(cudaMemcpyAsync(flag.p, &mine, sizeof(int), cudaMemcpyHostToDevice, h->st));
+            LRN_NCCL(nccl_api().AllReduce(flag.p, flag.p, 1, ncclInt32, ncclMax, ctx->comm, h->st));
+            int any = 0;
+            LRN_CUDA(cudaMemcpyAsync(&any, flag.p, sizeof(int), cudaMemcpyDeviceToHost, h->st));
+            LRN_CUDA(cudaStreamSynchronize(h->st));
+            if (any) {
+                h->err = "lrn_dist_init: the exchange buffers of the distributed factorisation need " + std::to_string(need) +
+                         " bytes of device memory on this rank, " + std::to_string(free_b) + " bytes are free" +
+                         (mine ? "" : " (another rank is short of memory)");
+                return LRN_ERR_ARG;
+            }
+        }
         if (h->nccl) delete static_cast<DistCtx*>(h->nccl);
-        h->nccl = ctx;
+        h->nccl = ctx.release();
         h->rank = rank;
         h->world = world;
-        h->dist_pw = (h->n_var >= 16384) ? 512 : (h->n_var >= 4096 ? 256 : 128);
+        h->dist_pw = pw;
         return LRN_OK;
     } catch (const std::exception& e) {
         h->err = e.what();

@@ -56,6 +56,8 @@ struct CholWork;
 // rank then updates its own row blocks of the trailing matrix (strided-batch lower-staircase GEMM on the TMA-fed kernel).
 // The panel chain of step p+1 runs on a high-priority stream while the main stream still applies the update of step p.
 void cholesky_dist(double* A, int n, int lda, CholWork& work, DistCtx& ctx, int pw, cudaStream_t st);
+// device bytes of the exchange buffers cholesky_dist keeps in its DistCtx
+size_t dist_work_bytes(int n, int pw, int world);
 // Schur assembly, rank-one path, for the row blocks of one rank:  H[rows g, 0:(g+1) pw] += ((BG)(BG)').^2 (lower staircase)
 void syrk_sq_row_blocks(const double* BG, int ldbg, int n, int K, double* H, int ldh, int rank, int world, int pw, cudaStream_t st);
 // in-place sum of a device buffer over all ranks

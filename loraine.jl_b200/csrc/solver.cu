@@ -480,8 +480,8 @@ int32_t lrn_create(lrn_handle_t* out, int64_t n_var, int64_t nlmi, const int64_t
             h->err = "loraine_b200 requires an sm_100 (Blackwell) GPU; there is no fallback path";
             return LRN_ERR_NO_DEVICE;
         }
-        // kit = 0: the Schur matrix and its factor are dense n_var x n_var FP64 (2 x 8 n_var^2 bytes): 140 000 is what 180 GB
-        // of HBM holds.  kit = 1 forms neither; its limit is the device memory lrn_finalize checks (indices stay int).
+        // kit = 0: see KIT0_MAX_NVAR; below it, the device memory lrn_finalize checks decides.  kit = 1 forms no dense Schur
+        // matrix; its limit is the device memory lrn_finalize checks (indices stay int).
         if (h->opt.kit == 1) LRN_REQUIRE(n_var >= 1 && n_var <= INT32_MAX, "n_var out of range (1..2147483647 for kit = 1)");
         else LRN_REQUIRE(n_var >= 1 && n_var <= KIT0_MAX_NVAR, "n_var out of range (1..140000)");
         LRN_REQUIRE(nlmi >= 0 && nlin >= 0 && nlin < 2000000000LL, "nlmi/nlin out of range");
@@ -555,12 +555,12 @@ int32_t lrn_set_b(lrn_handle_t h, const double* b) {
     });
 }
 
-// Device bytes of the kit = 1 state, from the staged model: model data, the n_var-long vectors, the m x m block arrays, and
-// for H_alpha the kS x kS matrix S and one slab of its row-slab build (the dense AAAATtau of an LP block below KIT0_MAX_NVAR).
-static size_t cg_footprint(const lrn_solver* h) {
+// Device bytes both kits need, from the staged model: model data, the n_var-long vectors of the iteration and the m x m block
+// arrays.  kS (sum of erank x m) and maxm are returned for the kit-specific parts.
+static size_t model_footprint(const lrn_solver* h, int& kS, int& maxm) {
     const size_t n = (size_t)h->n_var, d = sizeof(double), ix = sizeof(int);
-    size_t bytes = 14 * n * d;                                    // y, dely, rhs, Rp, tn1, tn2, ones, b, 4 CG vectors, pDiag, pDsq
-    int kS = 0, maxm = 1;
+    size_t bytes = 8 * n * d;                                     // y, dely, rhs, Rp, tn1, tn2, ones, b
+    kS = 0; maxm = 1;
     for (const auto& B : h->blk) {
         const size_t nnz = B.hAA.rowval.size(), nnzB = B.hB.rowval.size(), mm = (size_t)pad_ld(B.m) * B.m;
         bytes += nnz * (3 * ix + 3 * d) + nnz * (3 * ix + d);     // by-constraint (p, q, v, values), by-position lists
@@ -570,6 +570,28 @@ static size_t cg_footprint(const lrn_solver* h) {
         maxm = std::max(maxm, B.m);
     }
     if (h->nlin > 0) bytes += 2 * h->hClin.rowval.size() * (ix + d) + (n + h->nlin + 2) * ix + 12 * (size_t)h->nlin * d;
+    return bytes;
+}
+
+// Device bytes of the kit = 0 state on this rank: the model, the dense Schur matrix H and its factor L (n_var x n_var each),
+// the rank-one product B G, the Cholesky workspace, and the panel-exchange buffers of the distributed factorisation.
+static size_t direct_footprint(const lrn_solver* h) {
+    int kS = 0, maxm = 1;
+    const size_t n = (size_t)h->n_var, d = sizeof(double), ld = (size_t)pad_ld(h->n_var);
+    size_t bytes = model_footprint(h, kS, maxm) + 2 * ld * n * d;
+    if (h->opt.datarank == -1) bytes += ld * round_up(maxm, 32) * d;
+    const bool dist = h->nccl && static_cast<DistCtx*>(h->nccl)->comm;
+    bytes += chol_work_bytes(h->n_var, dist ? 0 : h->chol_int8);
+    if (dist) bytes += dist_work_bytes(h->n_var, h->dist_pw, h->world);
+    return bytes;
+}
+
+// Device bytes of the kit = 1 state: the model, four CG vectors and the diagonal preconditioner, and for H_alpha the kS x kS
+// matrix S and one slab of its row-slab build (the dense AAAATtau of an LP block below KIT0_MAX_NVAR).
+static size_t cg_footprint(const lrn_solver* h) {
+    const size_t n = (size_t)h->n_var, d = sizeof(double);
+    int kS = 0, maxm = 1;
+    size_t bytes = model_footprint(h, kS, maxm) + 6 * n * d;     // 4 CG vectors, pDiag, pDsq
     if (h->opt.preconditioner == 1 || h->opt.preconditioner == 4) {
         bytes += ((size_t)pad_ld(kS) * kS + 2 * (size_t)kS) * d;
         bytes += prec_slab_bytes(prec_slab_rows(h->n_var, kS, maxm, h->slab_force), kS, maxm);
@@ -583,14 +605,15 @@ int32_t lrn_finalize(lrn_handle_t h) {
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(!h->finalized, "already finalized");
         LRN_REQUIRE(h->b.p, "lrn_set_b was not called");
-        if (h->opt.kit == 1) {
-            // refuse a model whose CG state cannot fit before anything is allocated, instead of failing partway through a solve
+        {
+            // refuse a model whose state cannot fit before anything is allocated, instead of failing with a bare out-of-memory
+            // error here or partway through a solve
             size_t free_b = 0, total_b = 0;
             LRN_CUDA(cudaMemGetInfo(&free_b, &total_b));
-            const size_t need = cg_footprint(h);
+            const size_t need = h->opt.kit == 1 ? cg_footprint(h) : direct_footprint(h);
             if (need > free_b)
-                throw std::invalid_argument("kit = 1 state needs " + std::to_string(need) + " bytes of device memory, " +
-                                            std::to_string(free_b) + " bytes are free");
+                throw std::invalid_argument("kit = " + std::to_string(h->opt.kit) + " state needs " + std::to_string(need) +
+                                            " bytes of device memory, " + std::to_string(free_b) + " bytes are free");
         }
         const int n = h->n_var;
         int maxm = 1;

@@ -52,8 +52,11 @@ struct PhaseEvt {
     int phase;
 };
 
-// Largest n_var of the direct (kit = 0) path: its Schur matrix and factor are dense n_var x n_var FP64 (2 x 8 n_var^2 bytes),
-// and 140 000 is what 180 GB of HBM holds.  The CG path (kit = 1) forms neither.
+// Largest n_var lrn_create admits for the direct (kit = 0) path.  Every rank holds the dense n_var x n_var FP64 Schur matrix
+// and its factor (16 n_var^2 bytes) plus about 19 KB per row of Cholesky workspace (chol_work_bytes), so on a 180 GB B200 the
+// path ends near n_var = 105 000 (178 GB), less the CUDA context, the model and the block arrays; 140 000 (314 GB) fits no
+// single GPU.  lrn_finalize refuses any kit = 0 model whose state does not fit the free device memory (direct_footprint in
+// solver.cu).  The CG path (kit = 1) forms neither matrix.
 constexpr int64_t KIT0_MAX_NVAR = 140000;
 // Row-slab height of the H_alpha build (pcg.cu): n_var when the whole T (n_var x kS) and A_j u_r (n_var x maxm) fit the slab
 // budget, otherwise the largest multiple of 8 that does; force > 0 is used as given (clamped to n_var).
