@@ -83,8 +83,28 @@ int32_t lrn_dbg_prec_slab(lrn_handle_t h, int64_t set_rows, int64_t* rows_used);
  * (which = LRN_ARR_H) or Cholesky factors (LRN_ARR_L) of two handles living on the same device; computed on the device
  * (bench.py's dist_parity: sharded handle against a single-GPU handle at n_var = 40000 without a 12.8 GB download) */
 int32_t lrn_dbg_compare(lrn_handle_t a, lrn_handle_t b, int32_t which, double* relerr);
-/* multi-GPU: sum the row-block shards of the Schur matrix over all ranks in place (collective; every rank calls) */
+/* multi-GPU: sum the row-block shards of the Schur matrix over all ranks in place (collective; every rank calls).
+ * LRN_ERR_STATE on a handle in the own-rows layout (it holds no full matrix); so does lrn_dbg_compare. */
 int32_t lrn_dbg_gather_H(lrn_handle_t h);
+/* test hook: storage layout of the kit = 0 Schur matrix H and its factor L.  force (before lrn_finalize): -1 lrn_finalize
+ * decides (default), 0 replicated (n_var rows on every rank), 1 own rows (only the rank's own row blocks, stacked; the sharded
+ * assembly, lrn_dist_init / lrn_dbg_set_shard ownership, must be set before lrn_finalize); -2 leaves the setting.  *layout
+ * (optional) receives the layout in use: 0, 1, or -1 before lrn_finalize.  A group handle sets every member, reports member 0. */
+int32_t lrn_dbg_schur_layout(lrn_handle_t h, int32_t force, int32_t* layout);
+/* test hook: the device bytes lrn_finalize counts for the kit = 0 state of this handle (its rank, world and block height)
+ * in the replicated (rows_local = 0) or the own-rows layout (1).  A group handle reports member 0. */
+int32_t lrn_dbg_schur_footprint(lrn_handle_t h, int32_t rows_local, int64_t* bytes);
+/* test hook: load the kit = 0 Schur matrix H (n_var x n_var, column-major, host; the lower triangle is used) into the
+ * handle's layout: a replicated handle takes all of it, an own-rows handle its own row blocks; every member of a group
+ * handle reads the same array.  lrn_schur_factor then factors it (checks of the factorisation on known matrices). */
+int32_t lrn_dbg_set_H(lrn_handle_t h, const double* H);
+/* test hook: the lrn_create_multi facade with `world` (1..8) members that all live on the CURRENT device and exchange data
+ * through an in-process loopback transport instead of NCCL (host rendezvous of the member threads, device-to-device copies;
+ * a member that does not arrive within 120 s makes the collective fail).  The peer-memory exchange is off.  block_rows: row
+ * block height of the Schur distribution (a multiple of 64, at most 512; 0 = the library's default for n_var).  Lets world =
+ * 2 or 3 of the distributed factorisation and solves run on one GPU. */
+int32_t lrn_dbg_create_loopback(lrn_handle_t* out, int64_t n_var, int64_t nlmi, const int64_t* msizes, int64_t nlin,
+                                const lrn_options_t* opt, int32_t world, int32_t block_rows);
 
 #ifdef __cplusplus
 }

@@ -332,7 +332,7 @@ __global__ void __launch_bounds__(256) k_schur_pairs(int npart, int first, const
         acc += va * s;
     }
     const int r = j > k ? j : k, c = j > k ? k : j;
-    H[(size_t)c * ldh + r] += acc;
+    H[(size_t)c * ldh + own.local(r)] += acc;
 }
 __global__ void k_schur_f1_column(int npart, int jj, const int* __restrict__ part, const int* __restrict__ rowptr,
                                   const int* __restrict__ ep, const int* __restrict__ eq, const double* __restrict__ ev,
@@ -346,7 +346,7 @@ __global__ void k_schur_f1_column(int npart, int jj, const int* __restrict__ par
     s = warp_sum(s);
     if (lane == 0) {
         const int r = j > k ? j : k, c = j > k ? k : j;
-        H[(size_t)c * ldh + r] += s;
+        H[(size_t)c * ldh + own.local(r)] += s;
     }
 }
 __global__ void k_densify(int e0, int e1, const int* __restrict__ ep, const int* __restrict__ eq, const double* __restrict__ ev,
@@ -380,13 +380,14 @@ __global__ void k_lin_schur(int n_var, const int* __restrict__ r_ptr, const int*
     int j = blockIdx.x * TB + threadIdx.x;
     if (j >= n_var) return;
     if (H && !own.owns(j)) return;          // thread j writes row j of the lower triangle
+    const int jl = own.local(j);
     for (int t = r_ptr[j]; t < r_ptr[j + 1]; t++) {
         const int r = r_col[t];
         const double w = r_val[t] * d[r];
         if (H) {
             for (int u = c_ptr[r]; u < c_ptr[r + 1]; u++) {
                 const int k = c_row[u];
-                if (k <= j) H[(size_t)k * ldh + j] += w * c_val[u];
+                if (k <= j) H[(size_t)k * ldh + jl] += w * c_val[u];
             }
         } else {
             diag[j] += w * r_val[t];

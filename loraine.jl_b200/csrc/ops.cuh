@@ -68,13 +68,29 @@ struct Reducer {
 // Row ownership of the Schur matrix in multi-GPU runs: 1-D block-cyclic by ROW blocks of height `pw`
 // (row block g -> rank g % world); a rank assembles and factors the part of the lower triangle that lies in its rows
 // (entry (r, c), c <= r, belongs to the owner of row r).  world <= 1: everything is owned.
+// Storage of H and L: replicated (n_var rows on every rank, rows_local = false) or "own rows" (rows_local = true: only the
+// rank's own row blocks, stacked in block order into local_rows(...) rows; local(row) maps a global row to its local one).
 struct RowOwner {
     int rank = 0, world = 1, pw = 512;
+    bool rows_local = false;
 #ifdef __CUDACC__
     __host__ __device__
 #endif
     bool owns(int row) const { return world <= 1 || ((row / pw) % world) == rank; }
+    // local row of an owned global row: block g = row / pw is the (g / world)-th block of its owner
+#ifdef __CUDACC__
+    __host__ __device__
+#endif
+    int local(int row) const { return rows_local && world > 1 ? (row / pw / world) * pw + row % pw : row; }
 };
+// rows of `rank` in the own-rows layout (its blocks g = rank, rank + world, ...; a ragged last block counts its real rows)
+inline int local_rows(int n, int pw, int rank, int world) {
+    if (world <= 1) return n;
+    const int nblk = (n + pw - 1) / pw;
+    if (rank >= nblk) return 0;
+    const int cnt = (nblk - 1 - rank) / world + 1, glast = rank + (cnt - 1) * world;
+    return (cnt - 1) * pw + (n - glast * pw < pw ? n - glast * pw : pw);
+}
 
 // ---- staged sparse-pair Schur assembly (pairs.cu) ------------------------------------------------------------------
 // Plan of the shared-memory staged pair kernel: constraints are taken in INDEX order in groups of up to 8 consecutive COLUMNS

@@ -73,7 +73,7 @@ __global__ void __launch_bounds__(PT, 1)
             const int j = b_ids[t];
             if (!own.owns(j)) continue;
             const int f0 = b_eptr[t], f1 = b_eptr[t + 1];
-            double* dst = H + (size_t)r0 * ldh + j;
+            double* dst = H + (size_t)r0 * ldh + own.local(j);      // own-rows layout: j's local row
             // rows of the group one after the other (the branch on the size class is uniform over the CTA); the few entries
             // of k are re-read from L1 for every row
 #pragma unroll 1

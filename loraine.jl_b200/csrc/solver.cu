@@ -573,17 +573,52 @@ static size_t model_footprint(const lrn_solver* h, int& kS, int& maxm) {
     return bytes;
 }
 
-// Device bytes of the kit = 0 state on this rank: the model, the dense Schur matrix H and its factor L (n_var x n_var each),
-// the rank-one product B G, the Cholesky workspace, and the panel-exchange buffers of the distributed factorisation.
-static size_t direct_footprint(const lrn_solver* h) {
+static bool has_comm(const lrn_solver* h) { return h->nccl && static_cast<DistCtx*>(h->nccl)->active(); }
+
+// Device bytes of the kit = 0 state on this rank: the model, the Schur matrix H and its factor L (n_var x n_var each, or only
+// the rank's own rows in the own-rows layout), the rank-one product B G, the Cholesky workspace, the panel-exchange buffers
+// of the distributed factorisation, and in the own-rows layout its panel slots and stored diagonal-block inverses.
+static size_t direct_footprint(const lrn_solver* h, bool rows_local) {
     int kS = 0, maxm = 1;
     const size_t n = (size_t)h->n_var, d = sizeof(double), ld = (size_t)pad_ld(h->n_var);
-    size_t bytes = model_footprint(h, kS, maxm) + 2 * ld * n * d;
+    const int rows = rows_local ? local_rows(h->n_var, h->dist_pw, h->rank, h->world) : h->n_var;
+    size_t bytes = model_footprint(h, kS, maxm) + 2 * (size_t)pad_ld(rows) * n * d;
     if (h->opt.datarank == -1) bytes += ld * round_up(maxm, 32) * d;
-    const bool dist = h->nccl && static_cast<DistCtx*>(h->nccl)->comm;
+    const bool dist = has_comm(h);
     bytes += chol_work_bytes(h->n_var, dist ? 0 : h->chol_int8);
     if (dist) bytes += dist_work_bytes(h->n_var, h->dist_pw, h->world);
+    if (rows_local) bytes += dist_rows_local_bytes(h->n_var, h->dist_pw);
     return bytes;
+}
+
+// kit = 0 storage: the replicated layout wherever it fits; the own-rows layout when the handle has a communicator with
+// world > 1, the replicated state does not fit some rank and the own-rows state fits every rank (the ranks agree with one
+// all-reduce).  Throws the byte counts when the chosen layout does not fit.
+static void choose_layout(lrn_solver* h, size_t free_b) {
+    const size_t rep = direct_footprint(h, false);
+    bool own = h->layout_force == 1;
+    size_t need = rep;
+    if (h->layout_force == -1 && has_comm(h) && h->world > 1) {
+        const size_t loc = direct_footprint(h, true);
+        int flags[2] = {rep > free_b ? 1 : 0, loc > free_b ? 1 : 0};
+        DevBuf<int> f(2);
+        LRN_CUDA(cudaMemcpyAsync(f.p, flags, sizeof flags, cudaMemcpyHostToDevice, h->st));
+        static_cast<DistCtx*>(h->nccl)->allreduce_max(f.p, 2, h->st);
+        LRN_CUDA(cudaMemcpyAsync(flags, f.p, sizeof flags, cudaMemcpyDeviceToHost, h->st));
+        LRN_CUDA(cudaStreamSynchronize(h->st));
+        own = flags[0] && !flags[1];
+        if (own) need = loc;
+        else if (flags[0])                 // neither layout fits some rank: every rank refuses
+            throw std::invalid_argument("kit = 0 state needs " + std::to_string(rep) + " bytes of device memory (" +
+                                        std::to_string(loc) + " with own Schur rows only), " + std::to_string(free_b) +
+                                        " bytes are free" + (rep > free_b && loc > free_b ? "" : " (another rank is short of memory)"));
+    } else if (own) {
+        need = direct_footprint(h, true);
+    }
+    if (need > free_b)
+        throw std::invalid_argument("kit = 0 state needs " + std::to_string(need) + " bytes of device memory, " +
+                                    std::to_string(free_b) + " bytes are free");
+    h->rows_local = own;
 }
 
 // Device bytes of the kit = 1 state: the model, four CG vectors and the diagonal preconditioner, and for H_alpha the kS x kS
@@ -600,6 +635,39 @@ static size_t cg_footprint(const lrn_solver* h) {
     return bytes;
 }
 
+// test hook (loraine_b200_debug.h): direct_footprint of either layout for this handle's rank, world and block height
+extern "C" int32_t lrn_dbg_schur_footprint(lrn_handle_t h, int32_t rows_local, int64_t* bytes) {
+    if (h && h->group) h = static_cast<Group*>(h->group)->members[0];
+    if (!h || !bytes || rows_local < 0 || rows_local > 1) return LRN_ERR_ARG;
+    *bytes = (int64_t)direct_footprint(h, rows_local != 0);
+    return LRN_OK;
+}
+
+// test hook (loraine_b200_debug.h): load the Schur matrix (n x n, column-major, host) into the layout in use
+extern "C" int32_t lrn_dbg_set_H(lrn_handle_t h, const double* Hh) {
+    LRN_GROUP(h, lrn_dbg_set_H(m_, Hh));
+    if (!h || !Hh) return LRN_ERR_ARG;
+    return guarded(h, [&]() -> int32_t {
+        LRN_REQUIRE(h->H.p(), "Schur matrix is only allocated for kit = 0");
+        const size_t n = (size_t)h->n_var;
+        const int pw = h->dist_pw;
+        if (h->rows_local) {
+            for (int g = h->rank; (size_t)g * pw < n; g += h->world) {
+                const size_t r0 = (size_t)g * pw, rows = std::min<size_t>(pw, n - r0), l0 = (size_t)(g / h->world) * pw;
+                LRN_CUDA(cudaMemcpy2DAsync(h->H.p() + l0, (size_t)h->H.ld * sizeof(double), Hh + r0, n * sizeof(double),
+                                           rows * sizeof(double), n, cudaMemcpyHostToDevice, h->st));
+            }
+        } else {
+            LRN_CUDA(cudaMemcpy2DAsync(h->H.p(), (size_t)h->H.ld * sizeof(double), Hh, n * sizeof(double), n * sizeof(double), n,
+                                       cudaMemcpyHostToDevice, h->st));
+        }
+        LRN_CUDA(cudaStreamSynchronize(h->st));
+        h->H_gathered = h->world > 1 && !h->rows_local;      // a replicated handle now holds every row
+        h->have_factor = false;
+        return LRN_OK;
+    });
+}
+
 int32_t lrn_finalize(lrn_handle_t h) {
     LRN_GROUP(h, lrn_finalize(m_));
     return guarded(h, [&]() -> int32_t {
@@ -610,10 +678,14 @@ int32_t lrn_finalize(lrn_handle_t h) {
             // error here or partway through a solve
             size_t free_b = 0, total_b = 0;
             LRN_CUDA(cudaMemGetInfo(&free_b, &total_b));
-            const size_t need = h->opt.kit == 1 ? cg_footprint(h) : direct_footprint(h);
-            if (need > free_b)
-                throw std::invalid_argument("kit = " + std::to_string(h->opt.kit) + " state needs " + std::to_string(need) +
-                                            " bytes of device memory, " + std::to_string(free_b) + " bytes are free");
+            if (h->opt.kit == 1) {
+                const size_t need = cg_footprint(h);
+                if (need > free_b)
+                    throw std::invalid_argument("kit = 1 state needs " + std::to_string(need) + " bytes of device memory, " +
+                                                std::to_string(free_b) + " bytes are free");
+            } else {
+                choose_layout(h, free_b);
+            }
         }
         const int n = h->n_var;
         int maxm = 1;
@@ -698,8 +770,9 @@ int32_t lrn_finalize(lrn_handle_t h) {
         for (auto& B : h->blk) rank1 = rank1 && B.sp.has_B;
         if (h->opt.datarank == -1 && !rank1) h->opt.datarank = 0;      // src/Solvers.jl:435-444
         if (h->opt.kit == 0) {
-            h->H.init(n, n);
-            h->L.init(n, n);
+            const int rows = h->rows_local ? local_rows(n, h->dist_pw, h->rank, h->world) : n;
+            h->H.init(rows, n);
+            h->L.init(rows, n);
             if (rank1) h->BG.init(n, round_up(maxm, 32));   // K padded to a multiple of 32 (zero columns) for the TMA-fed SYRK
         }
         LRN_CUDA(cudaStreamSynchronize(h->st));
@@ -965,7 +1038,7 @@ int32_t lrn_schur_assemble(lrn_handle_t h) {
         LRN_CUDA(cudaMemsetAsync(h->H.p(), 0, h->H.bytes(), st));
         h->H_gathered = false;
         RowOwner own;                                  // multi-GPU: every rank assembles only the row blocks it owns
-        own.rank = h->rank; own.world = h->world; own.pw = h->dist_pw;
+        own.rank = h->rank; own.world = h->world; own.pw = h->dist_pw; own.rows_local = h->rows_local;
         bool first_block = true;                       // H is still all zeros
         for (auto& B : h->blk) {
             const int m = B.m, ld = B.ld;
@@ -982,7 +1055,7 @@ int32_t lrn_schur_assemble(lrn_handle_t h) {
                 p.M = n; p.N = n; p.K = Kp; p.lda = h->BG.ld; p.ldb = h->BG.ld; p.ldc = h->H.ld;
                 p.transB = true; p.alpha = 1.0; p.beta = 1.0; p.mode = 1; p.lower = 1;
                 if (h->world <= 1) gemm(p, st);
-                else syrk_sq_row_blocks(h->BG.p(), h->BG.ld, n, Kp, h->H.p(), h->H.ld, own.rank, own.world, own.pw, st);
+                else syrk_sq_row_blocks(h->BG.p(), h->BG.ld, n, Kp, h->H.p(), h->H.ld, own.rank, own.world, own.pw, st, h->rows_local);
             } else {
                 for (int jj = 0; jj < B.sp.nF1; jj++) {
                     // F1: U = W calA_j W, column of <calA_k, U>                (src/makeBBBB.jl:81-104)
@@ -1087,10 +1160,10 @@ int32_t lrn_schur_factor(lrn_handle_t h) {
             Phase ph(h, LRN_T_FACTOR);
             cudaStream_t st = h->st;
             LRN_CUDA(cudaMemcpyAsync(h->L.p(), h->H.p(), h->H.bytes(), cudaMemcpyDeviceToDevice, st));
-            LRN_REQUIRE(h->world <= 1 || (h->nccl && static_cast<DistCtx*>(h->nccl)->comm),
+            LRN_REQUIRE(h->world <= 1 || has_comm(h),
                         "the Schur rows are sharded but the handle has no NCCL communicator (lrn_dist_init / lrn_create_multi)");
-            if (h->nccl && static_cast<DistCtx*>(h->nccl)->comm)
-                cholesky_dist(h->L.p(), h->n_var, h->L.ld, h->cholH, *static_cast<DistCtx*>(h->nccl), h->dist_pw, st);
+            if (has_comm(h))
+                cholesky_dist(h->L.p(), h->n_var, h->L.ld, h->cholH, *static_cast<DistCtx*>(h->nccl), h->dist_pw, st, h->rows_local);
             else {
                 h->cholH.int8 = h->chol_int8;
                 cholesky_lower(h->L.p(), h->n_var, h->L.ld, h->cholH, st);
@@ -1113,7 +1186,8 @@ int32_t lrn_schur_shift(lrn_handle_t h, double delta) {
             const int pw = h->dist_pw, n = h->n_var;
             for (int g = h->rank; g * pw < n; g += h->world) {
                 const int r0 = g * pw, rb = std::min(pw, n - r0);
-                mat_add_diag(h->st, rb, h->H.p() + (size_t)r0 * h->H.ld + r0, h->H.ld, delta);
+                const int l0 = h->rows_local ? (g / h->world) * pw : r0;      // local row of the block
+                mat_add_diag(h->st, rb, h->H.p() + (size_t)r0 * h->H.ld + l0, h->H.ld, delta);
             }
         } else {
             mat_add_diag(h->st, h->n_var, h->H.p(), h->H.ld, delta);
@@ -1133,7 +1207,12 @@ int32_t lrn_schur_solve(lrn_handle_t h, int32_t which) {
         LRN_CUDA(cudaMemcpyAsync(h->dely.p, h->rhs.p, h->n_var * sizeof(double), cudaMemcpyDeviceToDevice, st));
         const int reps = (which == 6) ? 2 : 1;
         const int w = (which == 6) ? 3 : which;
-        for (int r = 0; r < reps; r++) chol_solve(h->L.p(), h->n_var, h->L.ld, h->cholH, h->dely.p, h->tn1.p, w, st);
+        if (h->rows_local && has_comm(h)) {
+            for (int r = 0; r < reps; r++)
+                chol_solve_dist(h->L.p(), h->n_var, h->L.ld, *static_cast<DistCtx*>(h->nccl), h->dist_pw, h->dely.p, w, st);
+        } else {
+            for (int r = 0; r < reps; r++) chol_solve(h->L.p(), h->n_var, h->L.ld, h->cholH, h->dely.p, h->tn1.p, w, st);
+        }
         return LRN_OK;
     });
 }
@@ -1392,7 +1471,43 @@ int32_t lrn_dimacs(lrn_handle_t h, double* err6, double* by_out, double* trCX_ou
 }
 
 // ---- parity hooks -------------------------------------------------------------------------------------------------------
+// own-rows layout: this rank's rows of H (lower triangle and its mirror image) or of L (lower triangle, zeros above) at their
+// global places of the n x n host array; `zero_rest` clears everything else first (a rank on its own: zeros elsewhere)
+static void get_rows_local(lrn_solver* h, int32_t which, double* out, bool zero_rest) {
+    LRN_REQUIRE(h->H.p(), "Schur matrix is only allocated for kit = 0");
+    const size_t n = (size_t)h->n_var;
+    const int pw = h->dist_pw;
+    const DMat& M = (which == LRN_ARR_H) ? h->H : h->L;
+    if (zero_rest) std::memset(out, 0, n * n * sizeof(double));
+    std::vector<double> rb((size_t)pw * n);
+    for (int g = h->rank; (size_t)g * pw < n; g += h->world) {
+        const int r0 = g * pw, rows = (int)std::min<size_t>(pw, n - r0), l0 = (g / h->world) * pw;
+        LRN_CUDA(cudaMemcpy2DAsync(rb.data(), (size_t)rows * sizeof(double), M.p() + l0, (size_t)M.ld * sizeof(double),
+                                   (size_t)rows * sizeof(double), n, cudaMemcpyDeviceToHost, h->st));
+        LRN_CUDA(cudaStreamSynchronize(h->st));
+        for (int i = 0; i < rows; i++) {
+            const size_t r = (size_t)r0 + i;
+            for (size_t c = 0; c < n; c++) {
+                const double v = rb[c * rows + i];
+                if (c <= r) {
+                    out[c * n + r] = v;
+                    if (which == LRN_ARR_H) out[r * n + c] = v;
+                } else if (which == LRN_ARR_L) {
+                    out[c * n + r] = 0.0;
+                }
+            }
+        }
+    }
+}
+
 int32_t lrn_get_array(lrn_handle_t h, int32_t which, int64_t iblk, double* out) {
+    // own-rows layout: every member writes its rows of H / L into the caller's array
+    if (h && h->group && (which == LRN_ARR_H || which == LRN_ARR_L) && static_cast<Group*>(h->group)->members[0]->rows_local) {
+        if (!out) return LRN_ERR_ARG;
+        return group_call(h, [&](lrn_solver* m_, int) -> int32_t {
+            return guarded(m_, [&]() -> int32_t { get_rows_local(m_, which, out, false); return LRN_OK; });
+        });
+    }
     // Schur matrix: a collective (every member contributes its row blocks); everything else is replicated -> member 0
     if (h && h->group && which != LRN_ARR_H) return lrn_get_array(static_cast<Group*>(h->group)->members[0], which, iblk, out);
     LRN_GROUP(h, lrn_get_array(m_, which, iblk, r_ == 0 ? out : nullptr));
@@ -1403,11 +1518,14 @@ int32_t lrn_get_array(lrn_handle_t h, int32_t which, int64_t iblk, double* out) 
         auto vec_out = [&](const double* p, int len) {
             LRN_CUDA(cudaMemcpyAsync(out, p, (size_t)len * sizeof(double), cudaMemcpyDeviceToHost, st));
         };
-        if (which == LRN_ARR_H || which == LRN_ARR_L) {
+        if ((which == LRN_ARR_H || which == LRN_ARR_L) && h->rows_local) {
+            LRN_REQUIRE(out, "null output");
+            get_rows_local(h, which, out, true);
+        } else if (which == LRN_ARR_H || which == LRN_ARR_L) {
             LRN_REQUIRE(h->H.p(), "Schur matrix is only allocated for kit = 0");
             DMat& M = (which == LRN_ARR_H) ? h->H : h->L;
             // work on a copy in tn-sized chunks is not possible: use the spare matrix of the other kind only when safe
-            if (which == LRN_ARR_H && h->world > 1 && h->nccl && static_cast<DistCtx*>(h->nccl)->comm && !h->H_gathered) {
+            if (which == LRN_ARR_H && h->world > 1 && has_comm(h) && !h->H_gathered) {
                 // every rank holds only its own row blocks: sum them up (once per assembly)
                 dist_allreduce_sum(M.p(), (size_t)M.ld * n, *static_cast<DistCtx*>(h->nccl), st);
                 h->H_gathered = true;

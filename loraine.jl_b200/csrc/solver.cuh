@@ -52,10 +52,10 @@ struct PhaseEvt {
     int phase;
 };
 
-// Largest n_var lrn_create admits for the direct (kit = 0) path.  Every rank holds the dense n_var x n_var FP64 Schur matrix
-// and its factor (16 n_var^2 bytes) plus about 19 KB per row of Cholesky workspace (chol_work_bytes), so on a 180 GB B200 the
-// path ends near n_var = 105 000 (178 GB), less the CUDA context, the model and the block arrays; 140 000 (314 GB) fits no
-// single GPU.  lrn_finalize refuses any kit = 0 model whose state does not fit the free device memory (direct_footprint in
+// Largest n_var lrn_create admits for the direct (kit = 0) path.  In the replicated layout every rank holds the dense
+// n_var x n_var FP64 Schur matrix and its factor (16 n_var^2 bytes) plus about 19 KB per row of Cholesky workspace
+// (chol_work_bytes), so on a 180 GB B200 the path ends near n_var = 105 000 (178 GB); 140 000 (314 GB) fits no single GPU.
+// With several GPUs lrn_finalize falls back to the own-rows layout (rows_local: 16 n_var^2 / world bytes per rank).  lrn_finalize refuses any kit = 0 model whose state does not fit the free device memory (direct_footprint in
 // solver.cu).  The CG path (kit = 1) forms neither matrix.
 constexpr int64_t KIT0_MAX_NVAR = 140000;
 // Row-slab height of the H_alpha build (pcg.cu): n_var when the whole T (n_var x kS) and A_j u_r (n_var x maxm) fit the slab
@@ -135,5 +135,7 @@ struct lrn_solver {
     int chol_int8 = 1;                 // Schur factor: trailing updates as Ozaki INT8 products for n_var >= 16384 (CholWork::int8;
                                        // lrn_set_option("chol_int8", 0) keeps them on DMMA)
     bool H_gathered = false;           // the row-block shards of H have already been summed over the ranks (parity hooks)
+    bool rows_local = false;           // kit = 0 storage: H and L hold only this rank's own row blocks (RowOwner::local, ops.cuh)
+    int layout_force = -1;             // test hook lrn_dbg_schur_layout: -1 lrn_finalize decides, 0 replicated, 1 own rows
     void* group = nullptr;             // lrn::Group*: this handle is the facade of an in-process multi-GPU group (group.cuh)
 };

@@ -35,6 +35,40 @@ def count_blocks(p: int, rank: int, world: int, nblk: int) -> int:
     return 0 if f >= nblk else (nblk - 1 - f) // world + 1
 
 
+def local_row(row: int, pw: int, world: int) -> int:
+    """local row of an owned Schur row in the own-rows layout (mirrors lrn::RowOwner::local in csrc/ops.cuh): rank r stacks
+    its blocks g = r, r + world, ... so block g starts at local row (g // world) * pw"""
+    return (row // pw // world) * pw + row % pw if world > 1 else row
+
+
+def local_rows(n_var: int, pw: int, rank: int, world: int) -> int:
+    """rows rank `rank` holds in the own-rows layout (mirrors lrn::local_rows in csrc/ops.cuh); 0 for a rank without blocks"""
+    if world <= 1:
+        return n_var
+    nblk = -(-n_var // pw)
+    if rank >= nblk:
+        return 0
+    cnt = (nblk - 1 - rank) // world + 1
+    glast = rank + (cnt - 1) * world
+    return (cnt - 1) * pw + min(pw, n_var - glast * pw)
+
+
+def pad_ld(m: int) -> int:
+    """leading dimension of a dense device matrix (mirrors lrn::pad_ld in csrc/common.cuh)"""
+    return -(-max(m, 1) // 8) * 8
+
+
+def schur_bytes(n_var: int, pw: int, rank: int, world: int, rows_local: bool) -> int:
+    """device bytes of H and L together in either layout, plus (own rows) the panel slots, stored diagonal-block inverses and
+    partial sums of the distributed factorisation and solves (mirrors direct_footprint / dist_rows_local_bytes)"""
+    rows = local_rows(n_var, pw, rank, world) if rows_local else n_var
+    b = 2 * pad_ld(rows) * n_var * 8
+    if rows_local:
+        nblk = -(-n_var // pw)
+        b += (4 * pad_ld(n_var) * pw + nblk * pw * pw + pw) * 8
+    return b
+
+
 def exchange_unique_id(make_id, rank: int, world: int) -> bytes:
     """rank 0 calls make_id() -> 128 bytes; every rank returns the same bytes."""
     import torch.distributed as dist
@@ -47,8 +81,9 @@ def exchange_unique_id(make_id, rank: int, world: int) -> bytes:
 
 
 def init_distributed(solver) -> bool:
-    """Attach the solver's device handle to the job's NCCL communicator (call after setup_solver).  Returns True when the
-    Schur assembly / factorisation is sharded over more than one rank."""
+    """Attach the solver's device handle to the job's NCCL communicator.  Called after setup_solver, the handle keeps the
+    replicated Schur layout chosen at lrn_finalize; pass attach_before_finalize to setup_solver to let lrn_finalize choose the
+    own-rows layout.  Returns True when the Schur assembly / factorisation is sharded over more than one rank."""
     import torch.distributed as dist
     if not dist.is_available() or not dist.is_initialized() or dist.get_world_size() <= 1:
         return False
@@ -66,6 +101,14 @@ def init_distributed(solver) -> bool:
     solver._call("lrn_dist_init", rank, world, buf)
     solver.dist_rank, solver.dist_world = rank, world
     return True
+
+
+def attach_before_finalize(solver) -> None:
+    """Pre-finalize hook for solver.setup_solver (`before_finalize=dist.attach_before_finalize`): attaches the device handle to
+    the job's NCCL communicator between lrn_set_b and lrn_finalize.  lrn_finalize then knows the world and can choose the
+    own-rows layout of the kit = 0 Schur matrix, so a model whose H and L do not fit one GPU is still admitted when its own
+    rows fit every rank.  A no-op outside a multi-process job."""
+    init_distributed(solver)
 
 
 def init_distributed_dd(solver) -> bool:

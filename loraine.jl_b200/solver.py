@@ -191,8 +191,10 @@ def load(model: MyModel, options: dict, T=float):
     return s, Halpha(s.kit)
 
 
-def setup_solver(s: MySolver, halpha: Halpha):
-    """src/Solvers.jl:363-446: kit / datarank fall-backs, then device allocation (instead of the per-block `zeros`)."""
+def setup_solver(s: MySolver, halpha: Halpha, before_finalize=None):
+    """src/Solvers.jl:363-446: kit / datarank fall-backs, then device allocation (instead of the per-block `zeros`).
+    before_finalize (optional) is called with the solver after lrn_set_b and before lrn_finalize, e.g.
+    dist.attach_before_finalize, which attaches a torchrun rank to its communicator so that lrn_finalize can shard H and L."""
     md = s.model
     s.alpha = np.zeros(md.nlmi)
     s.beta = np.zeros(md.nlmi)
@@ -249,6 +251,8 @@ def setup_solver(s: MySolver, halpha: Halpha):
         s._call("lrn_set_lin", _ip(cp), _ip(rv), _dp(nz), _dp(d))
     b = np.ascontiguousarray(md.b, dtype=np.float64)
     s._call("lrn_set_b", _dp(b))
+    if before_finalize is not None:
+        before_finalize(s)
     s._call("lrn_finalize")
 
 
