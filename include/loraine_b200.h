@@ -100,6 +100,10 @@ int32_t lrn_initial_point(lrn_handle_t h, int32_t initpoint);
 /* ---- iterate upload / download (initial_point.jl output in; MOI getters out, src/MOI_wrapper.jl:315-354) ---- */
 int32_t lrn_set_iterate(lrn_handle_t h, const double* const* X, const double* const* S, const double* y,
                         const double* x_lin, const double* s_lin);
+/* With the PSD blocks distributed over the ranks (kit = 0, several blocks, a communicator attached before lrn_finalize) each
+ * block lives on one owner rank: lrn_set_iterate reads every block and keeps the owned ones; on a one-process-per-GPU handle
+ * lrn_get_solution, lrn_get_slack and the per-block ids of lrn_get_array are collectives (every rank calls them with the same
+ * blocks requested; the owner broadcasts each block), a lrn_create_multi handle reads each block from its owner. */
 int32_t lrn_get_solution(lrn_handle_t h, double* y, double* const* X, double* x_lin);
 int32_t lrn_get_slack(lrn_handle_t h, double* const* S, double* s_lin);
 

@@ -91,6 +91,21 @@ int32_t lrn_dbg_gather_H(lrn_handle_t h);
  * assembly, lrn_dist_init / lrn_dbg_set_shard ownership, must be set before lrn_finalize); -2 leaves the setting.  *layout
  * (optional) receives the layout in use: 0, 1, or -1 before lrn_finalize.  A group handle sets every member, reports member 0. */
 int32_t lrn_dbg_schur_layout(lrn_handle_t h, int32_t force, int32_t* layout);
+/* test hook: layout of the PSD block state.  force (before lrn_finalize): -1 lrn_finalize decides (default: distributed when
+ * kit = 0, nlmi >= 2 and the handle has a communicator with world > 1), 0 replicated (every rank holds every block), 1
+ * distributed (block i on rank block_owner(msizes, world)[i]; needs kit = 0 and such a communicator, or lrn_finalize fails);
+ * -2 leaves the setting.  *layout (optional) receives the layout in use: 0, 1, or -1 before lrn_finalize.  A group handle
+ * sets every member and reports member 0. */
+int32_t lrn_dbg_block_layout(lrn_handle_t h, int32_t force, int32_t* layout);
+/* test hook: the device bytes lrn_finalize counts for the kit = 0 state of group member `member` (0 for a plain handle) in its
+ * Schur layout, with the PSD blocks replicated (sharded = 0) or distributed (1), into *bytes (optional); held (optional, nlmi
+ * entries) receives per block the bytes of the m x m arrays and m-vectors the member holds for it: a block of another rank
+ * keeps only its gathered W (G when datarank = -1). */
+int32_t lrn_dbg_block_footprint(lrn_handle_t h, int32_t member, int32_t sharded, int64_t* bytes, int64_t* held);
+/* test hook: group member `member`'s own device copy (0 for a plain handle) of W (which = LRN_ARR_W) or G (LRN_ARR_G) of block
+ * iblk, m x m into out, without any collective: with distributed blocks a non-owner holds the copy the all-gather of
+ * lrn_prepare_W gave it (W, or G when datarank = -1); LRN_ERR_ARG when the member holds no such array. */
+int32_t lrn_dbg_member_block(lrn_handle_t h, int32_t member, int64_t iblk, int32_t which, double* out);
 /* test hook: the device bytes lrn_finalize counts for the kit = 0 state of this handle (its rank, world and block height)
  * in the replicated (rows_local = 0) or the own-rows layout (1).  A group handle reports member 0. */
 int32_t lrn_dbg_schur_footprint(lrn_handle_t h, int32_t rows_local, int64_t* bytes);

@@ -86,6 +86,9 @@ def lib():
         "lrn_dbg_schur_layout": (i32, [vp, i32, pi32]),
         "lrn_dbg_schur_footprint": (i32, [vp, i32, pi64]),
         "lrn_dbg_set_H": (i32, [vp, pdbl]),
+        "lrn_dbg_block_layout": (i32, [vp, i32, pi32]),
+        "lrn_dbg_block_footprint": (i32, [vp, i32, i32, pi64, pi64]),
+        "lrn_dbg_member_block": (i32, [vp, i32, i64, i32, pdbl]),
         "lrn_dbg_create_loopback": (i32, [C.POINTER(vp), i64, i64, pi64, i64, C.POINTER(lrn_options_t), i32, i32]),
         "lrn_dist_unique_id": (i32, [C.c_char_p]),
         "lrn_dist_init": (i32, [vp, i32, i32, C.c_char_p]),
@@ -144,4 +147,5 @@ DEBUG_SYMBOLS = ["lrn_dbg_gemm", "lrn_dbg_cholesky", "lrn_dbg_eig_small", "lrn_d
                  "lrn_dbg_batched_lambda_min", "lrn_dbg_peak", "lrn_dbg_gemm_profile", "lrn_dbg_set_shard", "lrn_dbg_compare",
                  "lrn_dbg_gather_H", "lrn_dbg_model_block", "lrn_dd_dbg_set_shard", "lrn_dbg_prec_slab",
                  "lrn_dbg_chol_int8", "lrn_dbg_syrk_i8", "lrn_dbg_schur_layout", "lrn_dbg_create_loopback",
-                 "lrn_dbg_schur_footprint", "lrn_dbg_set_H"]
+                 "lrn_dbg_schur_footprint", "lrn_dbg_set_H", "lrn_dbg_block_layout", "lrn_dbg_block_footprint",
+                 "lrn_dbg_member_block"]

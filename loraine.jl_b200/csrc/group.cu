@@ -112,6 +112,23 @@ int32_t lrn_dbg_schur_layout(lrn_handle_t h, int32_t force, int32_t* layout) {
     return LRN_OK;
 }
 
+int32_t lrn_dbg_block_layout(lrn_handle_t h, int32_t force, int32_t* layout) {
+    if (!h || force < -2 || force > 1) return LRN_ERR_ARG;
+    if (h->group) {
+        for (auto* m : static_cast<Group*>(h->group)->members) {
+            const int32_t rc = lrn_dbg_block_layout(m, force, nullptr);
+            if (rc != LRN_OK) return rc;
+        }
+        return lrn_dbg_block_layout(static_cast<Group*>(h->group)->members[0], -2, layout);
+    }
+    if (force != -2) {
+        if (h->finalized) { h->err = "lrn_dbg_block_layout: the layout is chosen by lrn_finalize"; return LRN_ERR_STATE; }
+        h->blk_force = force;
+    }
+    if (layout) *layout = h->finalized ? (h->blk_sharded ? 1 : 0) : -1;
+    return LRN_OK;
+}
+
 int32_t lrn_dbg_create_loopback(lrn_handle_t* out, int64_t n_var, int64_t nlmi, const int64_t* msizes, int64_t nlin,
                                 const lrn_options_t* opt, int32_t world, int32_t block_rows) {
     if (!out) return LRN_ERR_ARG;

@@ -375,6 +375,7 @@ int32_t lrn_initial_point(lrn_handle_t h, int32_t initpoint) {
         LRN_REQUIRE(h->finalized && h->ip_ready, "lrn_finalize first");
         cudaStream_t st = h->st;
         for (int i = 0; i < h->nlmi; i++) {
+            if (!h->owns(i)) continue;                 // blocks distributed over the ranks: the owner's
             Block& B = h->blk[i];
             const double sm = std::sqrt((double)B.m);
             double Eps = 1.0, Eta = (double)h->n_var;

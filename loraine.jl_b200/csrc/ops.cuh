@@ -1,6 +1,7 @@
 // Elementwise / reduction / sparse kernels of the IP hot path (HBM- or L2-bound work; no tensor cores).
 #pragma once
 #include "common.cuh"
+#include <algorithm>
 
 namespace lrn {
 
@@ -90,6 +91,24 @@ inline int local_rows(int n, int pw, int rank, int world) {
     if (rank >= nblk) return 0;
     const int cnt = (nblk - 1 - rank) / world + 1, glast = rank + (cnt - 1) * world;
     return (cnt - 1) * pw + (n - glast * pw < pw ? n - glast * pw : pw);
+}
+
+// Owner rank of every PSD block when the blocks are distributed over the ranks (lrn_finalize: kit = 0, nlmi >= 2 and a
+// communicator with world > 1).  Greedy balance of m_i^3: blocks by decreasing m_i^3 (ties: lower index first), each to the
+// least-loaded rank (ties: lowest rank).  Every rank computes the same assignment; a rank may own no block.
+inline std::vector<int> block_owner(const std::vector<int>& msizes, int world) {
+    const int nb = (int)msizes.size();
+    std::vector<int> order(nb), owner(nb, 0);
+    for (int i = 0; i < nb; i++) order[i] = i;
+    auto cube = [&](int i) { return (long long)msizes[i] * msizes[i] * msizes[i]; };
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return cube(a) > cube(b); });
+    std::vector<long long> load(world > 1 ? world : 1, 0);
+    for (int i : order) {
+        const int r = (int)(std::min_element(load.begin(), load.end()) - load.begin());
+        owner[i] = r;
+        load[r] += cube(i);
+    }
+    return owner;
 }
 
 // ---- staged sparse-pair Schur assembly (pairs.cu) ------------------------------------------------------------------

@@ -141,8 +141,10 @@ void copy_csc(HostCSC& dst, int64_t ncol, const int64_t* colptr, const int64_t* 
     dst.set = true;
 }
 
-// Build the device structures of one PSD block from the staged Julia CSC of AA_i (n_var x m^2).
-void build_block(lrn_solver* h, Block& B) {
+// Build the device structures of one PSD block from the staged Julia CSC of AA_i (n_var x m^2).  A rank that does not own the
+// block (blocks distributed over the ranks) keeps the sparse data and only the m x m array its Schur rows read: G when
+// `keep_G` (datarank = -1), W otherwise.
+void build_block(lrn_solver* h, Block& B, bool own, bool keep_G) {
     const int m = B.m, n = h->n_var;
     SparseBlock& sp = B.sp;
     sp.m = m;
@@ -277,22 +279,28 @@ void build_block(lrn_solver* h, Block& B) {
         sp.nnzB = bn;
         sp.b_rowptr.upload(brp, h->st); sp.b_col.upload(bcol, h->st); sp.b_val.upload(bval, h->st);
     }
-    // dense C_i
-    B.C.init(m, m);
+    // dense C_i (its norm enters the DIMACS errors on every rank)
+    const int ldc = pad_ld(m);
+    if (own) B.C.init(m, m);
     double nc = 0.0;
     if (B.hC.set) {
-        std::vector<double> Cd((size_t)B.C.ld * m, 0.0);
+        std::vector<double> Cd((size_t)ldc * m, 0.0);
         for (int c = 0; c < m; c++)
             for (int64_t e = B.hC.colptr[c]; e < B.hC.colptr[c + 1]; e++) {
-                Cd[(size_t)c * B.C.ld + B.hC.rowval[e]] += B.hC.nzval[e];
+                Cd[(size_t)c * ldc + B.hC.rowval[e]] += B.hC.nzval[e];
             }
         for (int c = 0; c < m; c++)
-            for (int r = 0; r < m; r++) nc += Cd[(size_t)c * B.C.ld + r] * Cd[(size_t)c * B.C.ld + r];
-        B.C.buf.upload(Cd.data(), Cd.size(), h->st);
+            for (int r = 0; r < m; r++) nc += Cd[(size_t)c * ldc + r] * Cd[(size_t)c * ldc + r];
+        if (own) B.C.buf.upload(Cd.data(), Cd.size(), h->st);
     }
     B.normC = std::sqrt(nc);
     LRN_CUDA(cudaStreamSynchronize(h->st));
     B.hAA = HostCSC(); B.hB = HostCSC(); B.hC = HostCSC();
+    if (!own) {
+        (keep_G ? B.G : B.W).init(m, m);
+        B.ld = ldc;
+        return;
+    }
     for (DMat* M : {&B.X, &B.S, &B.dX, &B.dS, &B.Xn, &B.Sn, &B.G, &B.Gi, &B.W, &B.Si, &B.Rd, &B.RNT, &B.LX, &B.LS, &B.T1, &B.T2, &B.T3, &B.T4})
         M->init(m, m);
     B.ld = B.X.ld;
@@ -418,6 +426,7 @@ bool try_cholesky(lrn_solver* h, DMat& X, DMat& L, CholWork& cw) {
 
 // out = A x  (MyA functor, src/Solvers.jl:582-614)
 void apply_A(lrn_solver* h, const double* x, double* out) {
+    LRN_REQUIRE(!h->blk_sharded, "the Schur operator needs every PSD block on this rank (the blocks are distributed)");
     cudaStream_t st = h->st;
     LRN_CUDA(cudaMemsetAsync(out, 0, (size_t)h->n_var * sizeof(double), st));
     for (auto& B : h->blk) {
@@ -556,16 +565,19 @@ int32_t lrn_set_b(lrn_handle_t h, const double* b) {
 }
 
 // Device bytes both kits need, from the staged model: model data, the n_var-long vectors of the iteration and the m x m block
-// arrays.  kS (sum of erank x m) and maxm are returned for the kit-specific parts.
-static size_t model_footprint(const lrn_solver* h, int& kS, int& maxm) {
+// arrays.  kS (sum of erank x m) and maxm are returned for the kit-specific parts.  `owner` (blocks distributed over the
+// ranks): a block of another rank counts its one gathered m x m array (W, or G for datarank = -1) only.
+static size_t model_footprint(const lrn_solver* h, int& kS, int& maxm, const std::vector<int>* owner = nullptr) {
     const size_t n = (size_t)h->n_var, d = sizeof(double), ix = sizeof(int);
     size_t bytes = 8 * n * d;                                     // y, dely, rhs, Rp, tn1, tn2, ones, b
     kS = 0; maxm = 1;
-    for (const auto& B : h->blk) {
+    for (int i = 0; i < h->nlmi; i++) {
+        const Block& B = h->blk[i];
         const size_t nnz = B.hAA.rowval.size(), nnzB = B.hB.rowval.size(), mm = (size_t)pad_ld(B.m) * B.m;
         bytes += nnz * (3 * ix + 3 * d) + nnz * (3 * ix + d);     // by-constraint (p, q, v, values), by-position lists
         bytes += 2 * (n + 1) * ix + nnzB * (ix + d);              // row pointers, constraint order, rank-one factors
-        bytes += 24 * mm * d;                                     // X, S, W, G, ... T1-T4, C, Z, work of the m x m kernels
+        const bool mine = !owner || (*owner)[i] == h->rank;
+        bytes += (mine ? 24 : 1) * mm * d;                        // X, S, W, G, ... T1-T4, C, Z, work of the m x m kernels
         kS += h->opt.erank * B.m;
         maxm = std::max(maxm, B.m);
     }
@@ -574,15 +586,33 @@ static size_t model_footprint(const lrn_solver* h, int& kS, int& maxm) {
 }
 
 static bool has_comm(const lrn_solver* h) { return h->nccl && static_cast<DistCtx*>(h->nccl)->active(); }
+static DistCtx& ctx_of(lrn_solver* h) { return *static_cast<DistCtx*>(h->nccl); }
+
+static std::vector<int> block_sizes(const lrn_solver* h) {
+    std::vector<int> ms(h->nlmi);
+    for (int i = 0; i < h->nlmi; i++) ms[i] = h->blk[i].m;
+    return ms;
+}
+// doubles per rank of the W / G all-gather of prepare_W: the largest packed load of one rank, plus its status flag
+static size_t gather_chunk(const lrn_solver* h, const std::vector<int>& owner) {
+    std::vector<size_t> load(std::max(h->world, 1), 0);
+    for (int i = 0; i < h->nlmi; i++) load[owner[i]] += (size_t)pad_ld(h->blk[i].m) * h->blk[i].m;
+    return *std::max_element(load.begin(), load.end()) + 1;
+}
 
 // Device bytes of the kit = 0 state on this rank: the model, the Schur matrix H and its factor L (n_var x n_var each, or only
 // the rank's own rows in the own-rows layout), the rank-one product B G, the Cholesky workspace, the panel-exchange buffers
-// of the distributed factorisation, and in the own-rows layout its panel slots and stored diagonal-block inverses.
-static size_t direct_footprint(const lrn_solver* h, bool rows_local) {
+// of the distributed factorisation, and in the own-rows layout its panel slots and stored diagonal-block inverses.  With the
+// PSD blocks distributed (blk_sharded), the block state of the owned blocks, one m x m array per other block, the all-gather
+// buffer of prepare_W (world + 1 chunks), the world + 1 partial n_var vectors of the residuals and right-hand sides and five
+// shared values per block.
+static size_t direct_footprint(const lrn_solver* h, bool rows_local, bool blk_sharded) {
     int kS = 0, maxm = 1;
     const size_t n = (size_t)h->n_var, d = sizeof(double), ld = (size_t)pad_ld(h->n_var);
     const int rows = rows_local ? local_rows(h->n_var, h->dist_pw, h->rank, h->world) : h->n_var;
-    size_t bytes = model_footprint(h, kS, maxm) + 2 * (size_t)pad_ld(rows) * n * d;
+    const std::vector<int> owner = blk_sharded ? block_owner(block_sizes(h), h->world) : std::vector<int>();
+    size_t bytes = model_footprint(h, kS, maxm, blk_sharded ? &owner : nullptr) + 2 * (size_t)pad_ld(rows) * n * d;
+    if (blk_sharded) bytes += ((size_t)(h->world + 1) * (gather_chunk(h, owner) + n) + 5 * (size_t)h->nlmi) * d;
     if (h->opt.datarank == -1) bytes += ld * round_up(maxm, 32) * d;
     const bool dist = has_comm(h);
     bytes += chol_work_bytes(h->n_var, dist ? 0 : h->chol_int8);
@@ -595,11 +625,11 @@ static size_t direct_footprint(const lrn_solver* h, bool rows_local) {
 // world > 1, the replicated state does not fit some rank and the own-rows state fits every rank (the ranks agree with one
 // all-reduce).  Throws the byte counts when the chosen layout does not fit.
 static void choose_layout(lrn_solver* h, size_t free_b) {
-    const size_t rep = direct_footprint(h, false);
+    const size_t rep = direct_footprint(h, false, h->blk_sharded);
     bool own = h->layout_force == 1;
     size_t need = rep;
     if (h->layout_force == -1 && has_comm(h) && h->world > 1) {
-        const size_t loc = direct_footprint(h, true);
+        const size_t loc = direct_footprint(h, true, h->blk_sharded);
         int flags[2] = {rep > free_b ? 1 : 0, loc > free_b ? 1 : 0};
         DevBuf<int> f(2);
         LRN_CUDA(cudaMemcpyAsync(f.p, flags, sizeof flags, cudaMemcpyHostToDevice, h->st));
@@ -613,7 +643,7 @@ static void choose_layout(lrn_solver* h, size_t free_b) {
                                         std::to_string(loc) + " with own Schur rows only), " + std::to_string(free_b) +
                                         " bytes are free" + (rep > free_b && loc > free_b ? "" : " (another rank is short of memory)"));
     } else if (own) {
-        need = direct_footprint(h, true);
+        need = direct_footprint(h, true, h->blk_sharded);
     }
     if (need > free_b)
         throw std::invalid_argument("kit = 0 state needs " + std::to_string(need) + " bytes of device memory, " +
@@ -639,8 +669,53 @@ static size_t cg_footprint(const lrn_solver* h) {
 extern "C" int32_t lrn_dbg_schur_footprint(lrn_handle_t h, int32_t rows_local, int64_t* bytes) {
     if (h && h->group) h = static_cast<Group*>(h->group)->members[0];
     if (!h || !bytes || rows_local < 0 || rows_local > 1) return LRN_ERR_ARG;
-    *bytes = (int64_t)direct_footprint(h, rows_local != 0);
+    *bytes = (int64_t)direct_footprint(h, rows_local != 0, h->blk_sharded);
     return LRN_OK;
+}
+
+// test hook (loraine_b200_debug.h): direct_footprint of group member `member` in its Schur layout with the PSD blocks
+// replicated (sharded = 0) or distributed (1), and the bytes of the m x m block arrays and m-vectors it holds per block
+extern "C" int32_t lrn_dbg_block_footprint(lrn_handle_t h, int32_t member, int32_t sharded, int64_t* bytes, int64_t* held) {
+    if (h && h->group) {
+        auto& mem = static_cast<Group*>(h->group)->members;
+        if (member < 0 || member >= (int)mem.size()) return LRN_ERR_ARG;
+        h = mem[member];
+    } else if (member != 0) {
+        return LRN_ERR_ARG;
+    }
+    if (!h || sharded < 0 || sharded > 1) return LRN_ERR_ARG;
+    if (bytes) *bytes = (int64_t)direct_footprint(h, h->rows_local, sharded != 0);
+    if (held)
+        for (int i = 0; i < h->nlmi; i++) {
+            Block& B = h->blk[i];
+            size_t b = 0;
+            for (const DMat* M : {&B.C, &B.X, &B.S, &B.dX, &B.dS, &B.Xn, &B.Sn, &B.G, &B.Gi, &B.W, &B.Si, &B.Rd, &B.RNT, &B.LX, &B.LS,
+                                  &B.T1, &B.T2, &B.T3, &B.T4, &B.RdB})
+                b += M->p() ? M->bytes() : 0;
+            for (const DevBuf<double>* v : {&B.D, &B.DDsi, &B.dm12, &B.dm32, &B.vtmp}) b += v->n * sizeof(double);
+            held[i] = (int64_t)b;
+        }
+    return LRN_OK;
+}
+
+// test hook (loraine_b200_debug.h): a member's own device copy of W or G of one block, without collectives
+extern "C" int32_t lrn_dbg_member_block(lrn_handle_t h, int32_t member, int64_t iblk, int32_t which, double* out) {
+    if (h && h->group) {
+        auto& mem = static_cast<Group*>(h->group)->members;
+        if (member < 0 || member >= (int)mem.size()) return LRN_ERR_ARG;
+        h = mem[member];
+    } else if (member != 0) {
+        return LRN_ERR_ARG;
+    }
+    if (!h || !out || iblk < 0 || iblk >= h->nlmi || (which != LRN_ARR_W && which != LRN_ARR_G)) return LRN_ERR_ARG;
+    return guarded(h, [&]() -> int32_t {
+        const Block& B = h->blk[iblk];
+        const DMat& M = which == LRN_ARR_W ? B.W : B.G;
+        LRN_REQUIRE(M.p(), "this member holds no such array for the block");
+        download_dense(h, M.p(), M.ld, B.m, B.m, out);
+        LRN_CUDA(cudaStreamSynchronize(h->st));
+        return LRN_OK;
+    });
 }
 
 // test hook (loraine_b200_debug.h): load the Schur matrix (n x n, column-major, host) into the layout in use
@@ -674,6 +749,19 @@ int32_t lrn_finalize(lrn_handle_t h) {
         LRN_REQUIRE(!h->finalized, "already finalized");
         LRN_REQUIRE(h->b.p, "lrn_set_b was not called");
         {
+            // PSD blocks: one owner each when the handle has a communicator with world > 1 (kit = 1 stays replicated: its
+            // operator would need one reduction per CG iteration)
+            const bool comm = has_comm(h) && h->world > 1;
+            bool shard = h->opt.kit == 0 && h->nlmi >= 2 && comm;
+            if (h->blk_force == 0) shard = false;
+            if (h->blk_force == 1) {
+                LRN_REQUIRE(h->opt.kit == 0 && comm, "the sharded block layout needs kit = 0 and a communicator with world > 1");
+                shard = true;
+            }
+            h->blk_sharded = shard;
+            if (shard) h->blk_owner = block_owner(block_sizes(h), h->world);
+        }
+        {
             // refuse a model whose state cannot fit before anything is allocated, instead of failing with a bare out-of-memory
             // error here or partway through a solve
             size_t free_b = 0, total_b = 0;
@@ -690,7 +778,9 @@ int32_t lrn_finalize(lrn_handle_t h) {
         const int n = h->n_var;
         int maxm = 1;
         record_model_norms(h, h->hb);          // norms of AA_i, b, C_lin rows for lrn_initial_point (host copies still exist)
-        for (auto& B : h->blk) { build_block(h, B); maxm = std::max(maxm, B.m); }
+        bool keep_G = h->opt.datarank == -1 && h->nlmi > 0;          // the rank-one test below, from the staged data
+        for (auto& B : h->blk) keep_G = keep_G && B.hB.set && !B.hB.rowval.empty();
+        for (int i = 0; i < h->nlmi; i++) { build_block(h, h->blk[i], h->owns(i), keep_G); maxm = std::max(maxm, h->blk[i].m); }
         if (h->nlin > 0) {
             LRN_REQUIRE(h->hClin.set, "lrn_set_lin was not called");
             SparseLin& L = h->lin;
@@ -733,6 +823,7 @@ int32_t lrn_finalize(lrn_handle_t h) {
         {   // equal-sized blocks share a batched SVD
             std::vector<std::pair<int, std::vector<int>>> bym;
             for (int i = 0; i < h->nlmi; i++) {
+                if (!h->owns(i)) continue;
                 bool found = false;
                 for (auto& g : bym) if (g.first == h->blk[i].m) { g.second.push_back(i); found = true; }
                 if (!found) bym.push_back({h->blk[i].m, {i}});
@@ -755,7 +846,7 @@ int32_t lrn_finalize(lrn_handle_t h) {
             std::vector<double*> ptrs; std::vector<int> ms, lds;
             for (int i = 0; i < h->nlmi; i++) {
                 Block& B = h->blk[i];
-                if (B.m > 64 && B.m <= 384) {
+                if (h->owns(i) && B.m > 64 && B.m <= 384) {
                     h->eig_small.push_back(i);
                     ptrs.push_back(B.T4.p()); ptrs.push_back(B.T1.p());
                     ms.push_back(B.m); ms.push_back(B.m); lds.push_back(B.ld); lds.push_back(B.ld);
@@ -774,6 +865,13 @@ int32_t lrn_finalize(lrn_handle_t h) {
             h->H.init(rows, n);
             h->L.init(rows, n);
             if (rank1) h->BG.init(n, round_up(maxm, 32));   // K padded to a multiple of 32 (zero columns) for the TMA-fed SYRK
+        }
+        if (h->blk_sharded) {
+            h->gchunk = gather_chunk(h, h->blk_owner);
+            h->gbuf.alloc((size_t)(h->world + 1) * h->gchunk);
+            h->vpart.alloc(n);
+            h->vparts.alloc((size_t)h->world * n);
+            h->vshare.alloc(5 * (size_t)h->nlmi);
         }
         LRN_CUDA(cudaStreamSynchronize(h->st));
         h->finalized = true;
@@ -834,6 +932,7 @@ int32_t lrn_set_iterate(lrn_handle_t h, const double* const* X, const double* co
         LRN_REQUIRE(h->finalized, "lrn_finalize first");
         for (int i = 0; i < h->nlmi; i++) {
             LRN_REQUIRE(X && S && X[i] && S[i], "null X/S block");
+            if (!h->owns(i)) continue;
             upload_dense(h, h->blk[i].X, X[i]);
             upload_dense(h, h->blk[i].S, S[i]);
             h->blk[i].chol_cached = false;
@@ -853,31 +952,67 @@ int32_t lrn_set_iterate(lrn_handle_t h, const double* const* X, const double* co
     });
 }
 
-int32_t lrn_get_solution(lrn_handle_t h, double* y, double* const* X, double* x_lin) {
-    if (h && h->group) return lrn_get_solution(static_cast<Group*>(h->group)->members[0], y, X, x_lin);
-    return guarded(h, [&]() -> int32_t {
-        if (y) LRN_CUDA(cudaMemcpyAsync(y, h->y.p, h->n_var * sizeof(double), cudaMemcpyDeviceToHost, h->st));
-        if (X)
-            for (int i = 0; i < h->nlmi; i++)
-                if (X[i]) download_dense(h, h->blk[i].X.p(), h->blk[i].ld, h->blk[i].m, h->blk[i].m, X[i]);
-        if (x_lin && h->nlin > 0)
-            LRN_CUDA(cudaMemcpyAsync(x_lin, h->x_lin.p, h->nlin * sizeof(double), cudaMemcpyDeviceToHost, h->st));
-        LRN_CUDA(cudaStreamSynchronize(h->st));
-        return LRN_OK;
-    });
+// Host copy of a per-block device array of block i (m x m, or m long when `vec`; `dev` is ignored off the owner).  The owner
+// downloads it.  With the blocks distributed over the ranks and `collective` (a process-per-GPU handle) the owner broadcasts
+// it and every other rank receives it, so every rank must ask for the same blocks; otherwise a non-owner skips the block
+// (a group facade asks each block's owner member).
+static void block_to_host(lrn_solver* h, int i, const double* dev, bool vec, double* out, bool collective) {
+    const Block& B = h->blk[i];
+    const int ld = pad_ld(B.m);
+    const size_t count = vec ? (size_t)B.m : (size_t)ld * B.m;
+    cudaStream_t st = h->st;
+    const bool bcast = collective && h->blk_sharded;
+    if (h->owns(i)) {
+        if (bcast) ctx_of(h).bcast(const_cast<double*>(dev), count, h->rank, st);
+        if (vec) LRN_CUDA(cudaMemcpyAsync(out, dev, count * sizeof(double), cudaMemcpyDeviceToHost, st));
+        else download_dense(h, dev, ld, B.m, B.m, out);
+        return;
+    }
+    if (!bcast) return;
+    DevBuf<double> tmp(count);
+    ctx_of(h).bcast(tmp.p, count, h->blk_owner[i], st);
+    if (vec) LRN_CUDA(cudaMemcpyAsync(out, tmp.p, count * sizeof(double), cudaMemcpyDeviceToHost, st));
+    else download_dense(h, tmp.p, ld, B.m, B.m, out);
+    LRN_CUDA(cudaStreamSynchronize(st));
 }
 
-int32_t lrn_get_slack(lrn_handle_t h, double* const* S, double* s_lin) {
-    if (h && h->group) return lrn_get_slack(static_cast<Group*>(h->group)->members[0], S, s_lin);
+// lrn_get_solution / lrn_get_slack of one handle; `collective` as in block_to_host
+static int32_t get_iterate(lrn_solver* h, double* y, double* const* X, double* x_lin, double* const* S, double* s_lin,
+                           bool collective) {
     return guarded(h, [&]() -> int32_t {
-        if (S)
-            for (int i = 0; i < h->nlmi; i++)
-                if (S[i]) download_dense(h, h->blk[i].S.p(), h->blk[i].ld, h->blk[i].m, h->blk[i].m, S[i]);
+        if (y) LRN_CUDA(cudaMemcpyAsync(y, h->y.p, h->n_var * sizeof(double), cudaMemcpyDeviceToHost, h->st));
+        for (int i = 0; i < h->nlmi; i++) {
+            if (X && X[i]) block_to_host(h, i, h->blk[i].X.p(), false, X[i], collective);
+            if (S && S[i]) block_to_host(h, i, h->blk[i].S.p(), false, S[i], collective);
+        }
+        if (x_lin && h->nlin > 0)
+            LRN_CUDA(cudaMemcpyAsync(x_lin, h->x_lin.p, h->nlin * sizeof(double), cudaMemcpyDeviceToHost, h->st));
         if (s_lin && h->nlin > 0)
             LRN_CUDA(cudaMemcpyAsync(s_lin, h->s_lin.p, h->nlin * sizeof(double), cudaMemcpyDeviceToHost, h->st));
         LRN_CUDA(cudaStreamSynchronize(h->st));
         return LRN_OK;
     });
+}
+// group facade: the replicated parts from member 0, each block from its owner member
+static int32_t group_get_iterate(lrn_solver* h, double* y, double* const* X, double* x_lin, double* const* S, double* s_lin) {
+    const auto& mem = static_cast<Group*>(h->group)->members;
+    if (!mem[0]->blk_sharded) return get_iterate(mem[0], y, X, x_lin, S, s_lin, false);
+    for (size_t r = 0; r < mem.size(); r++) {
+        const int32_t rc = r == 0 ? get_iterate(mem[r], y, X, x_lin, S, s_lin, false)
+                                  : get_iterate(mem[r], nullptr, X, nullptr, S, nullptr, false);
+        if (rc != LRN_OK) { h->err = mem[r]->err; return rc; }
+    }
+    return LRN_OK;
+}
+
+int32_t lrn_get_solution(lrn_handle_t h, double* y, double* const* X, double* x_lin) {
+    if (h && h->group) return group_get_iterate(h, y, X, x_lin, nullptr, nullptr);
+    return get_iterate(h, y, X, x_lin, nullptr, nullptr, true);
+}
+
+int32_t lrn_get_slack(lrn_handle_t h, double* const* S, double* s_lin) {
+    if (h && h->group) return group_get_iterate(h, nullptr, nullptr, nullptr, S, s_lin);
+    return get_iterate(h, nullptr, nullptr, nullptr, S, s_lin, true);
 }
 
 // symmetric m x m product op(A) op(B): only the tiles that meet the lower triangle are computed, then mirrored
@@ -922,6 +1057,74 @@ static void side_join(lrn_solver* h) {
     }
 }
 
+// ---- PSD blocks distributed over the ranks (blk_sharded) ---------------------------------------------------------------
+static int owned_blocks(const lrn_solver* h) {
+    int c = 0;
+    for (int i = 0; i < h->nlmi; i++) c += h->owns(i);
+    return c;
+}
+
+// out = base + (part_0 + part_1 + ... + part_{world-1}), the partials in rank order: the same bits on every rank, every run
+static __global__ void k_add_parts(int n, int world, const double* __restrict__ base, const double* __restrict__ parts,
+                                   double* __restrict__ out) {
+    const int i = blockIdx.x * TBK + threadIdx.x;
+    if (i >= n) return;
+    double s = parts[i];
+    for (int r = 1; r < world; r++) s += parts[(size_t)r * n + i];
+    out[i] = base[i] + s;
+}
+// the owners' block terms of the residual / right-hand side sit in vpart on every rank: one all-gather, then out = base + sum
+static void combine_parts(lrn_solver* h, const double* base, double* out) {
+    const int n = h->n_var;
+    ctx_of(h).allgather(h->vpart.p, h->vparts.p, (size_t)n * sizeof(double), h->st);
+    k_add_parts<<<nb(n), TBK, 0, h->st>>>(n, h->world, base, h->vparts.p, out);
+    LRN_CHECK_LAUNCH();
+}
+
+// v holds k values per block, set by the owner of each block and zero elsewhere; afterwards every rank holds all of them (a sum
+// with one nonzero term per entry is exact)
+static void share_block_values(lrn_solver* h, std::vector<double>& v) {
+    LRN_REQUIRE(v.size() <= h->vshare.n, "share_block_values: too many values");
+    cudaStream_t st = h->st;
+    LRN_CUDA(cudaMemcpyAsync(h->vshare.p, v.data(), v.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    ctx_of(h).allreduce_sum(h->vshare.p, v.size(), st);
+    LRN_CUDA(cudaMemcpyAsync(v.data(), h->vshare.p, v.size() * sizeof(double), cudaMemcpyDeviceToHost, st));
+    LRN_CUDA(cudaStreamSynchronize(st));
+}
+
+// end of prepare_W: ONE padded all-gather sends every owner's W_i (G_i for datarank = -1), packed in block order, with its
+// status flag, to all ranks; the other ranks copy the blocks into place.  Returns the OR of the flags.
+static bool gather_blocks(lrn_solver* h, bool failed) {
+    cudaStream_t st = h->st;
+    const bool useG = h->opt.datarank == -1;
+    const size_t c = h->gchunk;
+    double* send = h->gbuf.p;
+    size_t off = 0;
+    for (int i = 0; i < h->nlmi; i++) {
+        if (!h->owns(i)) continue;
+        const DMat& M = useG ? h->blk[i].G : h->blk[i].W;
+        LRN_CUDA(cudaMemcpyAsync(send + off, M.p(), M.bytes(), cudaMemcpyDeviceToDevice, st));
+        off += (size_t)M.ld * M.cols;
+    }
+    const double flag = failed ? 1.0 : 0.0;
+    LRN_CUDA(cudaMemcpyAsync(send + c - 1, &flag, sizeof(double), cudaMemcpyHostToDevice, st));
+    ctx_of(h).allgather(send, send + c, c * sizeof(double), st);
+    std::vector<size_t> roff(h->world, 0);
+    for (int i = 0; i < h->nlmi; i++) {
+        const int r = h->blk_owner[i];
+        const DMat& M = useG ? h->blk[i].G : h->blk[i].W;
+        const size_t cnt = (size_t)pad_ld(h->blk[i].m) * h->blk[i].m;
+        if (r != h->rank)
+            LRN_CUDA(cudaMemcpyAsync(M.p(), send + c * (1 + r) + roff[r], cnt * sizeof(double), cudaMemcpyDeviceToDevice, st));
+        roff[r] += cnt;
+    }
+    std::vector<double> flags(h->world);
+    LRN_CUDA(cudaMemcpy2DAsync(flags.data(), sizeof(double), send + 2 * c - 1, c * sizeof(double), sizeof(double), h->world,
+                               cudaMemcpyDeviceToHost, st));
+    LRN_CUDA(cudaStreamSynchronize(st));
+    return std::any_of(flags.begin(), flags.end(), [](double f) { return f != 0.0; });
+}
+
 // ---- hot path -------------------------------------------------------------------------------------------------------
 int32_t lrn_find_mu(lrn_handle_t h, double* mu) {
     LRN_GROUP(h, lrn_find_mu(m_, r_ == 0 ? mu : group_scratch().d));
@@ -929,6 +1132,22 @@ int32_t lrn_find_mu(lrn_handle_t h, double* mu) {
         LRN_REQUIRE(mu, "null output");
         cudaStream_t st = h->st;
         h->red.zero(st);
+        if (h->blk_sharded) {
+            // <X_i, S_i> on the owners, shared, and summed in block order
+            for (int i = 0; i < h->nlmi; i++)
+                if (h->owns(i)) { Block& B = h->blk[i]; h->red.dot_mat(st, B.m, B.m, B.X.p(), B.ld, B.S.p(), B.ld, 16 + 4 * i, false); }
+            if (h->nlin > 0) h->red.dot_vec(st, h->nlin, h->x_lin.p, h->s_lin.p, 0, false);
+            const double* r = h->red.fetch(st);
+            std::vector<double> v(h->nlmi, 0.0);
+            for (int i = 0; i < h->nlmi; i++) if (h->owns(i)) v[i] = r[16 + 4 * i];
+            const double lp = r[0];
+            share_block_values(h, v);
+            double t = 0.0;
+            for (double x : v) t += x;
+            if (h->nlin > 0) t += lp;
+            *mu = t / (double)(h->sum_m + h->nlin);
+            return LRN_OK;
+        }
         for (auto& B : h->blk) h->red.dot_mat(st, B.m, B.m, B.X.p(), B.ld, B.S.p(), B.ld, 0, true);
         if (h->nlin > 0) h->red.dot_vec(st, h->nlin, h->x_lin.p, h->s_lin.p, 0, true);
         const double* r = h->red.fetch(st);
@@ -943,12 +1162,16 @@ int32_t lrn_prepare_W(lrn_handle_t h, int32_t* status4) {
         Phase ph(h, LRN_T_PREPARE_W);
         cudaStream_t st = h->st;
         if (status4) *status4 = 0;
+        bool failed = false;
         const double svd_tol = h->opt.svd_tol > 0 ? h->opt.svd_tol : 1e-8;
-        for (auto& B : h->blk) {
+        for (int i = 0; i < h->nlmi; i++) {
+            if (!h->owns(i)) continue;
+            Block& B = h->blk[i];
             const int m = B.m, ld = B.ld;
             if (!B.chol_cached) {
                 bool okx = try_cholesky(h, B.X, B.LX, B.cholX);
                 bool oks = try_cholesky(h, B.S, B.LS, B.cholS);
+                if (!okx || !oks) failed = true;
                 if ((!okx || !oks) && status4) *status4 = 1;
             }
             B.chol_cached = false;
@@ -970,15 +1193,16 @@ int32_t lrn_prepare_W(lrn_handle_t h, int32_t* status4) {
                 h->stat_svd_sweeps = svd_block_jacobi_batched(G->A.p, h->blk[G->blocks[0]].ld, G->m, (int)G->blocks.size(), G->UD.p,
                                                               h->blk[G->blocks[0]].ld, G->sig.p, G->w, svd_tol, 30, st);
             for (int i = 0; i < h->nlmi; i++) {
-                if (h->svd_group_of[i] >= 0) continue;
+                if (h->svd_group_of[i] >= 0 || !h->owns(i)) continue;
                 Block& B = h->blk[i];
                 h->stat_svd_sweeps = svd_block_jacobi(B.T1.p(), B.ld, B.m, B.T2.p(), B.ld, nullptr, 0, B.D.p, B.svd, svd_tol, 30, st);
             }
         }
-        const bool fanw = h->nlmi >= 4;          // independent per-block post-processing chains -> side streams
+        const bool fanw = owned_blocks(h) >= 4;  // independent per-block post-processing chains -> side streams
         if (fanw) side_fork(h);
         cudaStream_t st_main = st;
         for (int ib = 0; ib < h->nlmi; ib++) {
+            if (!h->owns(ib)) continue;
             Block& B = h->blk[ib];
             const int m = B.m, ld = B.ld;
             cudaStream_t st = fanw ? h->side[ib % lrn_solver::NSIDE] : st_main;
@@ -1000,6 +1224,10 @@ int32_t lrn_prepare_W(lrn_handle_t h, int32_t* status4) {
             B.ud_valid = true;        // T2 = U D and LS stay intact until the next call that uses the scratch matrices
         }
         if (fanw) side_join(h);
+        if (h->blk_sharded) {
+            if (gather_blocks(h, failed) && status4) *status4 = 1;
+            for (auto& B : h->blk) B.ud_valid = true;     // the owners' U D (Gi hook): every rank takes part in that getter
+        }
         if (h->nlin > 0) vec_op(st, h->nlin, VEC_RECIP, h->si_lin.p, h->s_lin.p, nullptr);
         return LRN_OK;
     });
@@ -1011,13 +1239,18 @@ int32_t lrn_residuals(lrn_handle_t h) {
         Phase ph(h, LRN_T_RESIDUALS);
         cudaStream_t st = h->st;
         const int n = h->n_var;
-        LRN_CUDA(cudaMemcpyAsync(h->Rp.p, h->b.p, n * sizeof(double), cudaMemcpyDeviceToDevice, st));
-        for (auto& B : h->blk) {
+        double* acc = h->blk_sharded ? h->vpart.p : h->Rp.p;     // sharded: the owned blocks' terms, then one all-gather
+        if (h->blk_sharded) LRN_CUDA(cudaMemsetAsync(acc, 0, n * sizeof(double), st));
+        else LRN_CUDA(cudaMemcpyAsync(h->Rp.p, h->b.p, n * sizeof(double), cudaMemcpyDeviceToDevice, st));
+        for (int i = 0; i < h->nlmi; i++) {
+            Block& B = h->blk[i];
             B.rdb_valid = false;
-            sp_A_vec(st, B.sp, B.X.p(), B.ld, -1.0, h->Rp.p);
+            if (!h->owns(i)) continue;
+            sp_A_vec(st, B.sp, B.X.p(), B.ld, -1.0, acc);
             mat_lincomb(st, B.m, B.m, B.Rd.p(), B.ld, 1.0, B.C.p(), B.C.ld, -1.0, B.S.p(), B.ld, 0.0, nullptr, 0);
             sp_scatter_ATy(st, B.sp, h->y.p, -1.0, B.Rd.p(), B.ld);
         }
+        if (h->blk_sharded) combine_parts(h, h->b.p, h->Rp.p);
         if (h->nlin > 0) {
             lin_C_x(st, h->lin, h->x_lin.p, -1.0, h->Rp.p);
             vec_axpby(st, h->nlin, h->tl1.p, 1.0, h->d_lin.p, -1.0, h->s_lin.p);
@@ -1057,13 +1290,19 @@ int32_t lrn_schur_assemble(lrn_handle_t h) {
                 if (h->world <= 1) gemm(p, st);
                 else syrk_sq_row_blocks(h->BG.p(), h->BG.ld, n, Kp, h->H.p(), h->H.ld, own.rank, own.world, own.pw, st, h->rows_local);
             } else {
+                // a block of another rank has no scratch matrices: its F1 columns use the all-gather buffer, whose
+                // (world + 1) chunks hold three of them (its content is dead until the next prepare_W)
+                const size_t mm = (size_t)ld * m;
+                double* T1 = B.T1.p() ? B.T1.p() : h->gbuf.p;
+                double* T2 = B.T2.p() ? B.T2.p() : h->gbuf.p + mm;
+                double* T3 = B.T3.p() ? B.T3.p() : h->gbuf.p + 2 * mm;
                 for (int jj = 0; jj < B.sp.nF1; jj++) {
                     // F1: U = W calA_j W, column of <calA_k, U>                (src/makeBBBB.jl:81-104)
-                    LRN_CUDA(cudaMemsetAsync(B.T1.p(), 0, B.T1.bytes(), st));
-                    sp_densify(st, B.sp, B.sp.h_part[jj], B.T1.p(), ld);
-                    gemm_nn(st, m, m, m, 1.0, B.W.p(), ld, B.T1.p(), ld, 0.0, B.T2.p(), ld);
-                    gemm_nn(st, m, m, m, 1.0, B.T2.p(), ld, B.W.p(), ld, 0.0, B.T3.p(), ld);
-                    sp_schur_f1_column(st, B.sp, jj, B.T3.p(), ld, h->H.p(), h->H.ld, own);
+                    LRN_CUDA(cudaMemsetAsync(T1, 0, mm * sizeof(double), st));
+                    sp_densify(st, B.sp, B.sp.h_part[jj], T1, ld);
+                    gemm_nn(st, m, m, m, 1.0, B.W.p(), ld, T1, ld, 0.0, T2, ld);
+                    gemm_nn(st, m, m, m, 1.0, T2, ld, B.W.p(), ld, 0.0, T3, ld);
+                    sp_schur_f1_column(st, B.sp, jj, T3, ld, h->H.p(), h->H.ld, own);
                 }
                 // F3 for the remaining (sparse) matrices                       (src/makeBBBB.jl:139-213)
                 if (B.sp.pairs.ok && (h->use_staged_pairs == 1 || (h->use_staged_pairs < 0 && B.sp.npart >= 1024)))
@@ -1094,8 +1333,12 @@ int32_t lrn_rhs_predictor(lrn_handle_t h) {
         for (auto& Bk : h->blk) Bk.ud_valid = false;
         Phase ph(h, LRN_T_RHS);
         cudaStream_t st = h->st;
-        LRN_CUDA(cudaMemcpyAsync(h->rhs.p, h->Rp.p, h->n_var * sizeof(double), cudaMemcpyDeviceToDevice, st));
-        for (auto& B : h->blk) {
+        double* acc = h->blk_sharded ? h->vpart.p : h->rhs.p;    // sharded: the owned blocks' terms, then one all-gather
+        if (h->blk_sharded) LRN_CUDA(cudaMemsetAsync(acc, 0, h->n_var * sizeof(double), st));
+        else LRN_CUDA(cudaMemcpyAsync(h->rhs.p, h->Rp.p, h->n_var * sizeof(double), cudaMemcpyDeviceToDevice, st));
+        for (int i = 0; i < h->nlmi; i++) {
+            if (!h->owns(i)) continue;
+            Block& B = h->blk[i];
             const int m = B.m, ld = B.ld;
             // h += AA * vec(W (Rd + S) W)                                     (src/makeBBBB.jl:225)
             mat_lincomb(st, m, m, B.T1.p(), ld, 1.0, B.Rd.p(), ld, 1.0, B.S.p(), ld, 0.0, nullptr, 0);
@@ -1103,13 +1346,14 @@ int32_t lrn_rhs_predictor(lrn_handle_t h) {
                 // sparse data: <calA_j, W T W> is only needed at the stored positions -- Z = T W (one product), then one
                 // m-long inner product <W(:,p), Z(:,q)> per stored entry instead of the second m^3 product
                 gemm_nn(st, m, m, m, 1.0, B.T1.p(), ld, B.W.p(), ld, 0.0, B.T2.p(), ld);
-                sp_A_sampled(st, B.sp, B.W.p(), ld, B.T2.p(), ld, 1.0, h->rhs.p);
+                sp_A_sampled(st, B.sp, B.W.p(), ld, B.T2.p(), ld, 1.0, acc);
             } else {
                 gemm_nn(st, m, m, m, 1.0, B.W.p(), ld, B.T1.p(), ld, 0.0, B.T2.p(), ld);
                 gemm_sym(st, false, false, m, B.T2.p(), ld, B.W.p(), ld, B.T3.p(), ld);
-                sp_A_vec(st, B.sp, B.T3.p(), ld, 1.0, h->rhs.p);
+                sp_A_vec(st, B.sp, B.T3.p(), ld, 1.0, acc);
             }
         }
+        if (h->blk_sharded) combine_parts(h, h->Rp.p, h->rhs.p);
         add_lp_rhs(h, 0, 0.0);
         return LRN_OK;
     });
@@ -1122,8 +1366,12 @@ int32_t lrn_rhs_corrector(lrn_handle_t h, double sigma, double mu) {
         Phase ph(h, LRN_T_RHS);
         cudaStream_t st = h->st;
         const double sm = sigma * mu;
-        LRN_CUDA(cudaMemcpyAsync(h->rhs.p, h->Rp.p, h->n_var * sizeof(double), cudaMemcpyDeviceToDevice, st));
-        for (auto& B : h->blk) {
+        double* acc = h->blk_sharded ? h->vpart.p : h->rhs.p;
+        if (h->blk_sharded) LRN_CUDA(cudaMemsetAsync(acc, 0, h->n_var * sizeof(double), st));
+        else LRN_CUDA(cudaMemcpyAsync(h->rhs.p, h->Rp.p, h->n_var * sizeof(double), cudaMemcpyDeviceToDevice, st));
+        for (int i = 0; i < h->nlmi; i++) {
+            if (!h->owns(i)) continue;
+            Block& B = h->blk[i];
             const int m = B.m, ld = B.ld;
             // h += AA * vec(G (G' Rd G + diag(D) - diag(sigma mu ./ D) - RNT) G')      (src/predictor_corrector.jl:186)
             if (use_rdb(B)) {
@@ -1139,13 +1387,14 @@ int32_t lrn_rhs_corrector(lrn_handle_t h, double sigma, double mu) {
                 // one product K G', an explicit G' (T4 is free here) and one m-long inner product per stored entry
                 gemm_nt(st, m, m, m, 1.0, B.T2.p(), ld, B.G.p(), ld, 0.0, B.T1.p(), ld);
                 mat_transpose(st, m, B.T4.p(), ld, B.G.p(), ld);
-                sp_A_sampled(st, B.sp, B.T1.p(), ld, B.T4.p(), ld, 1.0, h->rhs.p);
+                sp_A_sampled(st, B.sp, B.T1.p(), ld, B.T4.p(), ld, 1.0, acc);
             } else {
                 gemm_nn(st, m, m, m, 1.0, B.G.p(), ld, B.T2.p(), ld, 0.0, B.T1.p(), ld);
                 gemm_sym(st, false, true, m, B.T1.p(), ld, B.G.p(), ld, B.T3.p(), ld);
-                sp_A_vec(st, B.sp, B.T3.p(), ld, 1.0, h->rhs.p);
+                sp_A_vec(st, B.sp, B.T3.p(), ld, 1.0, acc);
             }
         }
+        if (h->blk_sharded) combine_parts(h, h->Rp.p, h->rhs.p);
         add_lp_rhs(h, 1, sm);
         return LRN_OK;
     });
@@ -1235,10 +1484,14 @@ int32_t lrn_find_step(lrn_handle_t h, int32_t predict, double sigma, double mu, 
         const double sm = sigma * mu;
         // multi-block problems whose blocks all go to the batched lambda_min kernel have no host synchronisation inside the
         // loop: the independent per-block chains of small kernels are spread over the side streams
-        bool fan = h->nlmi >= 4 && h->eig_small.size() == (size_t)h->nlmi;
+        const int nown = owned_blocks(h);
+        bool fan = nown >= 4 && h->eig_small.size() == (size_t)nown;
         if (fan) side_fork(h);
         cudaStream_t st_main = st;
+        if (h->blk_sharded)
+            for (int i = 0; i < h->nlmi; i++) alpha[i] = beta[i] = 0.0;
         for (int i = 0; i < h->nlmi; i++) {
+            if (!h->owns(i)) continue;
             Block& B = h->blk[i];
             const int m = B.m, ld = B.ld;
             cudaStream_t st = fan ? h->side[i % lrn_solver::NSIDE] : st_main;
@@ -1325,8 +1578,16 @@ int32_t lrn_find_step(lrn_handle_t h, int32_t predict, double sigma, double mu, 
             *alpha_lin = steplen(r[0], tau);
             *beta_lin = steplen(r[1], tau);
         }
+        if (h->blk_sharded) {
+            // every rank needs every alpha_i, beta_i: the corrector step is their minimum
+            std::vector<double> v(2 * (size_t)h->nlmi);
+            for (int i = 0; i < h->nlmi; i++) { v[2 * i] = alpha[i]; v[2 * i + 1] = beta[i]; }
+            share_block_values(h, v);
+            for (int i = 0; i < h->nlmi; i++) { alpha[i] = v[2 * i]; beta[i] = v[2 * i + 1]; }
+        }
         if (predict) {
             for (int i = 0; i < h->nlmi; i++) {
+                if (!h->owns(i)) continue;
                 Block& B = h->blk[i];
                 const int m = B.m, ld = B.ld;
                 // Xn, Sn, RNT                                                   (:306-309)
@@ -1341,7 +1602,9 @@ int32_t lrn_find_step(lrn_handle_t h, int32_t predict, double sigma, double mu, 
             for (int i = 0; i < h->nlmi; i++) { amin = std::min(amin, alpha[i]); bmin = std::min(bmin, beta[i]); }
             // y, X, S update                                                    (:313-321, :358-360)
             vec_axpby(st, h->n_var, h->y.p, 1.0, h->y.p, bmin, h->dely.p);
-            for (auto& B : h->blk) {
+            for (int i = 0; i < h->nlmi; i++) {
+                if (!h->owns(i)) continue;
+                Block& B = h->blk[i];
                 const int m = B.m, ld = B.ld;
                 mat_lincomb(st, m, m, B.X.p(), ld, 1.0, B.X.p(), ld, amin, B.dX.p(), ld, 0.0, nullptr, 0);
                 mat_symmetrize(st, m, B.X.p(), ld);
@@ -1367,11 +1630,23 @@ int32_t lrn_sigma_trace(lrn_handle_t h, double* tr, double* dl) {
         LRN_REQUIRE(tr && dl, "null outputs");
         cudaStream_t st = h->st;
         h->red.zero(st);
-        for (auto& B : h->blk) h->red.dot_mat(st, B.m, B.m, B.Xn.p(), B.ld, B.Sn.p(), B.ld, 0, true);
+        if (h->blk_sharded) {
+            for (int i = 0; i < h->nlmi; i++)
+                if (h->owns(i)) { Block& B = h->blk[i]; h->red.dot_mat(st, B.m, B.m, B.Xn.p(), B.ld, B.Sn.p(), B.ld, 16 + 4 * i, false); }
+        } else {
+            for (auto& B : h->blk) h->red.dot_mat(st, B.m, B.m, B.Xn.p(), B.ld, B.Sn.p(), B.ld, 0, true);
+        }
         if (h->nlin > 0) h->red.dot_vec(st, h->nlin, h->xn_lin.p, h->sn_lin.p, 1, false);
         const double* r = h->red.fetch(st);
         *tr = r[0];
         *dl = r[1];
+        if (h->blk_sharded) {
+            std::vector<double> v(h->nlmi, 0.0);
+            for (int i = 0; i < h->nlmi; i++) if (h->owns(i)) v[i] = r[16 + 4 * i];
+            share_block_values(h, v);
+            *tr = 0.0;
+            for (double x : v) *tr += x;
+        }
         return LRN_OK;
     });
 }
@@ -1390,6 +1665,7 @@ int32_t lrn_dimacs(lrn_handle_t h, double* err6, double* by_out, double* trCX_ou
         R.dot_vec(st, h->n_var, h->Rp.p, h->Rp.p, 0, false);
         R.dot_vec(st, h->n_var, h->b.p, h->y.p, 1, false);
         for (int i = 0; i < h->nlmi; i++) {
+            if (!h->owns(i)) continue;
             Block& B = h->blk[i];
             R.dot_mat(st, B.m, B.m, B.Rd.p(), B.ld, B.Rd.p(), B.ld, 16 + 4 * i, false);
             R.dot_mat(st, B.m, B.m, B.S.p(), B.ld, B.X.p(), B.ld, 16 + 4 * i + 1, false);
@@ -1400,7 +1676,7 @@ int32_t lrn_dimacs(lrn_handle_t h, double* err6, double* by_out, double* trCX_ou
             // are kept for the next prepare_W (X and S do not change in between).  The 2 nlmi factorisations are independent
             // and, for small blocks, latency-bound single-CTA-group kernels: multi-block problems spread them over side
             // streams (fork / join with events) so that they overlap.
-            const bool fan = h->nlmi >= 4;
+            const bool fan = owned_blocks(h) >= 4;
             if (fan && !h->side[0]) {
                 for (auto& s_ : h->side) LRN_CUDA(cudaStreamCreateWithFlags(&s_, cudaStreamNonBlocking));
                 LRN_CUDA(cudaEventCreateWithFlags(&h->evFork, cudaEventDisableTiming));
@@ -1411,6 +1687,7 @@ int32_t lrn_dimacs(lrn_handle_t h, double* err6, double* by_out, double* trCX_ou
                 for (auto& s_ : h->side) LRN_CUDA(cudaStreamWaitEvent(s_, h->evFork, 0));
             }
             for (int i = 0; i < h->nlmi; i++) {
+                if (!h->owns(i)) continue;
                 Block& B = h->blk[i];
                 cudaStream_t sx = fan ? h->side[(2 * i) % lrn_solver::NSIDE] : st;
                 cudaStream_t ss = fan ? h->side[(2 * i + 1) % lrn_solver::NSIDE] : st;
@@ -1439,18 +1716,27 @@ int32_t lrn_dimacs(lrn_handle_t h, double* err6, double* by_out, double* trCX_ou
         std::vector<double> v(r, r + R.nslots);
         const double nb_ = h->normb, by = v[1];
         double e1 = std::sqrt(v[0]) / (1 + nb_), e2 = 0, e3 = 0, e4 = 0, e5 = 0, e6 = 0, trCX = 0;
+        // per block: <Rd, Rd>, <S, X>, <C, X>, eigmin(X), eigmin(S) -- from the owner when the blocks are distributed
+        std::vector<double> bv(5 * (size_t)h->nlmi, 0.0);
         for (int i = 0; i < h->nlmi; i++) {
+            if (!h->owns(i)) continue;
             Block& B = h->blk[i];
-            const double CX = v[16 + 4 * i + 2];
-            trCX += CX;
             double lx = 1.0, ls = 1.0;
             if (infos[2 * i] != 0) lx = lambda_min(h, B.X.p(), B.m, B.ld);
             if (infos[2 * i + 1] != 0) ls = lambda_min(h, B.S.p(), B.m, B.ld);
             B.chol_cached = (infos[2 * i] == 0 && infos[2 * i + 1] == 0);
+            bv[5 * i] = v[16 + 4 * i]; bv[5 * i + 1] = v[16 + 4 * i + 1]; bv[5 * i + 2] = v[16 + 4 * i + 2];
+            bv[5 * i + 3] = lx; bv[5 * i + 4] = ls;
+        }
+        if (h->blk_sharded) share_block_values(h, bv);
+        for (int i = 0; i < h->nlmi; i++) {
+            const Block& B = h->blk[i];
+            const double CX = bv[5 * i + 2], lx = bv[5 * i + 3], ls = bv[5 * i + 4];
+            trCX += CX;
             e2 += std::max(0.0, -lx / (1 + nb_));
-            e3 += std::sqrt(v[16 + 4 * i]) / (1 + B.normC);
+            e3 += std::sqrt(bv[5 * i]) / (1 + B.normC);
             e4 += std::max(0.0, -ls / (1 + B.normC));
-            e6 += v[16 + 4 * i + 1] / (1 + std::fabs(CX) + std::fabs(by));
+            e6 += bv[5 * i + 1] / (1 + std::fabs(CX) + std::fabs(by));
         }
         e5 = (trCX - by) / (1 + std::fabs(trCX) + std::fabs(by));
         double dx = 0.0;
@@ -1500,17 +1786,8 @@ static void get_rows_local(lrn_solver* h, int32_t which, double* out, bool zero_
     }
 }
 
-int32_t lrn_get_array(lrn_handle_t h, int32_t which, int64_t iblk, double* out) {
-    // own-rows layout: every member writes its rows of H / L into the caller's array
-    if (h && h->group && (which == LRN_ARR_H || which == LRN_ARR_L) && static_cast<Group*>(h->group)->members[0]->rows_local) {
-        if (!out) return LRN_ERR_ARG;
-        return group_call(h, [&](lrn_solver* m_, int) -> int32_t {
-            return guarded(m_, [&]() -> int32_t { get_rows_local(m_, which, out, false); return LRN_OK; });
-        });
-    }
-    // Schur matrix: a collective (every member contributes its row blocks); everything else is replicated -> member 0
-    if (h && h->group && which != LRN_ARR_H) return lrn_get_array(static_cast<Group*>(h->group)->members[0], which, iblk, out);
-    LRN_GROUP(h, lrn_get_array(m_, which, iblk, r_ == 0 ? out : nullptr));
+// lrn_get_array of one handle; `collective` as in block_to_host
+static int32_t get_array(lrn_solver* h, int32_t which, int64_t iblk, double* out, bool collective) {
     return guarded(h, [&]() -> int32_t {
         LRN_REQUIRE(out || which == LRN_ARR_H, "null output");
         cudaStream_t st = h->st;
@@ -1538,38 +1815,64 @@ int32_t lrn_get_array(lrn_handle_t h, int32_t which, int64_t iblk, double* out) 
         else if (which == LRN_ARR_RP) vec_out(h->Rp.p, n);
         else {
             LRN_REQUIRE(iblk >= 0 && iblk < h->nlmi, "bad block index");
+            LRN_REQUIRE(which >= LRN_ARR_W && which <= LRN_ARR_SN, "unknown array id");
             Block& B = h->blk[iblk];
-            const DMat* M = nullptr;
-            switch (which) {
-                case LRN_ARR_W: M = &B.W; break;
-                case LRN_ARR_G: M = &B.G; break;
+            // Gi = D^{-1/2} U' L_S' = (L_S (U D) D^{-3/2})'  -- valid until the next prepare_W / find_step scratch reuse
+            LRN_REQUIRE(which != LRN_ARR_GI || B.ud_valid, "Gi is only available right after lrn_prepare_W (before any other hot-path call)");
+            const double* src = nullptr;                   // stays null off the owner (block_to_host receives it there)
+            if (h->owns((int)iblk)) switch (which) {
+                case LRN_ARR_W: src = B.W.p(); break;
+                case LRN_ARR_G: src = B.G.p(); break;
                 case LRN_ARR_GI: {
-                    // Gi = D^{-1/2} U' L_S' = (L_S (U D) D^{-3/2})'  -- valid until the next prepare_W / find_step scratch reuse
-                    LRN_REQUIRE(B.ud_valid, "Gi is only available right after lrn_prepare_W (before any other hot-path call)");
                     GemmParams p;
                     p.A = B.LS.p(); p.B = B.T2.p(); p.C = B.T1.p(); p.M = B.m; p.N = B.m; p.K = B.m;
                     p.lda = B.ld; p.ldb = B.ld; p.ldc = B.ld; p.colscale = B.dm32.p;
                     gemm(p, st);
                     mat_transpose(st, B.m, B.Gi.p(), B.ld, B.T1.p(), B.ld);
-                    M = &B.Gi;
+                    src = B.Gi.p();
                     break;
                 }
-                case LRN_ARR_SI: M = &B.Si; break;
-                case LRN_ARR_RD: M = &B.Rd; break;
-                case LRN_ARR_DELX: M = &B.dX; break;
-                case LRN_ARR_DELS: M = &B.dS; break;
-                case LRN_ARR_RNT: M = &B.RNT; break;
-                case LRN_ARR_XN: M = &B.Xn; break;
-                case LRN_ARR_SN: M = &B.Sn; break;
-                case LRN_ARR_D: vec_out(B.D.p, B.m); break;
-                case LRN_ARR_DDSI: vec_out(B.DDsi.p, B.m); break;
+                case LRN_ARR_SI: src = B.Si.p(); break;
+                case LRN_ARR_RD: src = B.Rd.p(); break;
+                case LRN_ARR_DELX: src = B.dX.p(); break;
+                case LRN_ARR_DELS: src = B.dS.p(); break;
+                case LRN_ARR_RNT: src = B.RNT.p(); break;
+                case LRN_ARR_XN: src = B.Xn.p(); break;
+                case LRN_ARR_SN: src = B.Sn.p(); break;
+                case LRN_ARR_D: src = B.D.p; break;
+                case LRN_ARR_DDSI: src = B.DDsi.p; break;
                 default: LRN_REQUIRE(false, "unknown array id");
             }
-            if (M) download_dense(h, M->p(), M->ld, B.m, B.m, out);
+            block_to_host(h, (int)iblk, src, which == LRN_ARR_D || which == LRN_ARR_DDSI, out, collective);
         }
         LRN_CUDA(cudaStreamSynchronize(st));
         return LRN_OK;
     });
+}
+
+int32_t lrn_get_array(lrn_handle_t h, int32_t which, int64_t iblk, double* out) {
+    // own-rows layout: every member writes its rows of H / L into the caller's array
+    if (h && h->group && (which == LRN_ARR_H || which == LRN_ARR_L) && static_cast<Group*>(h->group)->members[0]->rows_local) {
+        if (!out) return LRN_ERR_ARG;
+        return group_call(h, [&](lrn_solver* m_, int) -> int32_t {
+            return guarded(m_, [&]() -> int32_t { get_rows_local(m_, which, out, false); return LRN_OK; });
+        });
+    }
+    // Schur matrix: a collective (every member contributes its row blocks); everything else is replicated -> member 0, except
+    // the arrays of a block that lives on one member only
+    if (h && h->group && which != LRN_ARR_H) {
+        const auto& mem = static_cast<Group*>(h->group)->members;
+        if (mem[0]->blk_sharded && which >= LRN_ARR_W) {
+            if (iblk < 0 || iblk >= mem[0]->nlmi) { h->err = "bad block index"; return LRN_ERR_ARG; }
+            lrn_solver* o = mem[mem[0]->blk_owner[iblk]];
+            const int32_t rc = get_array(o, which, iblk, out, false);
+            if (rc != LRN_OK) h->err = o->err;
+            return rc;
+        }
+        return lrn_get_array(mem[0], which, iblk, out);
+    }
+    LRN_GROUP(h, lrn_get_array(m_, which, iblk, r_ == 0 ? out : nullptr));
+    return get_array(h, which, iblk, out, true);
 }
 
 int32_t lrn_timers(lrn_handle_t h, double* ms, int64_t* calls, int32_t reset) {

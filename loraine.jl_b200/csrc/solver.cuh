@@ -137,5 +137,17 @@ struct lrn_solver {
     bool H_gathered = false;           // the row-block shards of H have already been summed over the ranks (parity hooks)
     bool rows_local = false;           // kit = 0 storage: H and L hold only this rank's own row blocks (RowOwner::local, ops.cuh)
     int layout_force = -1;             // test hook lrn_dbg_schur_layout: -1 lrn_finalize decides, 0 replicated, 1 own rows
+    // PSD blocks distributed over the ranks (lrn_finalize: kit = 0, nlmi >= 2, a communicator with world > 1): block i lives
+    // on rank blk_owner[i] (lrn::block_owner, ops.cuh); the other ranks keep its sparse data and the gathered W_i (G_i when
+    // datarank = -1), which is all their Schur rows need
+    bool blk_sharded = false;
+    int blk_force = -1;                // test hook lrn_dbg_block_layout: -1 lrn_finalize decides, 0 replicated, 1 sharded
+    std::vector<int> blk_owner;
+    lrn::DevBuf<double> gbuf;          // W / G all-gather: chunk 0 this rank's packed blocks, chunk 1 + r rank r's (gchunk doubles
+                                       // each, the last one a status flag); between two prepare_W calls the F1 scratch
+    size_t gchunk = 0;
+    lrn::DevBuf<double> vpart, vparts; // residual / RHS partial n_var vectors: this rank's, every rank's (rank order)
+    lrn::DevBuf<double> vshare;        // per-block values (mu, step lengths, DIMACS terms) filled in by the owners, then summed
+    bool owns(int i) const { return !blk_sharded || blk_owner[i] == rank; }
     void* group = nullptr;             // lrn::Group*: this handle is the facade of an in-process multi-GPU group (group.cuh)
 };

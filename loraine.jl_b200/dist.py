@@ -69,6 +69,35 @@ def schur_bytes(n_var: int, pw: int, rank: int, world: int, rows_local: bool) ->
     return b
 
 
+def block_owner(msizes, world: int) -> list[int]:
+    """owner rank of every PSD block when the blocks are distributed over the ranks (mirrors lrn::block_owner in
+    csrc/ops.cuh): blocks by decreasing m_i^3 (ties: lower index first), each to the least-loaded rank (ties: lowest rank)"""
+    order = sorted(range(len(msizes)), key=lambda i: (-int(msizes[i]) ** 3, i))
+    load = [0] * max(world, 1)
+    owner = [0] * len(msizes)
+    for i in order:
+        r = min(range(len(load)), key=lambda k: (load[k], k))
+        owner[i] = r
+        load[r] += int(msizes[i]) ** 3
+    return owner
+
+
+def block_shard_bytes(msizes, n_var: int, rank: int, world: int) -> int:
+    """device bytes the distributed block layout adds on `rank` over the replicated one (mirrors direct_footprint in
+    csrc/solver.cu): each block of another rank keeps one m x m array instead of 24, plus the W / G all-gather buffer
+    ((world + 1) chunks of the largest per-rank load and a status flag), world + 1 partial n_var vectors and five shared
+    values per block"""
+    owner = block_owner(msizes, world)
+    mm = [pad_ld(m) * m for m in msizes]
+    load = [0] * world
+    for i, r in enumerate(owner):
+        load[r] += mm[i]
+    chunk = max(load) + 1
+    d = 8
+    saved = sum(23 * mm[i] for i, r in enumerate(owner) if r != rank) * d
+    return ((world + 1) * (chunk + n_var) + 5 * len(msizes)) * d - saved
+
+
 def exchange_unique_id(make_id, rank: int, world: int) -> bytes:
     """rank 0 calls make_id() -> 128 bytes; every rank returns the same bytes."""
     import torch.distributed as dist
